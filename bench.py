@@ -74,7 +74,13 @@ def parse_args():
     ap.add_argument("--no-mode-a", action="store_true", help="N>1: skip the independent-replica side measurement")
     ap.add_argument("--no-small", action="store_true", help="N=1: skip the fandisk-sized CAD-weights side measurement")
     ap.add_argument("--detail", default=None, help="write a per-kernel-group timing table (JSON) to this path")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step computed (loss, PosNet / NormalNet outputs, updated "
+                         "parameters) as DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -94,6 +100,28 @@ def build_case(n, device=None):
     n_mesh = Mesh(vs=case.noise_vs, faces=case.faces)
     s_mesh = SimpleNamespace(vs=case.smooth_vs)      # only the smoothed vertices are read (reference datamaker.py:87)
     return n_mesh, s_mesh, dataset_from_meshes(n_mesh, s_mesh)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, loss, pos, norm, posnet, normnet):
+    """Write the results of one step as float32 / float64 .npy files.  The mesh, its noise and the initial weights are
+    seeded, so the same arguments give the same inputs on every run.  Meshes so large that the files would exceed
+    DUMP_LIMIT_BYTES keep a fixed, seeded sample of the rows of ``pos`` and ``norm`` (sorted row indices, seed 0)."""
+    flat = lambda net: torch.cat([p.detach().reshape(-1) for p in net.parameters()]).cpu().numpy()   # noqa: E731
+    fixed = {"loss": np.asarray([loss.item()], dtype=np.float64),
+             "posnet_params": flat(posnet), "normnet_params": flat(normnet)}
+    rows = {"pos": pos.detach().float().cpu().numpy(), "norm": norm.detach().float().cpu().numpy()}
+    budget = DUMP_LIMIT_BYTES - 4096 - sum(a.nbytes for a in fixed.values())      # 4096: room for the .npy headers
+    total = sum(a.nbytes for a in rows.values())
+    if total > budget:
+        rng = np.random.default_rng(0)
+        rows = {k_: a[np.sort(rng.choice(len(a), int(len(a) * budget / total), replace=False))]
+                for k_, a in rows.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in {**fixed, **rows}.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def spmm_bytes(n_nodes, nnz, C):
@@ -316,8 +344,15 @@ def run_ours(args):
     sampler.start()
     for i in range(max(args.warmup, 5)):            # 3 eager warm-up calls, then capture, then replays
         stepper.step(epoch0 + i)
-    ms, _ = timed(lambda i: stepper.step(epoch0 + i), args.steps, 0)
+    last_loss = [None]
+
+    def timed_step(i):
+        last_loss[0] = stepper.step(epoch0 + i)
+
+    ms, _ = timed(timed_step, args.steps, 0)
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:             # before the passes below move the parameters on
+        dump_outputs(args.dump_outputs, last_loss[0], stepper.pos, stepper.norm, posnet, normnet)
     ms_per_step = ms / args.steps
     value = world * 1000.0 / ms_per_step
 
@@ -906,6 +941,10 @@ def run_partitioned(args, weak):
 if __name__ == "__main__":
     a = parse_args()
     world_ = int(os.environ.get("WORLD_SIZE", "1"))
+    if a.dump_outputs and (a.impl == "reference" or a.mode.startswith("partition")
+                           or (a.mode == "auto" and world_ > 1)):
+        sys.exit("--dump-outputs is implemented for our arm's one-mesh-per-GPU run (--mode auto on one GPU, "
+                 "or --mode independent)")
     if a.impl == "reference":
         run_reference(a)
     elif a.mode == "partition":
