@@ -246,6 +246,30 @@ int ddmp_face_normals_fwd(const float* pos, const int32_t* faces, float* fn, int
 int ddmp_face_normals_bwd(const float* pos, const int32_t* faces, const int32_t* corner_ptr,
                           const int32_t* corner_slot, const float* gfn, float* face_tmp, float* gpos, int64_t V,
                           int64_t F, void* stream);
+/* Point-to-surface distance (csrc/distance.cu), float64.  For a query point p and a target mesh (vs [V,3], faces [F,3]):
+ *   dist(p) = min over faces f of |p - closest_point(p, triangle f)|  (exact Euclidean distance, no cutoff),
+ *   face(p) = the face attaining it, the lowest face id on an exact tie.
+ * A zero-area face (collinear or coincident corners) is the segment or point it spans; no input gives NaN or inf.
+ * Linear BVH (Karras 2012): 64-byte internal nodes holding both children's float32 boxes (rounded outward) and ids.
+ * The BVH query returns bit for bit the distance and face id of ddmp_point_mesh_distance_exhaustive.
+ * [ref: util/loss.py:279-284 distance_from_reference_mesh and check/hausdorff_checker.py, both pymeshlab] */
+/* keys [F] = 63-bit Morton code of each face centroid, 21 bits per axis quantised in bbox6 (ddmp_prep_bbox of vs),
+ * to be sorted stably by the caller -> sorted_keys, order (order[k] = face at sorted position k). */
+int ddmp_bvh_keys(const double* vs, const int32_t* faces, const double* bbox6, int64_t* keys, int64_t F, void* stream);
+/* nodes: max(F-1,1) x 64 bytes, 64-byte aligned; leaves [F][4] int32 = (v0, v1, v2, face) in sorted order; parent
+ * [2F-1] int32 scratch; counters [max(F-1,1)] int32, zero on entry and left zeroed.  F < 2^30. */
+int ddmp_bvh_build(const double* vs, const int32_t* faces, const int64_t* sorted_keys, const int64_t* order,
+                   void* nodes, int32_t* leaves, int32_t* parent, int32_t* counters, int64_t F, void* stream);
+/* points [P,3]; dist [P] float64, face [P] int32 (ids of the caller's face numbering) */
+int ddmp_point_mesh_distance(const double* points, int64_t P, const double* vs, const void* nodes,
+                             const int32_t* leaves, int64_t F, double* dist, int32_t* face, void* stream);
+/* the same outputs by scanning every face with the same leaf routine (reference for tests and benchmarks) */
+int ddmp_point_mesh_distance_exhaustive(const double* points, int64_t P, const double* vs, const int32_t* faces,
+                                        int64_t F, double* dist, int32_t* face, void* stream);
+/* out [4] = (min, max, sum, sum of squares) of dist [P], float64, fixed combination order; scratch: zeroed buffer of
+ * ddmp_distance_scratch_bytes() bytes, left zeroed. */
+int64_t ddmp_distance_scratch_bytes(void);
+int ddmp_distance_stats(const double* dist, int64_t P, double* out, void* scratch, void* stream);
 /* ---- partitioned mode: BatchNorm reductions over NVLink peer memory (csrc/comm.cu) ------------------------- */
 /* Every rank owns one exchange buffer (ddmp_comm_buffer_bytes() bytes, allocated and zeroed by ddmp_comm_alloc) that all
  * peers of the box map through CUDA IPC (ddmp_comm_ipc_handle on the owner -> 64 opaque bytes -> ddmp_comm_ipc_open on
