@@ -8,9 +8,10 @@
 //   NT kernels (xw, dx):  C[M=rows, N] = act(A)[rows, K] * B[N, K]^T        A, B K-major
 //   TN kernels (dw)    :  C[M, N] = sum_rows A[rows, M]^T * act(B)[rows, N]  A, B MN-major, split-K over rows
 //
-// The activation operand cannot come straight from TMA: the previous layer's BatchNorm + LeakyReLU, the scale and
-// the hi/lo split are applied while the tile is staged, so producer warps do  ld.global -> transform -> st.shared
-// into the 128-byte-swizzled UMMA canonical layout; the (pre-split, pre-swizzled) weights arrive by cp.async.bulk.
+// The activation operand cannot go to the tensor core as loaded: the previous layer's BatchNorm + LeakyReLU, the scale
+// and the hi/lo split are applied while the tile is staged, so producer warps do  ld.global -> transform -> st.shared
+// into the 128-byte-swizzled UMMA canonical layout (fp16 kernels at K <= 256: raw fp32 tiles by TMA, then
+// ld.shared -> transform -> st.shared); the (pre-split, pre-swizzled) weights arrive by cp.async.bulk.
 // One elected thread issues the MMAs; `full`/`empty` mbarriers per smem stage; tcgen05.commit releases a stage /
 // publishes the accumulator; dedicated warps drain the double-buffered TMEM accumulator.  CTA pairs (cta_group::2)
 // where the shapes allow.  Kernel inventory and measured behaviour: DESIGN.md §4.2, profiles/README.md.
@@ -778,6 +779,133 @@ __device__ __forceinline__ void produce_loop(const Args& g, int64_t first_tile, 
         process(buf1, vm1, k1, it + 1);
     }
 }
+
+// ---- A operand by TMA (no row gather; where run_nt16 selects it) -----------------------------------------------------
+// The register-fed producers above keep at most two k-blocks of A in flight per warp (~64 KB per SM) and pay the load
+// latency plus the transform once per k-block, which set the pace at K <= 256 (2-4 k-blocks of ~1.5 k MMA cycles per
+// tile) and wherever the BatchNorm + LeakyReLU prologue is applied.  Here one thread streams the raw fp32 A tile into a ring of `RAW` slots with TMA tensor loads
+// (two 128-row x 32-column boxes per k-block, 128-byte swizzle: the inner box dimension is limited to 128 bytes), and
+// the producer warps become shared -> shared transform warps: ld.shared -> BatchNorm + LeakyReLU + scale -> hi/lo split
+// -> st.shared, the same arithmetic and the same output layout as produce_loop, so the products are bitwise equal.
+// Rows past M arrive zero-filled; their transformed values only reach accumulator rows that are never stored.
+constexpr uint32_t kRawBoxBytes = BM * 128;                    // 128 rows x 32 fp32
+constexpr uint32_t kRawSlotBytes = 2 * kRawBoxBytes;           // one k-block of A: 128 rows x 64 fp32
+
+__device__ __forceinline__ void tma_load_2d(uint32_t dst_smem, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
+    asm volatile(
+        "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(
+            dst_smem),
+        "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar))
+        : "memory");
+}
+__device__ __forceinline__ float4 lds128f(uint32_t saddr) {
+    float4 v;
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(saddr)
+                 : "memory");
+    return v;
+}
+
+// one elected thread: the (tile, k-block) sequence of produce/transform_loop, A rows row_mul*(tile/tiles_n)+row_add
+template <int RAW, class Args>
+__device__ __forceinline__ void tma_a_loop(const Args& g, const CUtensorMap* amap, int64_t first_tile, int64_t tile_step,
+                                           int64_t row_mul, int64_t row_add, int num_kb, uint32_t raw_base,
+                                           uint64_t* raw_full, uint64_t* raw_empty) {
+    const bool tr = g.trace && blockIdx.x == 0;
+    uint32_t it = 0;
+    for (int64_t tile = first_tile; tile < g.num_tiles; tile += tile_step) {
+        const int row0 = (int)((tile / g.tiles_n) * row_mul + row_add);
+        for (int kb = 0; kb < num_kb; ++kb, ++it) {
+            const int r = it % RAW;
+            const uint32_t rph = (it / RAW) & 1;
+            long long c0 = 0;
+            if (tr) c0 = clock64();
+            mbar_wait(raw_empty + r, rph ^ 1u);
+            if (tr) g.trace[12] += (unsigned long long)(clock64() - c0);   // A loader: wait for a free raw slot
+            mbar_arrive_expect_tx(raw_full + r, kRawSlotBytes);
+            const uint32_t dst = raw_base + (uint32_t)r * kRawSlotBytes;
+            tma_load_2d(dst, amap, kb * BK16, row0, raw_full + r);
+            tma_load_2d(dst + kRawBoxBytes, amap, kb * BK16 + 32, row0, raw_full + r);
+        }
+    }
+}
+
+template <int STAGES, int RAW, class Args, class WaitEmpty>
+__device__ __forceinline__ void transform_loop(const Args& g, int64_t first_tile, int64_t tile_step, int num_kb, float s_a,
+                                               uint32_t smem_base, uint32_t raw_base, uint32_t stage_bytes,
+                                               uint32_t a_bytes, uint64_t* full_bar, uint64_t* empty_bar,
+                                               uint64_t* raw_full, uint64_t* raw_empty, WaitEmpty wait_empty) {
+    constexpr int NJ = kProdNJ, RPP = kProdRPP;
+    const int t = threadIdx.x, lane = threadIdx.x & 31;
+    const uint32_t c4 = t & 15;                           // 4 consecutive k of the k-block: 16-byte chunk c4 & 7 of box c4 >> 3
+    const int c8 = (int)c4 * 4;
+    const bool has_act = g.scale != nullptr;
+    const bool tr = g.trace && blockIdx.x == 0 && t == 0;
+    const int64_t my_tiles = first_tile < g.num_tiles ? (g.num_tiles - first_tile + tile_step - 1) / tile_step : 0;
+    const uint32_t total = (uint32_t)(my_tiles * num_kb);
+    const uint32_t rd = raw_base + (c4 >> 3) * kRawBoxBytes;
+    int kb = 0;
+    for (uint32_t it = 0; it < total; ++it) {
+        const int s = it % STAGES, r = it % RAW;
+        const uint32_t ph = (it / STAGES) & 1, rph = (it / RAW) & 1;
+        const int k0 = kb * BK16;
+        if (++kb == num_kb) kb = 0;
+        long long c1 = 0, c2 = 0, c3 = 0, cA = 0, cB = 0, c4t = 0;
+        float4 sc = make_float4(s_a, s_a, s_a, s_a), sh = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (has_act) {
+            sc = ldg4(g.scale + k0 + c8);
+            sh = ldg4(g.shift + k0 + c8);
+            sc.x *= s_a; sc.y *= s_a; sc.z *= s_a; sc.w *= s_a;
+            sh.x *= s_a; sh.y *= s_a; sh.z *= s_a; sh.w *= s_a;
+        }
+        if (tr) c1 = clock64();
+        mbar_wait(raw_full + r, rph);
+        if (tr) c2 = clock64();
+        const uint32_t raw = rd + (uint32_t)r * kRawSlotBytes;
+        float4 av[NJ];
+#pragma unroll
+        for (int j = 0; j < NJ; ++j) {
+            const uint32_t row = (t >> 4) + j * RPP;
+            av[j] = lds128f(raw + row * 128u + (((c4 & 7u) ^ (row & 7u)) << 4));
+        }
+        wait_empty(empty_bar + s, ph ^ 1u);
+        if (tr) c3 = clock64();
+        const uint32_t st = smem_base + s * stage_bytes;
+#pragma unroll
+        for (int j = 0; j < NJ; ++j) {
+            const uint32_t row = (t >> 4) + j * RPP;
+            float4 a = av[j];
+            if (has_act) {
+                a.x = lrelu_max(fmaf(a.x, sc.x, sh.x), g.slope); a.y = lrelu_max(fmaf(a.y, sc.y, sh.y), g.slope);
+                a.z = lrelu_max(fmaf(a.z, sc.z, sh.z), g.slope); a.w = lrelu_max(fmaf(a.w, sc.w, sh.w), g.slope);
+            } else {
+                a.x *= s_a; a.y *= s_a; a.z *= s_a; a.w *= s_a;
+            }
+            uint32_t h0, l0, h1, l1;
+            split_f16x2(a.x, a.y, h0, l0);
+            split_f16x2(a.z, a.w, h1, l1);
+            const uint32_t off = sw128(row, c4 >> 1) + ((c4 & 1u) << 3);
+            sts64(st + off, h0, h1);
+            sts64(st + a_bytes + off, l0, l1);
+        }
+        if (tr) cA = clock64();
+        fence_proxy_async();
+        if (tr) cB = clock64();
+        __syncwarp();
+        if (tr) c4t = clock64();
+        if (lane == 0) {
+            mbar_arrive(raw_empty + r);
+            mbar_arrive(full_bar + s);
+        }
+        if (tr) {
+            g.trace[11] += (unsigned long long)(c2 - c1);    // wait for the raw A slot (TMA)
+            g.trace[1] += (unsigned long long)(c3 - c2);     // shared loads + wait for a free stage
+            g.trace[2] += (unsigned long long)(c4t - c3);    // transform + stores + fence
+            g.trace[3] += 1ull;
+            g.trace[14] += (unsigned long long)(cA - c3);    // ... of which: transform + store issue
+            g.trace[15] += (unsigned long long)(cB - cA);    // ... fence.proxy.async
+        }
+    }
+}
 // Epilogue of the fp16-split NT kernels: one warp drains its 32 rows x BN columns of the accumulator.
 // tcgen05.ld hands every thread one ROW; the 32 x 32 block goes through a swizzled staging tile so that a store
 // instruction writes 4 rows x 128 B, and the column scales are applied on the way out (there a lane owns 4 fixed
@@ -973,21 +1101,28 @@ __global__ void tc_prep_b16_kernel(const float* __restrict__ W, int transposed, 
     }
 }
 
-template <int BN, int STAGES>
+// RAW = 0: A by the register-fed producers (produce_loop); RAW > 0: A by TMA into RAW raw slots (tma_a_loop +
+// transform_loop).  ACC: depth of the TMEM accumulator ring (ACC x BN columns).
+template <int BN, int STAGES, int RAW, int ACC>
 __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __grid_constant__ CUtensorMap cmap,
+                                                                     const __grid_constant__ CUtensorMap amap,
                                                                      const Nt16Args g) {
     constexpr uint32_t A_BYTES = BM * 128;           // 128 rows x 64 fp16, one of hi / lo
     constexpr uint32_t B_BYTES = BN * 128;
     constexpr uint32_t STAGE_BYTES = 2 * A_BYTES + 2 * B_BYTES;
-    constexpr uint32_t TMEM_COLS = 2 * BN;
+    constexpr uint32_t TMEM_COLS = ACC * BN;
+    static_assert(TMEM_COLS <= 512 && (TMEM_COLS & (TMEM_COLS - 1)) == 0, "TMEM allocation: power of two <= 512");
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    uint8_t* staging = smem + STAGES * STAGE_BYTES;          // 4 epilogue warps x 2 buffers x 32 rows x 128 B (1 KB aligned)
+    uint8_t* raw = smem + STAGES * STAGE_BYTES;              // RAW x 32 KB of fp32 A (1 KB aligned)
+    uint8_t* staging = raw + RAW * kRawSlotBytes;            // 4 epilogue warps x 2 buffers x 32 rows x 128 B (1 KB aligned)
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(staging + kStagingBytes);
     uint64_t* empty_bar = full_bar + STAGES;
-    uint64_t* acc_full = empty_bar + STAGES;     // [2]
-    uint64_t* acc_empty = acc_full + 2;          // [2]
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
+    uint64_t* acc_full = empty_bar + STAGES;     // [ACC]
+    uint64_t* acc_empty = acc_full + ACC;        // [ACC]
+    uint64_t* raw_full = acc_empty + ACC;        // [RAW]
+    uint64_t* raw_empty = raw_full + RAW;        // [RAW]
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(raw_empty + RAW);
     uint32_t* amax_slot = tmem_slot + 1;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -997,9 +1132,13 @@ __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __gri
             mbar_init(full_bar + s, kProducerWarps + 1);
             mbar_init(empty_bar + s, 1);
         }
-        for (int b = 0; b < 2; ++b) {
+        for (int b = 0; b < ACC; ++b) {
             mbar_init(acc_full + b, 1);
             mbar_init(acc_empty + b, 4);
+        }
+        for (int r = 0; r < RAW; ++r) {
+            mbar_init(raw_full + r, 1);
+            mbar_init(raw_empty + r, kProducerWarps);
         }
         *amax_slot = 0u;
         fence_barrier_init();
@@ -1016,24 +1155,39 @@ __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __gri
     scale_from_bits(*amax_slot, s_a, inv_sa);
 
     if (warp < kProducerWarps) {
-        // ===== A producers (see produce_loop) =====
+        // ===== A producers (see produce_loop / transform_loop) =====
         auto wait_empty = [](uint64_t* bar, uint32_t parity) { mbar_wait(bar, parity); };
-        produce_loop<STAGES>(g, (int64_t)blockIdx.x, (int64_t)gridDim.x, (int64_t)BM, 0, num_kb, s_a,
-                                        smem_base, STAGE_BYTES, A_BYTES, full_bar, empty_bar, wait_empty);
+        if constexpr (RAW > 0)
+            transform_loop<STAGES, RAW>(g, (int64_t)blockIdx.x, (int64_t)gridDim.x, num_kb, s_a, smem_base,
+                                        smem_u32(raw), STAGE_BYTES, A_BYTES, full_bar, empty_bar, raw_full, raw_empty,
+                                        wait_empty);
+        else
+            produce_loop<STAGES>(g, (int64_t)blockIdx.x, (int64_t)gridDim.x, (int64_t)BM, 0, num_kb, s_a,
+                                 smem_base, STAGE_BYTES, A_BYTES, full_bar, empty_bar, wait_empty);
     } else if (warp == 8) {
         // ===== MMA issuer =====
         if (lane == 0) {
             constexpr uint32_t idesc = make_idesc16(BM, BN, false, false);
+            const bool tr = g.trace && blockIdx.x == 0;
             uint32_t it = 0, tile_no = 0;
             for (int64_t tile = blockIdx.x; tile < g.num_tiles; tile += gridDim.x, ++tile_no) {
-                const uint32_t buf = tile_no & 1u;
-                mbar_wait(acc_empty + buf, ((tile_no >> 1) & 1u) ^ 1u);
+                const uint32_t buf = tile_no % ACC;
+                long long a0 = 0;
+                if (tr) a0 = clock64();
+                mbar_wait(acc_empty + buf, ((tile_no / ACC) & 1u) ^ 1u);
+                if (tr) g.trace[7] += (unsigned long long)(clock64() - a0);   // wait for a free accumulator
                 tc_fence_after();
                 const uint32_t d_tmem = tmem_base + buf * BN;
                 for (int kb = 0; kb < num_kb; ++kb, ++it) {
                     const int s = it % STAGES;
                     const uint32_t ph = (it / STAGES) & 1;
+                    long long c0 = 0;
+                    if (tr) c0 = clock64();
                     mbar_wait(full_bar + s, ph);
+                    if (tr) {
+                        g.trace[4] += (unsigned long long)(clock64() - c0);     // MMA thread: wait stage full
+                        g.trace[6] += 1ull;
+                    }
                     tc_fence_after();
                     const uint32_t sa = smem_base + s * STAGE_BYTES;
 #pragma unroll
@@ -1071,6 +1225,14 @@ __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __gri
             }
         }
         __syncwarp();
+    } else if (warp == 10) {
+        // ===== A loader (RAW > 0): TMA tensor loads into the raw ring =====
+        if constexpr (RAW > 0) {
+            if (lane == 0)
+                tma_a_loop<RAW>(g, &amap, (int64_t)blockIdx.x, (int64_t)gridDim.x, (int64_t)BM, 0, num_kb, smem_u32(raw),
+                                raw_full, raw_empty);
+        }
+        __syncwarp();
     } else if (warp >= 12) {
         // ===== epilogue: TMEM -> registers (unscale) -> swizzled staging tile -> global =====
         const int q = warp & 3;
@@ -1078,16 +1240,28 @@ __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __gri
         const bool staged = (g.flags & 16) != 0;         // A/B switch: the ld.shared + st.global epilogue
         uint32_t tile_no = 0;
         for (int64_t tile = blockIdx.x; tile < g.num_tiles; tile += gridDim.x, ++tile_no) {
-            const uint32_t buf = tile_no & 1u;
+            const uint32_t buf = tile_no % ACC;
             const int64_t mrow0 = (tile / g.tiles_n) * BM + q * 32;
             const int n0 = (int)(tile % g.tiles_n) * BN;
-            mbar_wait(acc_full + buf, (tile_no >> 1) & 1u);
+            const bool tr = g.trace && blockIdx.x == 0 && warp == 12 && lane == 0;
+            long long e0 = 0;
+            if (tr) e0 = clock64();
+            mbar_wait(acc_full + buf, (tile_no / ACC) & 1u);
+            if (tr) {
+                const long long e1 = clock64();
+                g.trace[8] += (unsigned long long)(e1 - e0);                 // epilogue: wait accumulator
+                g.trace[9] -= (unsigned long long)e1;                        // epilogue: drain (completed below)
+            }
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + buf * BN;
             if (staged) epilogue_tile<BN>(g, taddr, inv_sa, stg, lane, mrow0, n0);
             else epilogue_tile_tma<BN>(&cmap, g.inv_sw, taddr, inv_sa, stg, lane, mrow0, n0);
             tc_fence_before();
             __syncwarp();
+            if (tr) {
+                g.trace[9] += (unsigned long long)clock64();
+                g.trace[10] += 1ull;
+            }
             if (lane == 0) mbar_arrive(acc_empty + buf);
         }
         if (lane == 0) bulk_wait_all();                  // the staging buffers must outlive the last tensor stores
@@ -1099,21 +1273,33 @@ __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __gri
     }
 }
 
-template <int BN, int STAGES>
+// dynamic shared memory of the fp16-split NT kernels: split stages, raw A slots, epilogue staging, barriers
+constexpr size_t nt16_smem(int stages, uint32_t b_bytes, int raw) {
+    return (size_t)stages * (2 * BM * 128 + 2 * b_bytes) + (size_t)raw * kRawSlotBytes + kStagingBytes + 1024 + 256;
+}
+
+// tensor map of A [M, K] for the raw ring: 128-row x 32-column boxes, 128-byte swizzle, rows past M zero-filled
+static int make_a_map(CUtensorMap* amap, const Nt16Args& g, const char* who) {
+    return make_tensor_map_2d(amap, g.A, g.M, g.K, BM, 32, true, who);
+}
+
+template <int BN, int STAGES, int RAW, int ACC>
 static int launch_nt16(const Nt16Args& g, cudaStream_t st) {
-    constexpr size_t smem = (size_t)STAGES * (2 * BM * 128 + 2 * BN * 128) + 1024 + 256 + kStagingBytes;
+    constexpr size_t smem = nt16_smem(STAGES, BN * 128, RAW);
     static_assert(smem <= 232448, "shared memory of the fp16-split NT kernel");
     static PerDeviceOnce configured;
     if (configured.need()) {
-        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_nt16_kernel<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)smem));
+        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_nt16_kernel<BN, STAGES, RAW, ACC>,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured.mark();
     }
     CUtensorMap cmap;                                    // result tensor [M, N], 32 x 32 boxes, 128-byte swizzle
     int rc = make_tensor_map_2d(&cmap, g.C, g.M, g.N, 32, 32, true, "tc_gemm_nt16");
     if (rc != DDMP_OK) return rc;
+    CUtensorMap amap = cmap;                             // unused by the register-fed configuration
+    if (RAW > 0 && (rc = make_a_map(&amap, g, "tc_gemm_nt16 A")) != DDMP_OK) return rc;
     const int64_t grid = g.num_tiles < kNumSMs ? g.num_tiles : kNumSMs;
-    tc_gemm_nt16_kernel<BN, STAGES><<<(unsigned)grid, kV2Threads, smem, st>>>(cmap, g);
+    tc_gemm_nt16_kernel<BN, STAGES, RAW, ACC><<<(unsigned)grid, kV2Threads, smem, st>>>(cmap, amap, g);
     return check_launch("tc_gemm_nt16");
 }
 
@@ -1133,11 +1319,11 @@ __device__ __forceinline__ void umma_f16_2cta(uint32_t tmem_d, uint64_t adesc, u
         : "memory");
 }
 
-constexpr int kNt16x2Stages = 3;
-
+// RAW = 0: A by the register-fed producers; RAW > 0: A by TMA into RAW raw slots (as in tc_gemm_nt16_kernel)
+template <int STAGES, int RAW>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kV2Threads, 1)
-tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const Nt16Args g) {
-    constexpr int STAGES = kNt16x2Stages;
+tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const __grid_constant__ CUtensorMap amap,
+                      const Nt16Args g) {
     constexpr int BN = 256;
     constexpr uint32_t A_BYTES = BM * 128;
     constexpr uint32_t B_HALF = (BN / 2) * 128;          // this CTA's half of the weight tile, one of hi / lo
@@ -1146,13 +1332,16 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const Nt16Args g
     constexpr uint32_t TMEM_COLS = 2 * BN;
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    uint8_t* staging = smem + STAGES * STAGE_BYTES;          // 1 KB aligned (128-byte swizzle of the tensor stores)
+    uint8_t* raw = smem + STAGES * STAGE_BYTES;              // RAW x 32 KB of fp32 A (1 KB aligned)
+    uint8_t* staging = raw + RAW * kRawSlotBytes;            // 1 KB aligned (128-byte swizzle of the tensor stores)
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(staging + kStagingBytes);
     uint64_t* empty_bar = full_bar + STAGES;
     uint64_t* peer_ready = empty_bar + STAGES;
     uint64_t* acc_full = peer_ready + STAGES;
     uint64_t* acc_empty = acc_full + 2;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
+    uint64_t* raw_full = acc_empty + 2;          // [RAW]
+    uint64_t* raw_empty = raw_full + RAW;        // [RAW]
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(raw_empty + RAW);
     uint32_t* amax_slot = tmem_slot + 1;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1168,6 +1357,10 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const Nt16Args g
         for (int b = 0; b < 2; ++b) {
             mbar_init(acc_full + b, 1);
             mbar_init(acc_empty + b, 8);
+        }
+        for (int r = 0; r < RAW; ++r) {
+            mbar_init(raw_full + r, 1);
+            mbar_init(raw_empty + r, kProducerWarps);
         }
         *amax_slot = 0u;
         fence_barrier_init();
@@ -1186,8 +1379,12 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const Nt16Args g
 
     if (warp < kProducerWarps) {
         auto wait_empty = [](uint64_t* bar, uint32_t parity) { mbar_wait_cluster(bar, parity); };
-        produce_loop<STAGES>(g, pair, num_pairs, (int64_t)(2 * BM), (int64_t)rank * BM, num_kb, s_a,
-                                        smem_base, STAGE_BYTES, A_BYTES, full_bar, empty_bar, wait_empty);
+        if constexpr (RAW > 0)
+            transform_loop<STAGES, RAW>(g, pair, num_pairs, num_kb, s_a, smem_base, smem_u32(raw), STAGE_BYTES, A_BYTES,
+                                        full_bar, empty_bar, raw_full, raw_empty, wait_empty);
+        else
+            produce_loop<STAGES>(g, pair, num_pairs, (int64_t)(2 * BM), (int64_t)rank * BM, num_kb, s_a,
+                                 smem_base, STAGE_BYTES, A_BYTES, full_bar, empty_bar, wait_empty);
     } else if (warp == 8) {
         if (lane == 0) {
             uint32_t it = 0, tile_no = 0;
@@ -1264,6 +1461,14 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const Nt16Args g
             }
         }
         __syncwarp();
+    } else if (warp == 10) {
+        // ===== A loader (RAW > 0): TMA tensor loads of this CTA's 128 rows into the raw ring =====
+        if constexpr (RAW > 0) {
+            if (lane == 0)
+                tma_a_loop<RAW>(g, &amap, pair, num_pairs, (int64_t)(2 * BM), (int64_t)rank * BM, num_kb, smem_u32(raw),
+                                raw_full, raw_empty);
+        }
+        __syncwarp();
     } else if (warp >= 12) {
         const int q = warp & 3;
         const uint32_t stg = smem_u32(staging) + (uint32_t)q * kStageWarpBytes;
@@ -1274,10 +1479,14 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const Nt16Args g
             const int64_t mrow0 = (tile / g.tiles_n) * (2 * BM) + rank * BM + q * 32;
             const int n0 = (int)(tile % g.tiles_n) * BN;
             const bool tr = g.trace && blockIdx.x == 0 && warp == 12 && lane == 0;
-            long long e0 = 0, e1 = 0;
+            long long e0 = 0;
             if (tr) e0 = clock64();
             mbar_wait_cluster(acc_full + buf, (tile_no >> 1) & 1u);
-            if (tr) e1 = clock64();
+            if (tr) {
+                const long long e1 = clock64();
+                g.trace[8] += (unsigned long long)(e1 - e0);                 // epilogue: wait accumulator
+                g.trace[9] -= (unsigned long long)e1;                        // epilogue: drain (completed below)
+            }
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + buf * BN;
             if (staged) epilogue_tile<BN>(g, taddr, inv_sa, stg, lane, mrow0, n0);
@@ -1285,8 +1494,7 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const Nt16Args g
             tc_fence_before();
             __syncwarp();
             if (tr) {
-                g.trace[8] += (unsigned long long)(e1 - e0);                 // epilogue: wait accumulator
-                g.trace[9] += (unsigned long long)(clock64() - e1);          // epilogue: drain
+                g.trace[9] += (unsigned long long)clock64();
                 g.trace[10] += 1ull;
             }
             if (lane == 0) {
@@ -1304,12 +1512,14 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const Nt16Args g
     }
 }
 
+template <int STAGES, int RAW>
 static int launch_nt16x2(const Nt16Args& g0, cudaStream_t st) {
-    constexpr size_t smem = (size_t)kNt16x2Stages * (2 * BM * 128 + 2 * 128 * 128) + 1024 + 256 + kStagingBytes;
+    constexpr size_t smem = nt16_smem(STAGES, 128 * 128, RAW);
     static_assert(smem <= 232448, "shared memory of the CTA-pair fp16-split NT kernel");
     static PerDeviceOnce configured;
     if (configured.need()) {
-        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_nt16x2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_nt16x2_kernel<STAGES, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)smem));
         configured.mark();
     }
     Nt16Args g = g0;
@@ -1317,13 +1527,17 @@ static int launch_nt16x2(const Nt16Args& g0, cudaStream_t st) {
     CUtensorMap cmap;                                    // result tensor [M, N], 32 x 32 boxes, 128-byte swizzle
     int rc = make_tensor_map_2d(&cmap, g.C, g.M, g.N, 32, 32, true, "tc_gemm_nt16x2");
     if (rc != DDMP_OK) return rc;
+    CUtensorMap amap = cmap;                             // unused by the register-fed configuration
+    if (RAW > 0 && (rc = make_a_map(&amap, g, "tc_gemm_nt16x2 A")) != DDMP_OK) return rc;
     const int64_t pairs = g.num_tiles < kNumSMs / 2 ? g.num_tiles : kNumSMs / 2;
-    tc_gemm_nt16x2_kernel<<<(unsigned)(2 * pairs), kV2Threads, smem, st>>>(cmap, g);
+    tc_gemm_nt16x2_kernel<STAGES, RAW><<<(unsigned)(2 * pairs), kV2Threads, smem, st>>>(cmap, amap, g);
     return check_launch("tc_gemm_nt16x2");
 }
 
 // switches of the fp16-split NT kernels (environment DDMP_TC_F16_FLAGS, ddmp_gemm_tc_flags): bit 0 = prefetch the next
-// tile's A rows into L2, bit 1 = the same for K <= 256 only, bit 3 = unstaged epilogue, bit 4 = staged ld.shared + st.global epilogue instead of TMA stores
+// tile's A rows into L2, bit 1 = the same for K <= 256 only, bit 3 = unstaged epilogue, bit 4 = staged ld.shared + st.global
+// epilogue instead of TMA stores, bit 5 = the previous configuration (register-fed A operand everywhere, CTA pairs for
+// every N % 256 == 0)
 int f16_flags(int set) {
     static std::atomic<int> v{-1};
     int cur = v.load(std::memory_order_relaxed);
@@ -1344,7 +1558,17 @@ static bool f16_split_enabled() {
 static int run_nt16(const float* A, const int* a_map, const float* scale, const float* shift, float slope,
                     const float* W, int transposed, void* workspace, float* C, int64_t M, int N, int K,
                     const float* amax, int64_t amax_len, cudaStream_t st) {
-    const int BN = (N % 256 == 0) ? 256 : ((N % 128 == 0) ? 128 : 64);
+    int flags = f16_flags(-1);
+    if ((flags & 2) && K <= 256) flags |= 1;         // bit 1: the L2 prefetch only where it measured faster (K <= 256)
+    // (TMA tensor coordinates are 32-bit: row counts near 2^31 keep the register-fed producers)
+    // TMA-fed A (DESIGN.md §4.2): at K <= 256, and at K = 512 when the BatchNorm + LeakyReLU prologue is fused (there
+    // the transform makes the register-fed producers the bound); without the prologue the producers keep pace at
+    // K = 512 and the raw ring's extra shared-memory traffic measured ~3 % slower.  The fused row gather (a_map) has
+    // no TMA tile form.
+    const bool tma_a = (K <= 256 || scale != nullptr) && a_map == nullptr && !(flags & 32) && M < (1ll << 31) - 2 * BM;
+    // N % 256 == 0 at K <= 128: a CTA pair's 128 x 256 tile has ~3 k cycles of MMA against 8-9 k cycles of drain, so
+    // 128-wide single-CTA tiles with the 4-deep accumulator ring are faster there (12-16 %); at K >= 256 the pair is faster
+    const int BN = (N % 256 == 0 && !(tma_a && K <= 128)) ? 256 : ((N % 128 == 0) ? 128 : 64);
     uint8_t* img = reinterpret_cast<uint8_t*>(workspace);
     float* inv_sw = reinterpret_cast<float*>(img + (int64_t)N * K * 4);          // after the hi + lo images
     tc_prep_b16_kernel<<<(unsigned)ceil_div((int64_t)N * 32, 256), 256, 0, st>>>(W, transposed, img, inv_sw, N, K, BN);
@@ -1353,8 +1577,7 @@ static int run_nt16(const float* A, const int* a_map, const float* scale, const 
     Nt16Args g{};
     g.A = A; g.Bimg = img; g.inv_sw = inv_sw; g.C = C; g.a_map = a_map; g.scale = scale; g.shift = shift;
     g.slope = slope; g.amax = amax; g.amax_len = amax_len;
-    g.flags = f16_flags(-1);
-    if ((g.flags & 2) && K <= 256) g.flags |= 1;     // bit 1: the L2 prefetch only where it measured faster (K <= 256)
+    g.flags = flags;
     static const bool trace = [] { const char* e = getenv("DDMP_TC_TRACE"); return e && e[0] == '1'; }();
     static unsigned long long* trace_buf = nullptr;
     if (trace) {
@@ -1367,13 +1590,15 @@ static int run_nt16(const float* A, const int* a_map, const float* scale, const 
             unsigned long long h[16];
             cudaStreamSynchronize(st);
             cudaMemcpy(h, trace_buf, sizeof(h), cudaMemcpyDeviceToHost);
-            fprintf(stderr, "[ddmp trace] M=%lld N=%d K=%d | producer/stage: issue %llu wait_free %llu data+store %llu (n=%llu) | "
-                    "mma/stage: wait_full %llu wait_peer %llu (n=%llu) wait_acc_total %llu | epilogue/tile: wait %llu drain %llu (n=%llu) "
-                    "[to staging %llu, to global %llu, tmem wait(1 of 2) %llu] producer detail: transform+stores %llu fence %llu\n",
-                    (long long)M, N, K, h[3] ? h[0] / h[3] : 0, h[3] ? h[1] / h[3] : 0, h[3] ? h[2] / h[3] : 0, h[3],
-                    h[6] ? h[4] / h[6] : 0, h[6] ? h[5] / h[6] : 0, h[6], h[7], h[10] ? h[8] / h[10] : 0,
-                    h[10] ? h[9] / h[10] : 0, h[10], h[10] ? h[11] / h[10] : 0, h[10] ? h[12] / h[10] : 0,
-                    h[10] ? h[13] / h[10] : 0, h[3] ? h[14] / h[3] : 0, h[3] ? h[15] / h[3] : 0);
+            // cycles of CTA 0 per k-block (producer thread 0, MMA thread, A loader) or per tile (epilogue warp 12)
+            auto per = [](unsigned long long x, unsigned long long n) { return n ? x / n : 0ull; };
+            fprintf(stderr, "[ddmp trace] M=%lld N=%d K=%d A=%s | producer/kb: wait_raw %llu wait_free %llu data+store %llu "
+                    "(n=%llu) [transform+stores %llu fence %llu] | tma_a/kb: wait_slot %llu | mma/kb: wait_full %llu "
+                    "wait_peer %llu (n=%llu) | mma/tile: wait_acc %llu | epilogue/tile: wait %llu drain %llu (n=%llu) "
+                    "[staged tmem wait %llu]\n",
+                    (long long)M, N, K, tma_a ? "tma" : "registers", per(h[11], h[3]), per(h[1], h[3]), per(h[2], h[3]),
+                    h[3], per(h[14], h[3]), per(h[15], h[3]), per(h[12], h[3]), per(h[4], h[6]), per(h[5], h[6]), h[6],
+                    per(h[7], h[10]), per(h[8], h[10]), per(h[9], h[10]), h[10], per(h[13], h[10]));
         }
         return rc;
     };
@@ -1381,10 +1606,15 @@ static int run_nt16(const float* A, const int* a_map, const float* scale, const 
     g.num_tiles = ceil_div(M, BM) * g.tiles_n;
     DDMP_REQUIRE(g.num_tiles < (1ll << 31), "tc gemm: too many tiles");
     static const bool one_cta = [] { const char* e = getenv("DDMP_TC_2CTA"); return e && e[0] == '0'; }();
-    if (BN == 256 && !one_cta) return dump_trace(launch_nt16x2(g, st));
-    if (BN == 256) return launch_nt16<256, 2>(g, st);
-    if (BN == 128) return launch_nt16<128, 3>(g, st);
-    return launch_nt16<64, 4>(g, st);
+    if (BN == 256 && one_cta) return dump_trace(launch_nt16<256, 2, 0, 2>(g, st));
+    if (tma_a) {                                     // one split stage traded for the raw fp32 slots
+        if (BN == 256) return dump_trace(launch_nt16x2<2, 2>(g, st));
+        if (BN == 128) return dump_trace(launch_nt16<128, 2, 2, 4>(g, st));
+        return dump_trace(launch_nt16<64, 2, 3, 4>(g, st));
+    }
+    if (BN == 256) return dump_trace(launch_nt16x2<3, 0>(g, st));
+    if (BN == 128) return dump_trace(launch_nt16<128, 3, 0, 2>(g, st));
+    return dump_trace(launch_nt16<64, 4, 0, 2>(g, st));
 }
 
 // ---- TN kernel (dW) -------------------------------------------------------------------------------------------------
