@@ -21,19 +21,23 @@ static inline unsigned loss_grid(int64_t count) {
     return (unsigned)g;
 }
 
-// finish a scalar reduction: returns true in thread 0 of the last block with the total in `total`
-__device__ __forceinline__ bool finish_sum(double local, LossScratch* sc, double& total) {
+// finish a scalar reduction over blocks blk = 0..nblk-1: returns true in thread 0 of the last block with the total in
+// `total`
+__device__ __forceinline__ bool finish_sum_of(double local, LossScratch* sc, double& total, unsigned blk, unsigned nblk) {
     __shared__ double sm[kLossThreads / 32];
     const double b = block_sum<kLossThreads>(local, sm);
-    if (threadIdx.x == 0) sc->partials[blockIdx.x] = b;
-    const bool last = publish_and_am_last(&sc->ticket, gridDim.x);
+    if (threadIdx.x == 0) sc->partials[blk] = b;
+    const bool last = publish_and_am_last(&sc->ticket, nblk);
     if (last && threadIdx.x == 0) {
         double t = 0.0;
-        for (unsigned i = 0; i < gridDim.x; ++i) t += __ldcg(&sc->partials[i]);
+        for (unsigned i = 0; i < nblk; ++i) t += __ldcg(&sc->partials[i]);
         total = t;
         return true;
     }
     return false;
+}
+__device__ __forceinline__ bool finish_sum(double local, LossScratch* sc, double& total) {
+    return finish_sum_of(local, sc, total, blockIdx.x, gridDim.x);
 }
 
 #define GRID_STRIDE(i, count) \
@@ -438,29 +442,101 @@ grad_norm_kernel(const float* __restrict__ g, float* norm_out, LossScratch* sc, 
 
 __global__ void counter_increment_kernel(int64_t* counter) { *counter += 1; }
 
+__device__ __forceinline__ void adam_bias_corrections(const int64_t* step_dev, float beta1, float beta2, float& bc1,
+                                                      float& bc2_sqrt) {
+    const double t = (double)*step_dev;
+    bc1 = (float)(1.0 - pow((double)beta1, t));
+    bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, t));
+}
+
+__device__ __forceinline__ float clip_coef(float norm, float max_norm) {
+    const float coef = max_norm / (norm + 1.0e-6f);
+    return coef > 1.f ? 1.f : coef;
+}
+
+__device__ __forceinline__ void adam_element(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
+                                             float* __restrict__ v, int64_t i, float coef, float beta1, float beta2,
+                                             float eps, float step_size, float bc2_sqrt) {
+    const float gi = g[i] * coef;
+    const float mi = m[i] + (gi - m[i]) * (1.f - beta1);      // torch lerp_
+    const float vi = beta2 * v[i] + (1.f - beta2) * gi * gi;
+    m[i] = mi; v[i] = vi;
+    const float denom = sqrtf(vi) / bc2_sqrt + eps;
+    p[i] -= step_size * (mi / denom);
+}
+
 __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                             float* __restrict__ v, const float* __restrict__ clip_norm, float max_norm, float lr,
                             float beta1, float beta2, float eps, float bc1, float bc2_sqrt,
                             const int64_t* __restrict__ step_dev, int64_t count) {
-    if (step_dev) {   // step count lives on the device (CUDA-graph replay: kernel arguments are frozen)
-        const double t = (double)*step_dev;
-        bc1 = (float)(1.0 - pow((double)beta1, t));
-        bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, t));
-    }
-    float coef = 1.f;
-    if (clip_norm) {
-        coef = max_norm / (*clip_norm + 1.0e-6f);
-        coef = coef > 1.f ? 1.f : coef;
-    }
+    // step count lives on the device (CUDA-graph replay: kernel arguments are frozen)
+    if (step_dev) adam_bias_corrections(step_dev, beta1, beta2, bc1, bc2_sqrt);
+    const float coef = clip_norm ? clip_coef(*clip_norm, max_norm) : 1.f;
     const float step_size = lr / bc1;
-    GRID_STRIDE(i, count) {
-        const float gi = g[i] * coef;
-        const float mi = m[i] + (gi - m[i]) * (1.f - beta1);      // torch lerp_
-        const float vi = beta2 * v[i] + (1.f - beta2) * gi * gi;
-        m[i] = mi; v[i] = vi;
-        const float denom = sqrtf(vi) / bc2_sqrt + eps;
-        p[i] -= step_size * (mi / denom);
-    }
+    GRID_STRIDE(i, count) adam_element(p, g, m, v, i, coef, beta1, beta2, eps, step_size, bc2_sqrt);
+}
+
+// ---- the optimizer of many networks over one flat buffer (ddmp_*_segments) -------------------------------------------
+// Segment s (a network) is row s of the table: DDMP_SEGMENT_WORDS int64 words, see include/ddmp_b200.h.  blockIdx.y is
+// the segment; a segment uses the blocks x < loss_grid(count) -- the grid its stand-alone call would launch -- and the
+// other blocks of its row return at once.
+struct Segment {
+    int64_t off, count;
+    bool clip;
+    float lr, max_norm;
+};
+__device__ __forceinline__ Segment load_segment(const int64_t* __restrict__ table, int s) {
+    const int64_t* w = table + (int64_t)s * DDMP_SEGMENT_WORDS;
+    Segment g;
+    g.off = w[0]; g.count = w[1]; g.clip = w[2] != 0;
+    g.lr = __uint_as_float((unsigned)(w[3] & 0xffffffffll));
+    g.max_norm = __uint_as_float((unsigned)(w[4] & 0xffffffffll));
+    return g;
+}
+__device__ __forceinline__ unsigned loss_grid_dev(int64_t count) {
+    int64_t g = (count + kLossThreads - 1) / kLossThreads;
+    if (g > 4 * kNumSMs) g = 4 * kNumSMs;
+    if (g < 1) g = 1;
+    return (unsigned)g;
+}
+
+__global__ void __launch_bounds__(kLossThreads)
+grad_norm_segments_kernel(const float* __restrict__ flat, const int64_t* __restrict__ table, float* norms,
+                          LossScratch* sc) {
+    const Segment sg = load_segment(table, blockIdx.y);
+    const unsigned nblk = loss_grid_dev(sg.count);
+    if (!sg.clip || blockIdx.x >= nblk) return;
+    const float* __restrict__ g = flat + sg.off;
+    double acc = 0.0;
+    for (int64_t i = (int64_t)blockIdx.x * kLossThreads + threadIdx.x; i < sg.count; i += (int64_t)nblk * kLossThreads)
+        acc += (double)g[i] * (double)g[i];
+    double tot;
+    if (finish_sum_of(acc, sc + blockIdx.y, tot, blockIdx.x, nblk)) norms[blockIdx.y] = (float)sqrt(tot);
+}
+
+__global__ void adam_segments_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
+                                     float* __restrict__ v, const int64_t* __restrict__ table,
+                                     const float* __restrict__ norms, float beta1, float beta2, float eps,
+                                     const int64_t* __restrict__ step_dev) {
+    const Segment sg = load_segment(table, blockIdx.y);
+    const unsigned nblk = loss_grid_dev(sg.count);
+    if (blockIdx.x >= nblk) return;
+    float bc1, bc2_sqrt;
+    adam_bias_corrections(step_dev, beta1, beta2, bc1, bc2_sqrt);
+    const float coef = sg.clip ? clip_coef(norms[blockIdx.y], sg.max_norm) : 1.f;
+    const float step_size = sg.lr / bc1;
+    for (int64_t i = sg.off + (int64_t)blockIdx.x * kLossThreads + threadIdx.x; i < sg.off + sg.count;
+         i += (int64_t)nblk * kLossThreads)
+        adam_element(p, g, m, v, i, coef, beta1, beta2, eps, step_size, bc2_sqrt);
+}
+
+// row s of the table: (source address, destination offset, count); blockIdx.y is the row
+__global__ void __launch_bounds__(256) gather_table_kernel(const int64_t* __restrict__ table, float* __restrict__ dst) {
+    const int64_t* w = table + 3 * (int64_t)blockIdx.y;
+    const float* __restrict__ src = reinterpret_cast<const float*>(w[0]);
+    float* __restrict__ out = dst + w[1];
+    const int64_t cnt = w[2];
+    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < cnt; i += (int64_t)gridDim.x * 256) out[i] = src[i];
 }
 
 // see ddmp_gather_flat
@@ -721,6 +797,40 @@ int ddmp_gather_flat(const void* const* srcs, const int64_t* offsets, const int6
         if (rc != DDMP_OK) return rc;
     }
     return DDMP_OK;
+}
+
+int ddmp_gather_table(const int64_t* table, int32_t n_src, int64_t longest, float* dst, void* stream) {
+    using namespace ddmp;
+    DDMP_REQUIRE(table && dst && n_src >= 0 && n_src <= 65535 && longest >= 0, "gather_table: bad arguments");
+    if (n_src == 0 || longest == 0) return DDMP_OK;
+    int64_t bx = ceil_div(longest, 256 * 4);
+    if (bx > 64) bx = 64;
+    gather_table_kernel<<<dim3((unsigned)bx, (unsigned)n_src), 256, 0, as_stream(stream)>>>(table, dst);
+    return check_launch("gather_table");
+}
+
+int ddmp_grad_norm_segments(const float* flat, const int64_t* table, int32_t n_seg, int64_t longest, float* norms,
+                            void* scratch, void* stream) {
+    using namespace ddmp;
+    DDMP_REQUIRE(flat && table && norms && scratch && n_seg > 0 && n_seg <= 65535 && longest > 0,
+                 "grad_norm_segments: bad arguments");
+    grad_norm_segments_kernel<<<dim3(loss_grid(longest), (unsigned)n_seg), kLossThreads, 0, as_stream(stream)>>>(
+        flat, table, norms, (LossScratch*)scratch);
+    return check_launch("grad_norm_segments");
+}
+
+int ddmp_adam_segments(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, const int64_t* table,
+                       int32_t n_seg, int64_t longest, const float* norms, float beta1, float beta2, float eps,
+                       int64_t* step_counter, void* stream) {
+    using namespace ddmp;
+    DDMP_REQUIRE(param && grad && exp_avg && exp_avg_sq && table && norms && step_counter && n_seg > 0 &&
+                     n_seg <= 65535 && longest > 0, "adam_segments: bad arguments");
+    counter_increment_kernel<<<1, 1, 0, as_stream(stream)>>>(step_counter);
+    int rc = check_launch("adam_segments(counter)");
+    if (rc) return rc;
+    adam_segments_kernel<<<dim3(loss_grid(longest), (unsigned)n_seg), kLossThreads, 0, as_stream(stream)>>>(
+        param, grad, exp_avg, exp_avg_sq, table, norms, beta1, beta2, eps, step_counter);
+    return check_launch("adam_segments");
 }
 
 }  // extern "C"

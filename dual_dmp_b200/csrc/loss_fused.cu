@@ -78,8 +78,8 @@ __device__ __forceinline__ Tri3 load_tri3(const float* __restrict__ pos, const i
     return t;
 }
 
-// block partial of `local` -> partials[slot][blockIdx.x]
-__device__ __forceinline__ void publish(double local, double* partials, int slot, double* sm) {
+// block partial of `local` -> partials[slot][blk]  (blk: the block's index among the blocks of its mesh)
+__device__ __forceinline__ void publish(double local, double* partials, int slot, double* sm, unsigned blk) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) local += __shfl_down_sync(0xffffffffu, local, o);
     if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5] = local;
@@ -88,7 +88,7 @@ __device__ __forceinline__ void publish(double local, double* partials, int slot
         double r = 0.0;
 #pragma unroll
         for (int i = 0; i < kT / 32; ++i) r += sm[i];
-        partials[slot * kMaxBlocks + blockIdx.x] = r;
+        partials[slot * kMaxBlocks + blk] = r;
     }
     __syncthreads();
 }
@@ -96,11 +96,11 @@ __device__ __forceinline__ void publish(double local, double* partials, int slot
 // sum of all blocks' partials of `slot`, identical in every thread of every block: lane l of warp 0 adds the partials
 // l, l+32, l+64, ... in ascending order, the 32 lane sums are folded by a fixed shuffle tree.  (One thread adding the
 // ~600 partials in a dependent chain of L2 loads and DADDs took ~15 us per scalar -- six scalars = 30 % of the kernel.)
-__device__ __forceinline__ double total(const double* partials, int slot, double* sm) {
+__device__ __forceinline__ double total(const double* partials, int slot, double* sm, unsigned nblk) {
     if (threadIdx.x < 32) {
         const double* p = partials + slot * kMaxBlocks;
         double r = 0.0;
-        for (unsigned i = threadIdx.x; i < gridDim.x; i += 32) r += __ldcg(p + i);
+        for (unsigned i = threadIdx.x; i < nblk; i += 32) r += __ldcg(p + i);
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) r += __shfl_xor_sync(0xffffffffu, r, o);
         if (threadIdx.x == 0) sm[0] = r;
@@ -126,12 +126,29 @@ constexpr float kSigmaS2 = 0.09f;
 
 #define STRIDE_LOOP(i, count) for (int64_t i = tid; i < (count); i += nth)
 
-__global__ void __launch_bounds__(kT, 4)
-dual_loss_kernel(const Args a) {
-    cg::grid_group grid = cg::this_grid();
-    __shared__ double sm[kT / 32];
-    const int64_t tid = (int64_t)blockIdx.x * kT + threadIdx.x;
-    const int64_t nth = (int64_t)gridDim.x * kT;
+// The loss phase of one mesh, run by `nblk` blocks of a cooperative grid; `blk` is the block's index among them.  The
+// stand-alone kernel gives a mesh the whole grid; the batched kernel gives each mesh the block range its stand-alone
+// launch would have, so the arithmetic, the grid-stride partition and the order of every sum are the same.  Every block
+// of the grid calls grid.sync() the same number of times (it depends on `loop` only).
+// `Range` supplies blk() / nblk(); both are re-read where used (special registers, shared memory) rather than kept live.
+struct WholeGrid {
+    __device__ __forceinline__ unsigned blk() const { return blockIdx.x; }
+    __device__ __forceinline__ unsigned nblk() const { return gridDim.x; }
+};
+__shared__ unsigned s_range[2];          // batched kernel: the block's index within its mesh, the mesh's block count
+struct MeshRange {
+    __device__ __forceinline__ unsigned blk() const { return s_range[0]; }
+    __device__ __forceinline__ unsigned nblk() const { return s_range[1]; }
+};
+
+// ArgT: `const Args` (the stand-alone kernel's parameter, read in place) or `const Args&` (the batched kernel's copy in
+// shared memory).
+template <class Range, class ArgT>
+__device__ __forceinline__ void dual_loss_body(ArgT a, cg::grid_group& grid, const Range rg, double* sm) {
+#define blk rg.blk()
+#define nblk rg.nblk()
+    const int64_t tid = (int64_t)blk * kT + threadIdx.x;
+    const int64_t nth = (int64_t)nblk * kT;
     const int64_t V = a.V, F = a.F;
     const int loop = a.loop;
 
@@ -216,17 +233,17 @@ dual_loss_kernel(const Args a) {
             }
         }
         stamp(2);
-        publish(acc_pr, a.partials, 0, sm);
-        publish(acc_lap, a.partials, 1, sm);
-        publish(acc_nr, a.partials, 2, sm);
-        publish(acc_pn, a.partials, 3, sm);
+        publish(acc_pr, a.partials, 0, sm, blk);
+        publish(acc_lap, a.partials, 1, sm, blk);
+        publish(acc_nr, a.partials, 2, sm, blk);
+        publish(acc_pn, a.partials, 3, sm, blk);
     }
     grid.sync();
     stamp(3);
-    const double l1 = sqrt(total(a.partials, 0, sm) / (double)V + 1.0e-6);
-    const float l2 = (float)sqrt(total(a.partials, 1, sm) / (double)V + 1.0e-12);
-    const double l3 = total(a.partials, 2, sm) / (double)F;
-    const float l5 = (float)(total(a.partials, 3, sm) / (double)V);
+    const double l1 = sqrt(total(a.partials, 0, sm, nblk) / (double)V + 1.0e-6);
+    const float l2 = (float)sqrt(total(a.partials, 1, sm, nblk) / (double)V + 1.0e-12);
+    const double l3 = total(a.partials, 2, sm, nblk) / (double)F;
+    const float l5 = (float)(total(a.partials, 3, sm, nblk) / (double)V);
 
     // ================= P2 =================================================================================
     stamp(4);
@@ -292,13 +309,13 @@ dual_loss_kernel(const Args a) {
             }
         }
         stamp(6);
-        publish(acc_sig, a.partials, 4, sm);
+        publish(acc_sig, a.partials, 4, sm, blk);
     }
     float l4 = 0.f;
     if (loop > 0) {
         grid.sync();
         stamp(7);
-        const float sg = (float)(total(a.partials, 4, sm) / (double)(3 * F));
+        const float sg = (float)(total(a.partials, 4, sm, nblk) / (double)(3 * F));
         const float den = 2.0f * (sg * sg);
         const float kb = (a.k[3] * a.bnf_scale) / (float)F;        // gout / F of the bnf L1 term
 
@@ -346,7 +363,7 @@ dual_loss_kernel(const Args a) {
             }
         }
         stamp(8);
-        publish(acc_bnf, a.partials, 5, sm);
+        publish(acc_bnf, a.partials, 5, sm, blk);
 
         // ================= P4: backward of the iterations ===================================================
         for (int t = loop - 1; t >= 0; --t) {
@@ -412,10 +429,10 @@ dual_loss_kernel(const Args a) {
             }
         }
         stamp(11);
-        l4 = (float)(total(a.partials, 5, sm) / (double)F);
+        l4 = (float)(total(a.partials, 5, sm, nblk) / (double)F);
     }
     stamp(12);
-    if (blockIdx.x == 0 && threadIdx.x == 0) {
+    if (blk == 0 && threadIdx.x == 0) {
         const float l4s = l4 * a.bnf_scale;                      // `loss_norm2 * 0.0` while epoch <= 100 (main.py:101)
         a.losses[0] = l1; a.losses[1] = (double)l2; a.losses[2] = l3; a.losses[3] = (double)l4s; a.losses[4] = (double)l5;
         // python: k1*l1 (f64) + k2*l2 (f32) + k3*l3 (f64) + k4*l4 (f32) + k5*l5 (f32), left to right
@@ -426,21 +443,103 @@ dual_loss_kernel(const Args a) {
         tot += (double)(a.k[4] * l5);
         a.losses[5] = tot;
     }
+#undef blk
+#undef nblk
 }
 
-static int grid_blocks() {
-    static int cached[64] = {0};
+__global__ void __launch_bounds__(kT, 4)
+dual_loss_kernel(const Args a) {
+    cg::grid_group grid = cg::this_grid();
+    __shared__ double sm[kT / 32];
+    dual_loss_body<WholeGrid, const Args>(a, grid, WholeGrid{}, sm);
+}
+
+// Workspace layout of one mesh (ddmp_dual_loss_workspace_bytes): the same for the stand-alone and the batched kernel.
+__host__ __device__ inline void carve_workspace(Args& a, void* workspace, int64_t V, int64_t F, int loop) {
+    float* w = static_cast<float*>(workspace);
+    w += (4 - ((reinterpret_cast<uintptr_t>(w) / 4) & 3)) & 3;       // 16-byte records first
+    a.ds = w; w += 4 * V;
+    a.face_tmp = w; w += 12 * F;
+    a.d = w; w += 3 * V;
+    a.fc = w; w += 3 * F;
+    a.fa = w; w += F;
+    a.wca = w; w += 3 * F;
+    a.normals = w; w += (int64_t)(loop > 0 ? loop : 1) * 3 * F;
+    a.g_last = w; w += 3 * F;
+    a.g = w; w += 3 * F;
+    a.msg = w; w += 18 * F;
+    const int64_t off = (((w - static_cast<float*>(workspace)) * 4 + 15) / 16) * 16;
+    a.partials = reinterpret_cast<double*>(static_cast<char*>(workspace) + off);
+}
+
+__host__ __device__ inline int64_t mesh_blocks(int64_t V, int64_t F, int g_single) {
+    const int64_t want = (((V > F) ? V : F) + kT - 1) / kT;
+    return want < g_single ? want : g_single;
+}
+
+// B meshes in one cooperative grid: mesh m owns mesh_blocks(V_m, F_m) consecutive blocks, in table order.  Thread 0 of
+// each block finds its mesh and unpacks the descriptor (include/ddmp_b200.h, DDMP_DUAL_LOSS_DESC_WORDS) into shared
+// memory; the meshes share the barriers, which is what makes one launch of all of them possible.
+__global__ void __launch_bounds__(kT, 4)
+dual_loss_multi_kernel(const int64_t* __restrict__ table, int n_mesh, int g_single, float bnf_scale, int loop) {
+    cg::grid_group grid = cg::this_grid();
+    __shared__ double sm[kT / 32];
+    __shared__ Args sa;
+    if (threadIdx.x == 0) {
+        int start = 0, m = 0, b = 0;
+        for (; m < n_mesh; ++m) {
+            const int64_t* d = table + (int64_t)m * DDMP_DUAL_LOSS_DESC_WORDS;
+            b = (int)mesh_blocks(d[15], d[16], g_single);
+            if ((int)blockIdx.x < start + b) break;
+            start += b;
+        }
+        const int64_t* d = table + (int64_t)m * DDMP_DUAL_LOSS_DESC_WORDS;
+        Args a{};
+        a.pos = reinterpret_cast<const float*>(d[0]);
+        a.nrm = reinterpret_cast<const float*>(d[1]);
+        a.tgt_vs = reinterpret_cast<const double*>(d[2]);
+        a.tgt_fn = reinterpret_cast<const double*>(d[3]);
+        a.faces = reinterpret_cast<const int*>(d[4]);
+        a.f2f = reinterpret_cast<const int*>(d[5]);
+        a.rslot = reinterpret_cast<const int*>(d[6]);
+        a.lap_rowptr = reinterpret_cast<const int*>(d[7]);
+        a.lap_col = reinterpret_cast<const int*>(d[8]);
+        a.corner_ptr = reinterpret_cast<const int*>(d[9]);
+        a.corner_slot = reinterpret_cast<const int*>(d[10]);
+        a.V = d[15]; a.F = d[16];
+        carve_workspace(a, reinterpret_cast<void*>(d[11]), a.V, a.F, loop);
+        a.gpos = reinterpret_cast<float*>(d[12]);
+        a.gnrm = reinterpret_cast<float*>(d[13]);
+        a.losses = reinterpret_cast<double*>(d[14]);
+#pragma unroll
+        for (int i = 0; i < 5; ++i) a.k[i] = __uint_as_float((unsigned)(d[17 + i] & 0xffffffffll));
+        a.loop = loop;
+        a.bnf_scale = bnf_scale;
+        sa = a;
+        s_range[0] = blockIdx.x - (unsigned)start;
+        s_range[1] = b;
+    }
+    __syncthreads();
+    dual_loss_body<MeshRange, const Args&>(sa, grid, MeshRange{}, sm);
+}
+
+static int occupancy_blocks(const void* kernel) {
+    int per_sm = 0, sms = 0, dev = 0;
+    cudaGetDevice(&dev);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kT, 0);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    int v = per_sm * sms;
+    if (v > kMaxBlocks) v = kMaxBlocks;
+    return v > 0 ? v : 1;
+}
+
+// blocks per cooperative launch: of the stand-alone kernel (batched = 0) and of the batched kernel (batched = 1)
+static int grid_blocks(int batched = 0) {
+    static int cached[2][64] = {{0}};
     int dev = 0;
     cudaGetDevice(&dev);
-    int& g = cached[dev & 63];
-    if (g == 0) {
-        int per_sm = 0, sms = 0;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, dual_loss_kernel, kT, 0);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        int v = per_sm * sms;
-        if (v > kMaxBlocks) v = kMaxBlocks;
-        g = v > 0 ? v : 1;
-    }
+    int& g = cached[batched ? 1 : 0][dev & 63];
+    if (g == 0) g = occupancy_blocks(batched ? (const void*)dual_loss_multi_kernel : (const void*)dual_loss_kernel);
     return g;
 }
 
@@ -481,27 +580,12 @@ int ddmp_dual_loss(const float* pos, const float* nrm, const double* tgt_vs, con
     Args a{};
     a.pos = pos; a.nrm = nrm; a.tgt_vs = tgt_vs; a.tgt_fn = tgt_fn; a.faces = faces; a.f2f = f2f; a.rslot = rslot;
     a.lap_rowptr = lap_rowptr; a.lap_col = lap_col; a.corner_ptr = corner_ptr; a.corner_slot = corner_slot;
-    float* w = static_cast<float*>(workspace);
-    w += (4 - ((reinterpret_cast<uintptr_t>(w) / 4) & 3)) & 3;       // 16-byte records first
-    a.ds = w; w += 4 * V;
-    a.face_tmp = w; w += 12 * F;
-    a.d = w; w += 3 * V;
-    a.fc = w; w += 3 * F;
-    a.fa = w; w += F;
-    a.wca = w; w += 3 * F;
-    a.normals = w; w += (int64_t)(loop > 0 ? loop : 1) * 3 * F;
-    a.g_last = w; w += 3 * F;
-    a.g = w; w += 3 * F;
-    a.msg = w; w += 18 * F;
-    const int64_t off = (((w - static_cast<float*>(workspace)) * 4 + 15) / 16) * 16;
-    a.partials = reinterpret_cast<double*>(static_cast<char*>(workspace) + off);
+    carve_workspace(a, workspace, V, F, loop);
     a.gpos = gpos; a.gnrm = gnrm; a.losses = losses;
     a.V = V; a.F = F; a.loop = loop;
     a.k[0] = k1; a.k[1] = k2; a.k[2] = k3; a.k[3] = k4; a.k[4] = k5;
     a.bnf_scale = bnf_scale;
-    int blocks = grid_blocks();
-    const int64_t want = ceil_div(V > F ? V : F, kT);
-    if (want < blocks) blocks = (int)want;
+    const int blocks = (int)mesh_blocks(V, F, grid_blocks());
     void* params[] = {&a};
     cudaError_t e = cudaLaunchCooperativeKernel((const void*)dual_loss_kernel, dim3((unsigned)blocks), dim3(kT), params, 0,
                                                 as_stream(stream));
@@ -510,6 +594,34 @@ int ddmp_dual_loss(const float* pos, const float* nrm, const double* tgt_vs, con
         return DDMP_ERR_CUDA;
     }
     return check_launch("dual_loss");
+}
+
+int64_t ddmp_dual_loss_grid(int32_t batched) { return ddmp::fusedloss::grid_blocks(batched); }
+
+int ddmp_dual_loss_multi(const int64_t* table, const int64_t* vf, int32_t n_mesh, float bnf_scale, int32_t loop,
+                         void* stream) {
+    using namespace ddmp;
+    using namespace ddmp::fusedloss;
+    DDMP_REQUIRE(table && vf && n_mesh > 0 && loop >= 0, "dual_loss_multi: bad arguments n_mesh=%d loop=%d", n_mesh,
+                 loop);
+    const int g_single = grid_blocks(0);
+    int64_t blocks = 0;
+    for (int m = 0; m < n_mesh; ++m) {
+        DDMP_REQUIRE(vf[2 * m] > 0 && vf[2 * m + 1] > 0, "dual_loss_multi: mesh %d has V=%lld F=%lld", m,
+                     (long long)vf[2 * m], (long long)vf[2 * m + 1]);
+        blocks += mesh_blocks(vf[2 * m], vf[2 * m + 1], g_single);
+    }
+    DDMP_REQUIRE(blocks <= grid_blocks(1), "dual_loss_multi: %lld blocks exceed one cooperative launch (%d)",
+                 (long long)blocks, grid_blocks(1));
+    int n = n_mesh, gs = g_single;
+    void* params[] = {(void*)&table, &n, &gs, &bnf_scale, &loop};
+    cudaError_t e = cudaLaunchCooperativeKernel((const void*)dual_loss_multi_kernel, dim3((unsigned)blocks), dim3(kT),
+                                                params, 0, as_stream(stream));
+    if (e != cudaSuccess) {
+        set_error("dual_loss_multi: cooperative launch failed: %s", cudaGetErrorString(e));
+        return DDMP_ERR_CUDA;
+    }
+    return check_launch("dual_loss_multi");
 }
 
 }  // extern "C"

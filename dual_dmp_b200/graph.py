@@ -153,6 +153,9 @@ class GcnGraph:
 
 
 _graph_cache: dict = {}
+# graphs a caller holds on to (pin_graphs): looked up after the cache, never evicted by it.  A batch of fits asks for
+# more graphs than the cache keeps, and rebuilding one inside CUDA-graph capture would fail.
+_pinned: dict = {}
 
 
 def graph_for(edge_index: torch.Tensor, num_nodes: int, device, coords=None, reorder: bool = True) -> GcnGraph:
@@ -163,11 +166,30 @@ def graph_for(edge_index: torch.Tensor, num_nodes: int, device, coords=None, reo
     hit = _graph_cache.get(key)
     if hit is not None and hit[0] is edge_index:
         return hit[1]
+    hit = _pinned.get(key)
+    if hit is not None and hit[0] is edge_index:
+        return hit[1]
     g = GcnGraph(edge_index, num_nodes, device, coords=coords, reorder=reorder)
+    g.cache_key = key
     if len(_graph_cache) > 64:
         _graph_cache.clear()
     _graph_cache[key] = (edge_index, g)
     return g
+
+
+def pin_graphs(pairs) -> list:
+    """Keep each (edge_index, graph) -- a graph as ``graph_for(edge_index, ...)`` returned it -- reachable by
+    ``graph_for`` until ``unpin_graphs`` of the returned keys."""
+    keys = []
+    for edge_index, g in pairs:
+        _pinned[g.cache_key] = (edge_index, g)
+        keys.append(g.cache_key)
+    return keys
+
+
+def unpin_graphs(keys) -> None:
+    for k in keys:
+        _pinned.pop(k, None)
 
 
 class MeshTopology:

@@ -13,6 +13,7 @@ from __future__ import annotations
 
 import copy
 
+import numpy as np
 import torch
 
 from .util import loss as L
@@ -227,3 +228,167 @@ class FusedAdam:
         lib.call("ddmp_adam_step_dev", ptr(self.flat), ptr(g), ptr(self.exp_avg), ptr(self.exp_avg_sq), ptr(clip),
                  float(self.max_norm or 0.0), self.lr, self.betas[0], self.betas[1], self.eps, ptr(self.step_count),
                  g.numel(), st)
+
+
+class GroupFusedAdam:
+    """``FusedAdam`` of many networks over ONE flat buffer: gather, clip norms and Adam are one library launch each for
+    all of them (``ddmp_gather_table``, ``ddmp_grad_norm_segments``, ``ddmp_adam_segments``), with a per-network lr and
+    clip.  Network ``i`` is segment ``i``; its results equal a ``FusedAdam`` of that network bit for bit.  Parameters are
+    re-pointed at views of the flat buffer, so ``parameters()`` / ``state_dict()`` keep working."""
+
+    def __init__(self, modules, lrs, max_norms, betas=(0.9, 0.999), eps=1e-8):
+        from ._lib import lib
+        from . import multi
+        self.params = [[p for p in m.parameters() if p.requires_grad] for m in modules]
+        flat_params = [p for ps in self.params for p in ps]
+        dev = flat_params[0].device
+        if dev.type != "cuda":
+            raise RuntimeError("GroupFusedAdam runs on CUDA only (dual_dmp_b200 has no CPU path)")
+        if any(p.device != dev for p in flat_params):
+            raise ValueError("GroupFusedAdam: every network must be on one device")
+        self.counts = [sum(p.numel() for p in ps) for ps in self.params]
+        self.offsets, total = multi.segment_offsets(self.counts)
+        self.flat = torch.zeros(total, dtype=torch.float32, device=dev)
+        gather = []
+        for ps, off in zip(self.params, self.offsets):
+            for p in ps:
+                k = p.numel()
+                self.flat[off: off + k].copy_(p.detach().reshape(-1))
+                p.data = self.flat[off: off + k].view_as(p)
+                gather.append((off, k))
+                off += k
+        self._gather_rows = np.array(gather, dtype=np.int64)
+        self._longest_param = max(k for _, k in gather)
+        self.gflat = torch.zeros_like(self.flat)
+        self.exp_avg = torch.zeros_like(self.flat)
+        self.exp_avg_sq = torch.zeros_like(self.flat)
+        self.step_count = torch.zeros((), dtype=torch.int64, device=dev)
+        n = len(self.params)
+        clip = [m is not None for m in max_norms]
+        seg = multi.segment_table(self.counts, clip, lrs, [m or 0.0 for m in max_norms])
+        self.segments = torch.from_numpy(seg).to(dev)          # no addresses in it: written once
+        self.clips = any(clip)
+        self.norms = torch.zeros(n, dtype=torch.float32, device=dev)
+        self.scratch = torch.zeros(n * int(lib.query("ddmp_loss_scratch_bytes")) // 8 + 1, dtype=torch.float64,
+                                   device=dev)
+        self.betas, self.eps, self.device = betas, float(eps), dev
+
+    def segment(self, i: int) -> slice:
+        """the slice of network ``i`` in ``flat`` / ``exp_avg`` / ``exp_avg_sq``"""
+        return slice(self.offsets[i], self.offsets[i] + self.counts[i])
+
+    def zero_grad(self, set_to_none=True):
+        for ps in self.params:
+            for p in ps:
+                p.grad = None
+
+    def step(self, tables):
+        """``tables``: the ``multi.DeviceTables`` that holds the gradient-address table of this iteration"""
+        from ._lib import lib, ptr, set_device, stream_ptr
+        set_device(self.device)
+        st = stream_ptr(self.device)
+        grads = [p.grad if p.grad.is_contiguous() else p.grad.contiguous() for ps in self.params for p in ps]
+        rows = np.concatenate([np.array([[g.data_ptr()] for g in grads], dtype=np.int64), self._gather_rows], axis=1)
+        table = tables.put("grads", rows)
+        lib.call("ddmp_gather_table", ptr(table), len(grads), self._longest_param, ptr(self.gflat), st)
+        n, longest = len(self.counts), max(self.counts)
+        if self.clips:
+            lib.call("ddmp_grad_norm_segments", ptr(self.gflat), ptr(self.segments), n, longest, ptr(self.norms),
+                     ptr(self.scratch), st)
+        lib.call("ddmp_adam_segments", ptr(self.flat), ptr(self.gflat), ptr(self.exp_avg), ptr(self.exp_avg_sq),
+                 ptr(self.segments), n, longest, ptr(self.norms), self.betas[0], self.betas[1], self.eps,
+                 ptr(self.step_count), st)
+
+
+class MultiDualStep(DualStep):
+    """``DualStep`` of B independent fits on one GPU as one iteration: each fit's PosNet and NormalNet forward on a
+    stream pair of its own, one batched loss phase (``multi.DualLossMulti``), the backward passes (autograd runs each
+    network's on the stream of its forward) and one batched optimizer (``GroupFusedAdam``); captured into one CUDA graph
+    per phase like ``DualStep``.  Every fit's numbers equal those of its own ``DualStep`` bit for bit.
+
+    ``fits``: one dict per mesh with ``posnet``, ``normnet``, ``dataset``, ``n_mesh`` and optionally ``k``, ``pos_lr``,
+    ``norm_lr``, ``grad_clip`` and ``bnfloop`` (the defaults of ``DualStep``).  All fits share ``bnfloop``: a batch that
+    mixes values is rejected, run it as two batches.  ``step(epoch)`` returns the per-fit totals ``[B]`` (float64);
+    ``.pos[i]``, ``.norm[i]``, ``.parts[i]`` are fit ``i``'s outputs."""
+
+    def __init__(self, fits, bnfloop=1, bnf_warmup_epochs=100, capture=True):
+        from . import multi
+        fits = [dict(f) for f in fits]
+        if not fits:
+            raise ValueError("MultiDualStep: no fits")
+        loops = {int(f.get("bnfloop", bnfloop)) for f in fits}
+        if len(loops) != 1:
+            raise ValueError(f"MultiDualStep: the fits mix bnfloop values {sorted(loops)}; run one batch per value")
+        devs = {torch.device(n.device) for f in fits for n in (f["posnet"], f["normnet"])}
+        if any(d.type != "cuda" for d in devs):
+            raise RuntimeError("MultiDualStep runs on CUDA only (dual_dmp_b200 has no CPU path)")
+        if len(devs) != 1:
+            raise ValueError(f"MultiDualStep: the fits are on several devices {sorted(map(str, devs))}; one batch "
+                             "runs on one device")
+        dev = devs.pop()
+        self.device = dev
+        self.bnfloop = loops.pop()
+        self.bnf_warmup_epochs = int(bnf_warmup_epochs)
+        self.capture = bool(capture)
+        self.fits = fits
+        self.ks = [tuple(float(x) for x in f.get("k", (3.0, 4.0, 4.0, 4.0, 1.0))) for f in fits]
+        self.datasets = [copy.copy(f["dataset"]).to(dev) for f in fits]
+        self.tgt_vs = [torch.from_numpy(f["n_mesh"].vs).to(dev) for f in fits]
+        self.tgt_fn = [torch.from_numpy(f["n_mesh"].fn).to(dev) for f in fits]
+        self._streams = [(torch.cuda.Stream(dev), torch.cuda.Stream(dev)) for _ in fits]
+        nets = [n for f in fits for n in (f["posnet"], f["normnet"])]
+        self.opt = GroupFusedAdam(
+            nets, [lr for f in fits for lr in (f.get("pos_lr", 0.01), f.get("norm_lr", 0.01))],
+            [m for f in fits for m in (None, float(f.get("grad_clip", 0.8)))])
+        self._tables = multi.DeviceTables(dev)
+        self._pinned = None
+        self._graphs: dict = {}
+        self._static_loss: dict = {}
+        self._pending = False
+        self._eager_calls = 0
+        self.pos = self.norm = self.parts = None
+
+    def prefetch(self, *args, **kwargs):
+        raise NotImplementedError("MultiDualStep keeps its inputs resident; streamed inputs are a DualStep feature")
+
+    def _body(self, bnf_off: bool) -> torch.Tensor:
+        from . import multi
+        from .graph import pin_graphs, topology_for
+        self._tables.phase = bnf_off
+        self.opt.zero_grad(set_to_none=True)
+        cur = torch.cuda.current_stream(self.device)
+        poss, nrms = [], []
+        for f, ds, (s_pos, s_nrm) in zip(self.fits, self.datasets, self._streams):
+            f["posnet"].train()
+            f["normnet"].train()
+            s_pos.wait_stream(cur)
+            s_nrm.wait_stream(cur)
+            with torch.cuda.stream(s_nrm):           # the larger network first
+                nrms.append(f["normnet"](ds))
+            with torch.cuda.stream(s_pos):
+                poss.append(f["posnet"](ds))
+        for (s_pos, s_nrm), pos, nrm in zip(self._streams, poss, nrms):
+            cur.wait_stream(s_pos)
+            cur.wait_stream(s_nrm)
+            pos.record_stream(cur)
+            nrm.record_stream(cur)
+        if self._pinned is None:      # B > 32 fits outgrow graph_for's cache: keep every fit's graphs reachable
+            import weakref
+            pairs = [(ds.edge_index, f["posnet"].last_graph) for f, ds in zip(self.fits, self.datasets)]
+            pairs += [(ds.face_index, f["normnet"].last_graph) for f, ds in zip(self.fits, self.datasets)]
+            self._pinned = pin_graphs(pairs)
+            from .graph import unpin_graphs
+            weakref.finalize(self, unpin_graphs, list(self._pinned))
+        topos = [topology_for(f["n_mesh"], self.device) for f in self.fits]
+        totals, self.parts = multi.DualLossMulti.apply(self._tables, topos, self.tgt_vs, self.tgt_fn, self.ks,
+                                                       self.bnfloop, 0.0 if bnf_off else 1.0, *poss, *nrms)
+        totals.sum().backward()
+        self.opt.step(self._tables)
+        self.pos = [p.detach() for p in poss]
+        self.norm = [n.detach() for n in nrms]
+        return totals.detach()
+
+    def _capture(self, bnf_off: bool) -> None:
+        self._tables.prepare(bnf_off)
+        super()._capture(bnf_off)
+        self._tables.flush()

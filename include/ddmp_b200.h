@@ -344,6 +344,23 @@ int ddmp_dual_loss(const float* pos, const float* nrm, const double* tgt_vs, con
  * out16[13..15] unused (scripts/bench_loss.py prints the differences).  Synchronises the device. */
 int ddmp_dual_loss_trace(uint64_t* out16);
 
+/* ddmp_dual_loss for n_mesh independent meshes as ONE cooperative launch.  Mesh m gets the min(G, ceil(max(V,F)/256))
+ * blocks its stand-alone launch would use (G = ddmp_dual_loss_grid(0)) and runs the stand-alone arithmetic on them, so
+ * its losses, gpos and gnrm equal a ddmp_dual_loss call bit for bit.  bnf_scale and loop are shared by the batch.
+ * table: DEVICE array of n_mesh descriptors of DDMP_DUAL_LOSS_DESC_WORDS 8-byte words each:
+ *   0 pos   1 nrm   2 tgt_vs   3 tgt_fn   4 faces   5 f2f   6 rslot   7 lap_rowptr   8 lap_col   9 corner_ptr
+ *   10 corner_slot   11 workspace (ddmp_dual_loss_workspace_bytes(V, F, loop) bytes, its own per mesh)
+ *   12 gpos   13 gnrm   14 losses[6]   (device addresses, as int64)
+ *   15 V   16 F   (int64)
+ *   17..21 k1..k5   (IEEE float32 in the low 4 bytes of the word, upper 4 bytes zero)
+ * vf: HOST array [n_mesh][2] of the same V, F (the launch size is computed from it; it must match the table).
+ * The sum of the meshes' blocks must not exceed ddmp_dual_loss_grid(1), the co-resident blocks of the batched kernel;
+ * callers split larger batches into consecutive launches on one stream. */
+#define DDMP_DUAL_LOSS_DESC_WORDS 22
+int64_t ddmp_dual_loss_grid(int32_t batched);
+int ddmp_dual_loss_multi(const int64_t* table, const int64_t* vf, int32_t n_mesh, float bnf_scale, int32_t loop,
+                         void* stream);
+
 /* mean angular distance in degrees between two sets of unit normals, float64 [ref: util/loss.py:261-272]. */
 int ddmp_mad(const float* n1, const float* n2, double* out, void* scratch, int64_t F, void* stream);
 /* vertex normals: normalise(sum of incident face normals) through the corner CSR [ref: util/models.py:12-29]. */
@@ -376,6 +393,24 @@ int ddmp_adam_step_dev(float* param, const float* grad, float* exp_avg, float* e
  * [ref: main.py:107-110: loss.backward() leaves one .grad per parameter; the optimizer walks them] */
 int ddmp_gather_flat(const void* const* srcs, const int64_t* offsets, const int64_t* counts, int32_t n_src, float* dst,
                      void* stream);
+
+/* ---- the optimizer of many networks at once (a batch of fits), one launch per stage ------------------------------ */
+/* ddmp_gather_flat from a DEVICE table of n_src rows (source address, destination offset, count), 3 int64 words each,
+ * in one launch (n_src <= 65535); `longest` is the largest count. */
+int ddmp_gather_table(const int64_t* table, int32_t n_src, int64_t longest, float* dst, void* stream);
+/* Segment table: DEVICE array of n_seg rows of DDMP_SEGMENT_WORDS int64 words, one row per network:
+ *   0 offset into the flat buffers   1 count   2 clip (0 / 1)   3 lr   4 max_norm
+ *   (lr, max_norm: IEEE float32 in the low 4 bytes of the word, upper 4 bytes zero).  `longest` is the largest count.
+ * ddmp_grad_norm_segments: norms[s] = ddmp_grad_norm of segment s, for every segment with clip = 1, bit for bit (the
+ * same block partition and summation order).  scratch: n_seg * ddmp_loss_scratch_bytes() bytes, zeroed once.
+ * ddmp_adam_segments: increments *step_counter, then the update of ddmp_adam_step_dev on every segment with its lr
+ * and, where clip = 1, the clip coefficient min(1, max_norm/(norms[s]+1e-6)). */
+#define DDMP_SEGMENT_WORDS 5
+int ddmp_grad_norm_segments(const float* flat, const int64_t* table, int32_t n_seg, int64_t longest, float* norms,
+                            void* scratch, void* stream);
+int ddmp_adam_segments(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, const int64_t* table,
+                       int32_t n_seg, int64_t longest, const float* norms, float beta1, float beta2, float eps,
+                       int64_t* step_counter, void* stream);
 
 #ifdef __cplusplus
 }
