@@ -603,6 +603,23 @@ __device__ __forceinline__ void split_f16x8(const float4& a, const float4& b, ui
     split_f16x2(a.x, a.y, hi.x, lo.x); split_f16x2(a.z, a.w, hi.y, lo.y);
     split_f16x2(b.x, b.y, hi.z, lo.z); split_f16x2(b.z, b.w, hi.w, lo.w);
 }
+// ---- single-product mode (TERMS = 1, DDMP_GEMM_F16X1) -----------------------------------------------------------------
+// The fp16-split kernels below take a compile-time term count.  TERMS = 3 is the fp32 emulation above.  TERMS = 1 keeps
+// only hi = fp16(s*x) of both operands and issues one MMA (hi*hi) per k-step: the same power-of-two scales, BatchNorm +
+// LeakyReLU prologue, fp32 accumulation in TMEM, epilogue and unscale, but each product carries the relative error of
+// two fp16 roundings, |fl16(sa)*fl16(sb)/s^2 - ab| <= (2u + u^2)|a||b| with u = 2^-11 (elements below 2^-14 after
+// scaling round to fp16 subnormals: at most 2^-25 absolute per scaled element).  One third of the MMAs, half the
+// operand bytes in shared memory and in the weight image; the freed shared memory doubles the pipeline depth.
+// The caller chooses it per call (a lower-precision accuracy contract, never automatic).
+template <int TERMS>
+struct Terms {
+    static_assert(TERMS == 3 || TERMS == 1, "fp16-split kernels: 3 (hi*hi + hi*lo + lo*hi) or 1 (hi*hi) terms");
+    static constexpr int PIECES = TERMS == 3 ? 2 : 1;        // fp16 pieces per operand element: hi, lo | hi
+};
+__device__ __forceinline__ uint32_t pack_f16x2(float x0, float x1) {
+    const __half2 h = __floats2half2_rn(x0, x1);                     // x0 -> low half, as split_f16x2's hi
+    return *reinterpret_cast<const uint32_t*>(&h);
+}
 // max |arr[i]| over the whole CTA -> bits, via `slot` (shared, zeroed before the preceding __syncthreads)
 __device__ __forceinline__ void block_amax_bits(const float* __restrict__ arr, int64_t len, uint32_t* slot) {
     uint32_t m = 0;
@@ -668,7 +685,7 @@ __device__ __forceinline__ float4 ldg4_pinned(const float* p) {
 // not the tensor pipe, set the pace of the fp16-split kernel: per k-block 420 cycles issuing loads, ~100 waiting for
 // a free stage and 1600 between the wait and the arrive, most of it load latency, while the MMA thread waited
 // 1100 cycles per k-block for `full`.
-template <int STAGES, class Args, class WaitEmpty>
+template <int STAGES, int TERMS, class Args, class WaitEmpty>
 __device__ __forceinline__ void produce_loop(const Args& g, int64_t first_tile, int64_t tile_step, int64_t row_mul,
                                                     int64_t row_add, int num_kb, float s_a, uint32_t smem_base,
                                                     uint32_t stage_bytes, uint32_t a_bytes, uint64_t* full_bar,
@@ -742,12 +759,16 @@ __device__ __forceinline__ void produce_loop(const Args& g, int64_t first_tile, 
             } else {
                 a.x *= s_a; a.y *= s_a; a.z *= s_a; a.w *= s_a;
             }
-            uint32_t h0, l0, h1, l1;
-            split_f16x2(a.x, a.y, h0, l0);
-            split_f16x2(a.z, a.w, h1, l1);
-            const uint32_t off = sw128(row, c4 >> 1) + ((c4 & 1u) << 3);
-            sts64(st + off, h0, h1);
-            sts64(st + a_bytes + off, l0, l1);
+            if constexpr (TERMS == 3) {
+                uint32_t h0, l0, h1, l1;
+                split_f16x2(a.x, a.y, h0, l0);
+                split_f16x2(a.z, a.w, h1, l1);
+                const uint32_t off = sw128(row, c4 >> 1) + ((c4 & 1u) << 3);
+                sts64(st + off, h0, h1);
+                sts64(st + a_bytes + off, l0, l1);
+            } else {
+                sts64(st + sw128(row, c4 >> 1) + ((c4 & 1u) << 3), pack_f16x2(a.x, a.y), pack_f16x2(a.z, a.w));
+            }
         }
         long long cA = 0, cB = 0;
         if (tr) cA = clock64();
@@ -829,7 +850,7 @@ __device__ __forceinline__ void tma_a_loop(const Args& g, const CUtensorMap* ama
     }
 }
 
-template <int STAGES, int RAW, class Args, class WaitEmpty>
+template <int STAGES, int RAW, int TERMS, class Args, class WaitEmpty>
 __device__ __forceinline__ void transform_loop(const Args& g, int64_t first_tile, int64_t tile_step, int num_kb, float s_a,
                                                uint32_t smem_base, uint32_t raw_base, uint32_t stage_bytes,
                                                uint32_t a_bytes, uint64_t* full_bar, uint64_t* empty_bar,
@@ -880,12 +901,16 @@ __device__ __forceinline__ void transform_loop(const Args& g, int64_t first_tile
             } else {
                 a.x *= s_a; a.y *= s_a; a.z *= s_a; a.w *= s_a;
             }
-            uint32_t h0, l0, h1, l1;
-            split_f16x2(a.x, a.y, h0, l0);
-            split_f16x2(a.z, a.w, h1, l1);
-            const uint32_t off = sw128(row, c4 >> 1) + ((c4 & 1u) << 3);
-            sts64(st + off, h0, h1);
-            sts64(st + a_bytes + off, l0, l1);
+            if constexpr (TERMS == 3) {
+                uint32_t h0, l0, h1, l1;
+                split_f16x2(a.x, a.y, h0, l0);
+                split_f16x2(a.z, a.w, h1, l1);
+                const uint32_t off = sw128(row, c4 >> 1) + ((c4 & 1u) << 3);
+                sts64(st + off, h0, h1);
+                sts64(st + a_bytes + off, l0, l1);
+            } else {
+                sts64(st + sw128(row, c4 >> 1) + ((c4 & 1u) << 3), pack_f16x2(a.x, a.y), pack_f16x2(a.z, a.w));
+            }
         }
         if (tr) cA = clock64();
         fence_proxy_async();
@@ -1053,7 +1078,9 @@ __device__ __forceinline__ void epilogue_tile_tma(const CUtensorMap* cmap, const
     }
 }
 
-// W [N,K] (or, transposed, W^T given as [K,N]) -> per-row scaled fp16 hi/lo image; one warp per weight row n
+// W [N,K] (or, transposed, W^T given as [K,N]) -> per-row scaled fp16 hi/lo image (TERMS = 1: hi only,
+// [n_tile][k_block][BN rows x 128 B]); one warp per weight row n
+template <int TERMS>
 __global__ void tc_prep_b16_kernel(const float* __restrict__ W, int transposed, uint8_t* __restrict__ img,
                                    float* __restrict__ inv_sw, int N, int K, int BN) {
     const int n = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
@@ -1091,25 +1118,33 @@ __global__ void tc_prep_b16_kernel(const float* __restrict__ W, int transposed, 
         float4 a, b;
         load8(c, a, b);
         a.x *= s; a.y *= s; a.z *= s; a.w *= s; b.x *= s; b.y *= s; b.z *= s; b.w *= s;
-        uint4 hi, lo;
-        split_f16x8(a, b, hi, lo);
-        const int kb = c / 8, cc = c % 8;
-        const int64_t base = ((int64_t)n_tile * num_kb + kb) * 2 * half_bytes;
-        const uint32_t off = sw128((uint32_t)r, (uint32_t)cc);
-        *reinterpret_cast<uint4*>(img + base + off) = hi;
-        *reinterpret_cast<uint4*>(img + base + half_bytes + off) = lo;
+        if constexpr (TERMS == 3) {
+            uint4 hi, lo;
+            split_f16x8(a, b, hi, lo);
+            const int kb = c / 8, cc = c % 8;
+            const int64_t base = ((int64_t)n_tile * num_kb + kb) * 2 * half_bytes;
+            const uint32_t off = sw128((uint32_t)r, (uint32_t)cc);
+            *reinterpret_cast<uint4*>(img + base + off) = hi;
+            *reinterpret_cast<uint4*>(img + base + half_bytes + off) = lo;
+        } else {
+            const int kb = c / 8, cc = c % 8;
+            const int64_t base = ((int64_t)n_tile * num_kb + kb) * half_bytes;
+            *reinterpret_cast<uint4*>(img + base + sw128((uint32_t)r, (uint32_t)cc)) =
+                make_uint4(pack_f16x2(a.x, a.y), pack_f16x2(a.z, a.w), pack_f16x2(b.x, b.y), pack_f16x2(b.z, b.w));
+        }
     }
 }
 
 // RAW = 0: A by the register-fed producers (produce_loop); RAW > 0: A by TMA into RAW raw slots (tma_a_loop +
-// transform_loop).  ACC: depth of the TMEM accumulator ring (ACC x BN columns).
-template <int BN, int STAGES, int RAW, int ACC>
+// transform_loop).  ACC: depth of the TMEM accumulator ring (ACC x BN columns).  TERMS: 3 or 1 (see Terms).
+template <int BN, int STAGES, int RAW, int ACC, int TERMS>
 __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __grid_constant__ CUtensorMap cmap,
                                                                      const __grid_constant__ CUtensorMap amap,
                                                                      const Nt16Args g) {
+    constexpr uint32_t P = Terms<TERMS>::PIECES;
     constexpr uint32_t A_BYTES = BM * 128;           // 128 rows x 64 fp16, one of hi / lo
     constexpr uint32_t B_BYTES = BN * 128;
-    constexpr uint32_t STAGE_BYTES = 2 * A_BYTES + 2 * B_BYTES;
+    constexpr uint32_t STAGE_BYTES = P * A_BYTES + P * B_BYTES;
     constexpr uint32_t TMEM_COLS = ACC * BN;
     static_assert(TMEM_COLS <= 512 && (TMEM_COLS & (TMEM_COLS - 1)) == 0, "TMEM allocation: power of two <= 512");
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -1158,12 +1193,12 @@ __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __gri
         // ===== A producers (see produce_loop / transform_loop) =====
         auto wait_empty = [](uint64_t* bar, uint32_t parity) { mbar_wait(bar, parity); };
         if constexpr (RAW > 0)
-            transform_loop<STAGES, RAW>(g, (int64_t)blockIdx.x, (int64_t)gridDim.x, num_kb, s_a, smem_base,
-                                        smem_u32(raw), STAGE_BYTES, A_BYTES, full_bar, empty_bar, raw_full, raw_empty,
-                                        wait_empty);
+            transform_loop<STAGES, RAW, TERMS>(g, (int64_t)blockIdx.x, (int64_t)gridDim.x, num_kb, s_a, smem_base,
+                                               smem_u32(raw), STAGE_BYTES, A_BYTES, full_bar, empty_bar, raw_full,
+                                               raw_empty, wait_empty);
         else
-            produce_loop<STAGES>(g, (int64_t)blockIdx.x, (int64_t)gridDim.x, (int64_t)BM, 0, num_kb, s_a,
-                                 smem_base, STAGE_BYTES, A_BYTES, full_bar, empty_bar, wait_empty);
+            produce_loop<STAGES, TERMS>(g, (int64_t)blockIdx.x, (int64_t)gridDim.x, (int64_t)BM, 0, num_kb, s_a,
+                                        smem_base, STAGE_BYTES, A_BYTES, full_bar, empty_bar, wait_empty);
     } else if (warp == 8) {
         // ===== MMA issuer =====
         if (lane == 0) {
@@ -1193,13 +1228,18 @@ __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __gri
 #pragma unroll
                     for (int ks = 0; ks < BK16 / UMMA_K16; ++ks) {
                         const uint32_t koff = ks * UMMA_K16 * 2;
-                        const uint64_t a_hi = make_desc(sa + koff, 16, 1024);
-                        const uint64_t a_lo = make_desc(sa + A_BYTES + koff, 16, 1024);
-                        const uint64_t b_hi = make_desc(sa + 2 * A_BYTES + koff, 16, 1024);
-                        const uint64_t b_lo = make_desc(sa + 2 * A_BYTES + B_BYTES + koff, 16, 1024);
-                        umma_f16(d_tmem, a_lo, b_hi, idesc, (kb | ks) != 0);
-                        umma_f16(d_tmem, a_hi, b_lo, idesc, 1);
-                        umma_f16(d_tmem, a_hi, b_hi, idesc, 1);
+                        if constexpr (TERMS == 3) {
+                            const uint64_t a_hi = make_desc(sa + koff, 16, 1024);
+                            const uint64_t a_lo = make_desc(sa + A_BYTES + koff, 16, 1024);
+                            const uint64_t b_hi = make_desc(sa + 2 * A_BYTES + koff, 16, 1024);
+                            const uint64_t b_lo = make_desc(sa + 2 * A_BYTES + B_BYTES + koff, 16, 1024);
+                            umma_f16(d_tmem, a_lo, b_hi, idesc, (kb | ks) != 0);
+                            umma_f16(d_tmem, a_hi, b_lo, idesc, 1);
+                            umma_f16(d_tmem, a_hi, b_hi, idesc, 1);
+                        } else {
+                            umma_f16(d_tmem, make_desc(sa + koff, 16, 1024), make_desc(sa + A_BYTES + koff, 16, 1024),
+                                     idesc, (kb | ks) != 0);
+                        }
                     }
                     umma_commit(empty_bar + s);
                 }
@@ -1213,14 +1253,14 @@ __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __gri
             uint32_t it = 0;
             for (int64_t tile = blockIdx.x; tile < g.num_tiles; tile += gridDim.x) {
                 const int tn = (int)(tile % g.tiles_n);
-                const uint8_t* src = g.Bimg + (int64_t)tn * num_kb * (2 * (int64_t)B_BYTES);
+                const uint8_t* src = g.Bimg + (int64_t)tn * num_kb * (P * (int64_t)B_BYTES);
                 for (int kb = 0; kb < num_kb; ++kb, ++it) {
                     const int s = it % STAGES;
                     const uint32_t ph = (it / STAGES) & 1;
                     mbar_wait(empty_bar + s, ph ^ 1u);
-                    mbar_arrive_expect_tx(full_bar + s, 2 * B_BYTES);
-                    bulk_g2s(smem_base + s * STAGE_BYTES + 2 * A_BYTES, src + (int64_t)kb * (2 * (int64_t)B_BYTES),
-                             2 * B_BYTES, full_bar + s);
+                    mbar_arrive_expect_tx(full_bar + s, P * B_BYTES);
+                    bulk_g2s(smem_base + s * STAGE_BYTES + P * A_BYTES, src + (int64_t)kb * (P * (int64_t)B_BYTES),
+                             P * B_BYTES, full_bar + s);
                 }
             }
         }
@@ -1274,8 +1314,9 @@ __global__ void __launch_bounds__(kV2Threads, 1) tc_gemm_nt16_kernel(const __gri
 }
 
 // dynamic shared memory of the fp16-split NT kernels: split stages, raw A slots, epilogue staging, barriers
-constexpr size_t nt16_smem(int stages, uint32_t b_bytes, int raw) {
-    return (size_t)stages * (2 * BM * 128 + 2 * b_bytes) + (size_t)raw * kRawSlotBytes + kStagingBytes + 1024 + 256;
+constexpr size_t nt16_smem(int stages, uint32_t b_bytes, int raw, int pieces = 2) {
+    return (size_t)stages * (pieces * BM * 128 + pieces * b_bytes) + (size_t)raw * kRawSlotBytes + kStagingBytes + 1024 +
+           256;
 }
 
 // tensor map of A [M, K] for the raw ring: 128-row x 32-column boxes, 128-byte swizzle, rows past M zero-filled
@@ -1283,13 +1324,13 @@ static int make_a_map(CUtensorMap* amap, const Nt16Args& g, const char* who) {
     return make_tensor_map_2d(amap, g.A, g.M, g.K, BM, 32, true, who);
 }
 
-template <int BN, int STAGES, int RAW, int ACC>
+template <int BN, int STAGES, int RAW, int ACC, int TERMS>
 static int launch_nt16(const Nt16Args& g, cudaStream_t st) {
-    constexpr size_t smem = nt16_smem(STAGES, BN * 128, RAW);
+    constexpr size_t smem = nt16_smem(STAGES, BN * 128, RAW, Terms<TERMS>::PIECES);
     static_assert(smem <= 232448, "shared memory of the fp16-split NT kernel");
     static PerDeviceOnce configured;
     if (configured.need()) {
-        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_nt16_kernel<BN, STAGES, RAW, ACC>,
+        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_nt16_kernel<BN, STAGES, RAW, ACC, TERMS>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured.mark();
     }
@@ -1299,7 +1340,7 @@ static int launch_nt16(const Nt16Args& g, cudaStream_t st) {
     CUtensorMap amap = cmap;                             // unused by the register-fed configuration
     if (RAW > 0 && (rc = make_a_map(&amap, g, "tc_gemm_nt16 A")) != DDMP_OK) return rc;
     const int64_t grid = g.num_tiles < kNumSMs ? g.num_tiles : kNumSMs;
-    tc_gemm_nt16_kernel<BN, STAGES, RAW, ACC><<<(unsigned)grid, kV2Threads, smem, st>>>(cmap, amap, g);
+    tc_gemm_nt16_kernel<BN, STAGES, RAW, ACC, TERMS><<<(unsigned)grid, kV2Threads, smem, st>>>(cmap, amap, g);
     return check_launch("tc_gemm_nt16");
 }
 
@@ -1320,15 +1361,16 @@ __device__ __forceinline__ void umma_f16_2cta(uint32_t tmem_d, uint64_t adesc, u
 }
 
 // RAW = 0: A by the register-fed producers; RAW > 0: A by TMA into RAW raw slots (as in tc_gemm_nt16_kernel)
-template <int STAGES, int RAW>
+template <int STAGES, int RAW, int TERMS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kV2Threads, 1)
 tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const __grid_constant__ CUtensorMap amap,
                       const Nt16Args g) {
     constexpr int BN = 256;
+    constexpr uint32_t P = Terms<TERMS>::PIECES;
     constexpr uint32_t A_BYTES = BM * 128;
     constexpr uint32_t B_HALF = (BN / 2) * 128;          // this CTA's half of the weight tile, one of hi / lo
     constexpr uint32_t B_FULL = BN * 128;
-    constexpr uint32_t STAGE_BYTES = 2 * A_BYTES + 2 * B_HALF;
+    constexpr uint32_t STAGE_BYTES = P * A_BYTES + P * B_HALF;
     constexpr uint32_t TMEM_COLS = 2 * BN;
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -1380,11 +1422,11 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const __grid_con
     if (warp < kProducerWarps) {
         auto wait_empty = [](uint64_t* bar, uint32_t parity) { mbar_wait_cluster(bar, parity); };
         if constexpr (RAW > 0)
-            transform_loop<STAGES, RAW>(g, pair, num_pairs, num_kb, s_a, smem_base, smem_u32(raw), STAGE_BYTES, A_BYTES,
-                                        full_bar, empty_bar, raw_full, raw_empty, wait_empty);
+            transform_loop<STAGES, RAW, TERMS>(g, pair, num_pairs, num_kb, s_a, smem_base, smem_u32(raw), STAGE_BYTES,
+                                               A_BYTES, full_bar, empty_bar, raw_full, raw_empty, wait_empty);
         else
-            produce_loop<STAGES>(g, pair, num_pairs, (int64_t)(2 * BM), (int64_t)rank * BM, num_kb, s_a,
-                                 smem_base, STAGE_BYTES, A_BYTES, full_bar, empty_bar, wait_empty);
+            produce_loop<STAGES, TERMS>(g, pair, num_pairs, (int64_t)(2 * BM), (int64_t)rank * BM, num_kb, s_a,
+                                        smem_base, STAGE_BYTES, A_BYTES, full_bar, empty_bar, wait_empty);
     } else if (warp == 8) {
         if (lane == 0) {
             uint32_t it = 0, tile_no = 0;
@@ -1418,13 +1460,18 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const __grid_con
 #pragma unroll
                         for (int ks = 0; ks < BK16 / UMMA_K16; ++ks) {
                             const uint32_t koff = ks * UMMA_K16 * 2;
-                            const uint64_t a_hi = make_desc(sa + koff, 16, 1024);
-                            const uint64_t a_lo = make_desc(sa + A_BYTES + koff, 16, 1024);
-                            const uint64_t b_hi = make_desc(sa + 2 * A_BYTES + koff, 16, 1024);
-                            const uint64_t b_lo = make_desc(sa + 2 * A_BYTES + B_HALF + koff, 16, 1024);
-                            umma_f16_2cta(d_tmem, a_lo, b_hi, idesc, (kb | ks) != 0);
-                            umma_f16_2cta(d_tmem, a_hi, b_lo, idesc, 1);
-                            umma_f16_2cta(d_tmem, a_hi, b_hi, idesc, 1);
+                            if constexpr (TERMS == 3) {
+                                const uint64_t a_hi = make_desc(sa + koff, 16, 1024);
+                                const uint64_t a_lo = make_desc(sa + A_BYTES + koff, 16, 1024);
+                                const uint64_t b_hi = make_desc(sa + 2 * A_BYTES + koff, 16, 1024);
+                                const uint64_t b_lo = make_desc(sa + 2 * A_BYTES + B_HALF + koff, 16, 1024);
+                                umma_f16_2cta(d_tmem, a_lo, b_hi, idesc, (kb | ks) != 0);
+                                umma_f16_2cta(d_tmem, a_hi, b_lo, idesc, 1);
+                                umma_f16_2cta(d_tmem, a_hi, b_hi, idesc, 1);
+                            } else {
+                                umma_f16_2cta(d_tmem, make_desc(sa + koff, 16, 1024),
+                                              make_desc(sa + A_BYTES + koff, 16, 1024), idesc, (kb | ks) != 0);
+                            }
                         }
                         umma_commit_2cta(empty_bar + s);
                     }
@@ -1447,16 +1494,16 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const __grid_con
             uint32_t it = 0;
             for (int64_t tile = pair; tile < g.num_tiles; tile += num_pairs) {
                 const int tn = (int)(tile % g.tiles_n);
-                const uint8_t* src = g.Bimg + (int64_t)tn * num_kb * (2 * (int64_t)B_FULL) + (int64_t)rank * B_HALF;
+                const uint8_t* src = g.Bimg + (int64_t)tn * num_kb * (P * (int64_t)B_FULL) + (int64_t)rank * B_HALF;
                 for (int kb = 0; kb < num_kb; ++kb, ++it) {
                     const int s = it % STAGES;
                     const uint32_t ph = (it / STAGES) & 1;
                     mbar_wait_cluster(empty_bar + s, ph ^ 1u);
-                    mbar_arrive_expect_tx(full_bar + s, 2 * B_HALF);
-                    const uint8_t* sk = src + (int64_t)kb * (2 * (int64_t)B_FULL);
-                    const uint32_t dst = smem_base + s * STAGE_BYTES + 2 * A_BYTES;
+                    mbar_arrive_expect_tx(full_bar + s, P * B_HALF);
+                    const uint8_t* sk = src + (int64_t)kb * (P * (int64_t)B_FULL);
+                    const uint32_t dst = smem_base + s * STAGE_BYTES + P * A_BYTES;
                     bulk_g2s(dst, sk, B_HALF, full_bar + s);
-                    bulk_g2s(dst + B_HALF, sk + B_FULL, B_HALF, full_bar + s);
+                    if constexpr (TERMS == 3) bulk_g2s(dst + B_HALF, sk + B_FULL, B_HALF, full_bar + s);
                 }
             }
         }
@@ -1512,14 +1559,14 @@ tc_gemm_nt16x2_kernel(const __grid_constant__ CUtensorMap cmap, const __grid_con
     }
 }
 
-template <int STAGES, int RAW>
+template <int STAGES, int RAW, int TERMS>
 static int launch_nt16x2(const Nt16Args& g0, cudaStream_t st) {
-    constexpr size_t smem = nt16_smem(STAGES, 128 * 128, RAW);
+    constexpr size_t smem = nt16_smem(STAGES, 128 * 128, RAW, Terms<TERMS>::PIECES);
     static_assert(smem <= 232448, "shared memory of the CTA-pair fp16-split NT kernel");
     static PerDeviceOnce configured;
     if (configured.need()) {
-        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_nt16x2_kernel<STAGES, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)smem));
+        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_nt16x2_kernel<STAGES, RAW, TERMS>,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured.mark();
     }
     Nt16Args g = g0;
@@ -1530,7 +1577,7 @@ static int launch_nt16x2(const Nt16Args& g0, cudaStream_t st) {
     CUtensorMap amap = cmap;                             // unused by the register-fed configuration
     if (RAW > 0 && (rc = make_a_map(&amap, g, "tc_gemm_nt16x2 A")) != DDMP_OK) return rc;
     const int64_t pairs = g.num_tiles < kNumSMs / 2 ? g.num_tiles : kNumSMs / 2;
-    tc_gemm_nt16x2_kernel<STAGES, RAW><<<(unsigned)(2 * pairs), kV2Threads, smem, st>>>(cmap, amap, g);
+    tc_gemm_nt16x2_kernel<STAGES, RAW, TERMS><<<(unsigned)(2 * pairs), kV2Threads, smem, st>>>(cmap, amap, g);
     return check_launch("tc_gemm_nt16x2");
 }
 
@@ -1555,9 +1602,26 @@ static bool f16_split_enabled() {
     return v;
 }
 
+// the shape choice of run_nt16 for one term count; TERMS = 1 halves a split stage, so the same shared memory holds
+// twice as many of them (a deeper pipeline; raw A slots, accumulator ring and staging unchanged)
+template <int TERMS>
+static int launch_nt16_choice(const Nt16Args& g, int BN, bool tma_a, bool one_cta, cudaStream_t st) {
+    constexpr int D = TERMS == 3 ? 1 : 2;
+    if (BN == 256 && one_cta) return launch_nt16<256, 2 * D, 0, 2, TERMS>(g, st);
+    if (tma_a) {                                     // one split stage traded for the raw fp32 slots
+        if (BN == 256) return launch_nt16x2<2 * D, 2, TERMS>(g, st);
+        if (BN == 128) return launch_nt16<128, 2 * D, 2, 4, TERMS>(g, st);
+        return launch_nt16<64, 2 * D, 3, 4, TERMS>(g, st);
+    }
+    if (BN == 256) return launch_nt16x2<3 * D, 0, TERMS>(g, st);
+    if (BN == 128) return launch_nt16<128, 3 * D, 0, 2, TERMS>(g, st);
+    return launch_nt16<64, 4 * D, 0, 2, TERMS>(g, st);
+}
+
+// terms: 3 (fp32 emulation) or 1 (single fp16 product, DDMP_GEMM_F16X1)
 static int run_nt16(const float* A, const int* a_map, const float* scale, const float* shift, float slope,
                     const float* W, int transposed, void* workspace, float* C, int64_t M, int N, int K,
-                    const float* amax, int64_t amax_len, cudaStream_t st) {
+                    const float* amax, int64_t amax_len, int terms, cudaStream_t st) {
     int flags = f16_flags(-1);
     if ((flags & 2) && K <= 256) flags |= 1;         // bit 1: the L2 prefetch only where it measured faster (K <= 256)
     // (TMA tensor coordinates are 32-bit: row counts near 2^31 keep the register-fed producers)
@@ -1571,7 +1635,9 @@ static int run_nt16(const float* A, const int* a_map, const float* scale, const 
     const int BN = (N % 256 == 0 && !(tma_a && K <= 128)) ? 256 : ((N % 128 == 0) ? 128 : 64);
     uint8_t* img = reinterpret_cast<uint8_t*>(workspace);
     float* inv_sw = reinterpret_cast<float*>(img + (int64_t)N * K * 4);          // after the hi + lo images
-    tc_prep_b16_kernel<<<(unsigned)ceil_div((int64_t)N * 32, 256), 256, 0, st>>>(W, transposed, img, inv_sw, N, K, BN);
+    const unsigned prep_blocks = (unsigned)ceil_div((int64_t)N * 32, 256);
+    if (terms == 1) tc_prep_b16_kernel<1><<<prep_blocks, 256, 0, st>>>(W, transposed, img, inv_sw, N, K, BN);
+    else tc_prep_b16_kernel<3><<<prep_blocks, 256, 0, st>>>(W, transposed, img, inv_sw, N, K, BN);
     int rc = check_launch("tc_prep_b16");
     if (rc) return rc;
     Nt16Args g{};
@@ -1606,15 +1672,8 @@ static int run_nt16(const float* A, const int* a_map, const float* scale, const 
     g.num_tiles = ceil_div(M, BM) * g.tiles_n;
     DDMP_REQUIRE(g.num_tiles < (1ll << 31), "tc gemm: too many tiles");
     static const bool one_cta = [] { const char* e = getenv("DDMP_TC_2CTA"); return e && e[0] == '0'; }();
-    if (BN == 256 && one_cta) return dump_trace(launch_nt16<256, 2, 0, 2>(g, st));
-    if (tma_a) {                                     // one split stage traded for the raw fp32 slots
-        if (BN == 256) return dump_trace(launch_nt16x2<2, 2>(g, st));
-        if (BN == 128) return dump_trace(launch_nt16<128, 2, 2, 4>(g, st));
-        return dump_trace(launch_nt16<64, 2, 3, 4>(g, st));
-    }
-    if (BN == 256) return dump_trace(launch_nt16x2<3, 0>(g, st));
-    if (BN == 128) return dump_trace(launch_nt16<128, 3, 0, 2>(g, st));
-    return dump_trace(launch_nt16<64, 4, 0, 2>(g, st));
+    if (terms == 1) return dump_trace(launch_nt16_choice<1>(g, BN, tma_a, one_cta, st));
+    return dump_trace(launch_nt16_choice<3>(g, BN, tma_a, one_cta, st));
 }
 
 // ---- TN kernel (dW) -------------------------------------------------------------------------------------------------
@@ -1890,13 +1949,14 @@ struct Tn16Args {
     int64_t num_items;
 };
 
-template <int BN, int STAGES>
+template <int BN, int STAGES, int TERMS>
 __global__ void __launch_bounds__(16 * 32 + 32, 1) tc_gemm_tn16_kernel(const Tn16Args g) {
     constexpr int PW = 16;
     constexpr int kPT = PW * 32;
+    constexpr uint32_t P = Terms<TERMS>::PIECES;
     constexpr uint32_t A_BYTES = BM * BK16 * 2;      // 64 k-rows x 128 m x 2 B
     constexpr uint32_t B_BYTES = BN * BK16 * 2;
-    constexpr uint32_t STAGE_BYTES = 2 * A_BYTES + 2 * B_BYTES;
+    constexpr uint32_t STAGE_BYTES = P * A_BYTES + P * B_BYTES;
     constexpr uint32_t TMEM_COLS = BN < 32 ? 32 : BN;
     constexpr uint32_t LBO = (BK16 / 8) * 1024;      // next 64-wide MN block
     constexpr uint32_t SBO = 1024;                   // next group of 8 k-rows
@@ -1993,12 +2053,17 @@ __global__ void __launch_bounds__(16 * 32 + 32, 1) tc_gemm_tn16_kernel(const Tn1
                     const uint32_t k = a_r + j * A_PASS;
                     float4 a = av[j];
                     a.x *= s_a; a.y *= s_a; a.z *= s_a; a.w *= s_a;
-                    uint32_t h0, l0, h1, l1;
-                    split_f16x2(a.x, a.y, h0, l0);
-                    split_f16x2(a.z, a.w, h1, l1);
-                    const uint32_t off = a_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((a_cj ^ (k & 7u)) << 4);
-                    sts64(st + off, h0, h1);
-                    sts64(st + A_BYTES + off, l0, l1);
+                    if constexpr (TERMS == 3) {
+                        uint32_t h0, l0, h1, l1;
+                        split_f16x2(a.x, a.y, h0, l0);
+                        split_f16x2(a.z, a.w, h1, l1);
+                        const uint32_t off = a_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((a_cj ^ (k & 7u)) << 4);
+                        sts64(st + off, h0, h1);
+                        sts64(st + A_BYTES + off, l0, l1);
+                    } else {
+                        sts64(st + a_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((a_cj ^ (k & 7u)) << 4),
+                              pack_f16x2(a.x, a.y), pack_f16x2(a.z, a.w));
+                    }
                 }
 #pragma unroll
                 for (int j = 0; j < B_N; ++j) {
@@ -2012,12 +2077,17 @@ __global__ void __launch_bounds__(16 * 32 + 32, 1) tc_gemm_tn16_kernel(const Tn1
                     } else {
                         a.x *= s_b; a.y *= s_b; a.z *= s_b; a.w *= s_b;
                     }
-                    uint32_t h0, l0, h1, l1;
-                    split_f16x2(a.x, a.y, h0, l0);
-                    split_f16x2(a.z, a.w, h1, l1);
-                    const uint32_t off = b_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((b_cj ^ (k & 7u)) << 4);
-                    sts64(st + 2 * A_BYTES + off, h0, h1);
-                    sts64(st + 2 * A_BYTES + B_BYTES + off, l0, l1);
+                    if constexpr (TERMS == 3) {
+                        uint32_t h0, l0, h1, l1;
+                        split_f16x2(a.x, a.y, h0, l0);
+                        split_f16x2(a.z, a.w, h1, l1);
+                        const uint32_t off = b_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((b_cj ^ (k & 7u)) << 4);
+                        sts64(st + 2 * A_BYTES + off, h0, h1);
+                        sts64(st + 2 * A_BYTES + B_BYTES + off, l0, l1);
+                    } else {
+                        sts64(st + A_BYTES + b_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((b_cj ^ (k & 7u)) << 4),
+                              pack_f16x2(a.x, a.y), pack_f16x2(a.z, a.w));
+                    }
                 }
                 fence_proxy_async();
                 __syncwarp();
@@ -2063,13 +2133,18 @@ __global__ void __launch_bounds__(16 * 32 + 32, 1) tc_gemm_tn16_kernel(const Tn1
 #pragma unroll
                     for (int ks = 0; ks < BK16 / UMMA_K16; ++ks) {
                         const uint32_t koff = ks * 2u * SBO;                    // 16 k-rows = two 8-row groups
-                        const uint64_t a_hi = make_desc(sa + koff, LBO, SBO, 2);
-                        const uint64_t a_lo = make_desc(sa + A_BYTES + koff, LBO, SBO, 2);
-                        const uint64_t b_hi = make_desc(sa + 2 * A_BYTES + koff, LBO, SBO, 2);
-                        const uint64_t b_lo = make_desc(sa + 2 * A_BYTES + B_BYTES + koff, LBO, SBO, 2);
-                        umma_f16(tmem_base, a_lo, b_hi, idesc, (kb | ks) != 0);
-                        umma_f16(tmem_base, a_hi, b_lo, idesc, 1);
-                        umma_f16(tmem_base, a_hi, b_hi, idesc, 1);
+                        if constexpr (TERMS == 3) {
+                            const uint64_t a_hi = make_desc(sa + koff, LBO, SBO, 2);
+                            const uint64_t a_lo = make_desc(sa + A_BYTES + koff, LBO, SBO, 2);
+                            const uint64_t b_hi = make_desc(sa + 2 * A_BYTES + koff, LBO, SBO, 2);
+                            const uint64_t b_lo = make_desc(sa + 2 * A_BYTES + B_BYTES + koff, LBO, SBO, 2);
+                            umma_f16(tmem_base, a_lo, b_hi, idesc, (kb | ks) != 0);
+                            umma_f16(tmem_base, a_hi, b_lo, idesc, 1);
+                            umma_f16(tmem_base, a_hi, b_hi, idesc, 1);
+                        } else {
+                            umma_f16(tmem_base, make_desc(sa + koff, LBO, SBO, 2), make_desc(sa + A_BYTES + koff, LBO, SBO, 2),
+                                     idesc, (kb | ks) != 0);
+                        }
                     }
                     umma_commit(empty_bar + s);
                 }
@@ -2087,33 +2162,38 @@ __global__ void __launch_bounds__(16 * 32 + 32, 1) tc_gemm_tn16_kernel(const Tn1
     }
 }
 
-template <int BN, int STAGES>
+template <int BN, int STAGES, int TERMS>
 static int launch_tn16(const Tn16Args& g, cudaStream_t st) {
-    constexpr size_t smem = (size_t)STAGES * (2 * BM * BK16 * 2 + 2 * BN * BK16 * 2) + 1024 + 256;
+    constexpr int P = Terms<TERMS>::PIECES;
+    constexpr size_t smem = (size_t)STAGES * (P * BM * BK16 * 2 + P * BN * BK16 * 2) + 1024 + 256;
     static PerDeviceOnce configured;
     if (configured.need()) {
-        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_tn16_kernel<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)smem));
+        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_tn16_kernel<BN, STAGES, TERMS>,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured.mark();
     }
     const int64_t grid = g.num_items < kNumSMs ? g.num_items : kNumSMs;
-    tc_gemm_tn16_kernel<BN, STAGES><<<(unsigned)grid, 16 * 32 + 32, smem, st>>>(g);
+    tc_gemm_tn16_kernel<BN, STAGES, TERMS><<<(unsigned)grid, 16 * 32 + 32, smem, st>>>(g);
     return check_launch("tc_gemm_tn16");
 }
+
+// split stages of the CTA-pair TN kernel: TERMS = 1 fits twice as many in the same shared memory
+constexpr int tn16x2_stages(int nacc, int terms) { return ((nacc == 2) ? 2 : 3) * (terms == 3 ? 1 : 2); }
 
 // TN kernel on CTA pairs (cta_group::2): the pair owns a 256 x (256*NACC) tile of dW.  Each CTA splits its 128
 // channels of dH and 128*NACC channels of X per k-row, the MMAs (M = 256, N = 256 per accumulator) read both CTAs'
 // halves, and each CTA's TMEM receives its 128 output rows x 256*NACC columns.  Against the single-CTA kernel
 // (128 x 256 tiles) every element of dH is split once instead of Cin/256 times and every element of X Cout/256
 // instead of Cout/128 times: the producer work per MMA -- which bounds this kernel -- halves for 512 x 512.
-template <int NACC>
+template <int NACC, int TERMS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(16 * 32 + 32, 1) tc_gemm_tn16x2_kernel(const Tn16Args g) {
     constexpr int PW = 16;
     constexpr int kPT = PW * 32;
-    constexpr int STAGES = (NACC == 2) ? 2 : 3;
+    constexpr uint32_t P = Terms<TERMS>::PIECES;
+    constexpr int STAGES = tn16x2_stages(NACC, TERMS);
     constexpr uint32_t A_BYTES = BM * BK16 * 2;          // this CTA's 128 dH channels x 64 k-rows, one of hi / lo
     constexpr uint32_t B_BLK = 128 * BK16 * 2;           // this CTA's 128 X channels of one accumulator
-    constexpr uint32_t STAGE_BYTES = 2 * A_BYTES + NACC * 2 * B_BLK;
+    constexpr uint32_t STAGE_BYTES = P * A_BYTES + NACC * P * B_BLK;
     constexpr uint32_t TMEM_COLS = NACC * 256;
     constexpr uint32_t LBO = (BK16 / 8) * 1024;
     constexpr uint32_t SBO = 1024;
@@ -2187,7 +2267,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(16 * 32 + 32, 1) tc_
             }
             const uint32_t a_cm = a_c4 >> 1, b_cm = b_in >> 1;
             const uint32_t a_off0 = (a_cm / 8) * LBO + ((a_c4 & 1u) << 3);
-            const uint32_t b_off0 = 2 * A_BYTES + b_acc * (2 * B_BLK) + (b_cm / 8) * LBO + ((b_in & 1u) << 3);
+            const uint32_t b_off0 = P * A_BYTES + b_acc * (P * B_BLK) + (b_cm / 8) * LBO + ((b_in & 1u) << 3);
             const uint32_t a_cj = a_cm & 7u, b_cj = b_cm & 7u;
             float4 av[A_N], bv[B_N];
             auto issue = [&](int kb) {
@@ -2216,12 +2296,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(16 * 32 + 32, 1) tc_
                     const uint32_t k = a_r + j * A_PASS;
                     float4 a = av[j];
                     a.x *= s_a; a.y *= s_a; a.z *= s_a; a.w *= s_a;
-                    uint32_t h0, l0, h1, l1;
-                    split_f16x2(a.x, a.y, h0, l0);
-                    split_f16x2(a.z, a.w, h1, l1);
-                    const uint32_t off = a_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((a_cj ^ (k & 7u)) << 4);
-                    sts64(st + off, h0, h1);
-                    sts64(st + A_BYTES + off, l0, l1);
+                    if constexpr (TERMS == 3) {
+                        uint32_t h0, l0, h1, l1;
+                        split_f16x2(a.x, a.y, h0, l0);
+                        split_f16x2(a.z, a.w, h1, l1);
+                        const uint32_t off = a_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((a_cj ^ (k & 7u)) << 4);
+                        sts64(st + off, h0, h1);
+                        sts64(st + A_BYTES + off, l0, l1);
+                    } else {
+                        sts64(st + a_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((a_cj ^ (k & 7u)) << 4),
+                              pack_f16x2(a.x, a.y), pack_f16x2(a.z, a.w));
+                    }
                 }
 #pragma unroll
                 for (int j = 0; j < B_N; ++j) {
@@ -2235,12 +2320,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(16 * 32 + 32, 1) tc_
                     } else {
                         a.x *= s_b; a.y *= s_b; a.z *= s_b; a.w *= s_b;
                     }
-                    uint32_t h0, l0, h1, l1;
-                    split_f16x2(a.x, a.y, h0, l0);
-                    split_f16x2(a.z, a.w, h1, l1);
-                    const uint32_t off = b_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((b_cj ^ (k & 7u)) << 4);
-                    sts64(st + off, h0, h1);
-                    sts64(st + B_BLK + off, l0, l1);
+                    if constexpr (TERMS == 3) {
+                        uint32_t h0, l0, h1, l1;
+                        split_f16x2(a.x, a.y, h0, l0);
+                        split_f16x2(a.z, a.w, h1, l1);
+                        const uint32_t off = b_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((b_cj ^ (k & 7u)) << 4);
+                        sts64(st + off, h0, h1);
+                        sts64(st + B_BLK + off, l0, l1);
+                    } else {
+                        sts64(st + b_off0 + (k >> 3) * SBO + (k & 7u) * 128u + ((b_cj ^ (k & 7u)) << 4),
+                              pack_f16x2(a.x, a.y), pack_f16x2(a.z, a.w));
+                    }
                 }
                 fence_proxy_async();
                 __syncwarp();
@@ -2292,16 +2382,24 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(16 * 32 + 32, 1) tc_
                         for (int ks = 0; ks < BK16 / UMMA_K16; ++ks) {
                             const uint32_t koff = ks * 2u * SBO;
                             const uint64_t a_hi = make_desc(sa + koff, LBO, SBO, 2);
-                            const uint64_t a_lo = make_desc(sa + A_BYTES + koff, LBO, SBO, 2);
+                            if constexpr (TERMS == 3) {
+                                const uint64_t a_lo = make_desc(sa + A_BYTES + koff, LBO, SBO, 2);
 #pragma unroll
-                            for (int j = 0; j < NACC; ++j) {
-                                const uint32_t sb = sa + 2 * A_BYTES + j * (2 * B_BLK) + koff;
-                                const uint64_t b_hi = make_desc(sb, LBO, SBO, 2);
-                                const uint64_t b_lo = make_desc(sb + B_BLK, LBO, SBO, 2);
-                                const uint32_t d = tmem_base + j * 256;
-                                umma_f16_2cta(d, a_lo, b_hi, idesc, (kb | ks) != 0);
-                                umma_f16_2cta(d, a_hi, b_lo, idesc, 1);
-                                umma_f16_2cta(d, a_hi, b_hi, idesc, 1);
+                                for (int j = 0; j < NACC; ++j) {
+                                    const uint32_t sb = sa + 2 * A_BYTES + j * (2 * B_BLK) + koff;
+                                    const uint64_t b_hi = make_desc(sb, LBO, SBO, 2);
+                                    const uint64_t b_lo = make_desc(sb + B_BLK, LBO, SBO, 2);
+                                    const uint32_t d = tmem_base + j * 256;
+                                    umma_f16_2cta(d, a_lo, b_hi, idesc, (kb | ks) != 0);
+                                    umma_f16_2cta(d, a_hi, b_lo, idesc, 1);
+                                    umma_f16_2cta(d, a_hi, b_hi, idesc, 1);
+                                }
+                            } else {
+#pragma unroll
+                                for (int j = 0; j < NACC; ++j)
+                                    umma_f16_2cta(tmem_base + j * 256, a_hi,
+                                                  make_desc(sa + A_BYTES + j * B_BLK + koff, LBO, SBO, 2), idesc,
+                                                  (kb | ks) != 0);
                             }
                         }
                         umma_commit_2cta(empty_bar + s);
@@ -2329,19 +2427,36 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(16 * 32 + 32, 1) tc_
     }
 }
 
-template <int NACC>
+template <int NACC, int TERMS>
 static int launch_tn16x2(const Tn16Args& g, cudaStream_t st) {
-    constexpr int STAGES = (NACC == 2) ? 2 : 3;
-    constexpr size_t smem = (size_t)STAGES * (2 * BM * BK16 * 2 + NACC * 2 * 128 * BK16 * 2) + 1024 + 256;
+    constexpr int STAGES = tn16x2_stages(NACC, TERMS);
+    constexpr int P = Terms<TERMS>::PIECES;
+    constexpr size_t smem = (size_t)STAGES * (P * BM * BK16 * 2 + NACC * P * 128 * BK16 * 2) + 1024 + 256;
     static PerDeviceOnce configured;
     if (configured.need()) {
-        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_tn16x2_kernel<NACC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        DDMP_CUDA(cudaFuncSetAttribute(tc_gemm_tn16x2_kernel<NACC, TERMS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)smem));
         configured.mark();
     }
     const int64_t pairs = g.num_items < kNumSMs / 2 ? g.num_items : kNumSMs / 2;
-    tc_gemm_tn16x2_kernel<NACC><<<(unsigned)(2 * pairs), 16 * 32 + 32, smem, st>>>(g);
+    tc_gemm_tn16x2_kernel<NACC, TERMS><<<(unsigned)(2 * pairs), 16 * 32 + 32, smem, st>>>(g);
     return check_launch("tc_gemm_tn16x2");
+}
+
+// the tile choice of tc_gemm_dw's fp16-split path for one term count (h: shape fields set, tiles_m = ceil(Cout / 128));
+// TERMS = 1 doubles the split stages in the same shared memory
+template <int TERMS>
+static int launch_tn16_choice(Tn16Args& h, int64_t segs, bool one_cta, cudaStream_t st) {
+    constexpr int D = TERMS == 3 ? 1 : 2;
+    const int Cout = h.M, Cin = h.N;
+    if (!one_cta && Cout % 256 == 0 && Cin % 256 == 0) {
+        h.tiles_m = Cout / 256;
+        if (Cin % 512 == 0) { h.tiles_n = Cin / 512; h.num_items = segs * h.tiles_m * h.tiles_n; return launch_tn16x2<2, TERMS>(h, st); }
+        h.tiles_n = Cin / 256; h.num_items = segs * h.tiles_m * h.tiles_n; return launch_tn16x2<1, TERMS>(h, st);
+    }
+    if (Cin % 256 == 0) { h.tiles_n = Cin / 256; h.num_items = segs * h.tiles_m * h.tiles_n; return launch_tn16<256, 2 * D, TERMS>(h, st); }
+    if (Cin % 128 == 0) { h.tiles_n = Cin / 128; h.num_items = segs * h.tiles_m * h.tiles_n; return launch_tn16<128, 3 * D, TERMS>(h, st); }
+    h.tiles_n = Cin / 64; h.num_items = segs * h.tiles_m * h.tiles_n; return launch_tn16<64, 4 * D, TERMS>(h, st);
 }
 
 }  // namespace tc
@@ -2365,25 +2480,28 @@ bool tc_supported_dw(int64_t n, int32_t Cin, int32_t Cout) {
 
 int64_t tc_gemm_nt_workspace_bytes(int32_t Cin, int32_t Cout) { return 2ll * Cin * Cout * (int64_t)sizeof(float); }
 
+// terms (3 or 1) selects the fp16-split kernels' term count; the 3xTF32 kernels ignore it
 int tc_gemm_xw(const float* X, const int32_t* row_map, const float* scale, const float* shift, float slope,
                const float* W, float* H, void* workspace, int64_t workspace_bytes, int64_t n, int32_t Cin,
-               int32_t Cout, const float* amax, int64_t amax_len, cudaStream_t st) {
+               int32_t Cout, const float* amax, int64_t amax_len, int terms, cudaStream_t st) {
     DDMP_REQUIRE(tc_aligned16(X) && tc_aligned16(W) && tc_aligned16(H), "tc_gemm_xw: pointers must be 16-byte aligned");
     DDMP_REQUIRE(workspace && tc_aligned16(workspace) && workspace_bytes >= tc_gemm_nt_workspace_bytes(Cin, Cout),
                  "tc_gemm_xw: workspace too small");
     if (amax && amax_len > 0 && Cin % tc::BK16 == 0 && Cout % 64 == 0 && tc::f16_split_enabled())
-        return tc::run_nt16(X, row_map, scale, shift, slope, W, 0, workspace, H, n, Cout, Cin, amax, amax_len, st);
+        return tc::run_nt16(X, row_map, scale, shift, slope, W, 0, workspace, H, n, Cout, Cin, amax, amax_len, terms,
+                            st);
     return tc::run_nt2(X, row_map, scale, shift, slope, W, 0, workspace, H, n, Cout, Cin, st);
 }
 
 // gX[n,Cin] = dH[n,Cout] * W[Cout,Cin]: B operand (K-major) is W^T, built directly into the swizzled image.
 int tc_gemm_dx(const float* dH, const float* W, float* gX, void* workspace, int64_t workspace_bytes, int64_t n,
-               int32_t Cin, int32_t Cout, const float* amax, int64_t amax_len, cudaStream_t st) {
+               int32_t Cin, int32_t Cout, const float* amax, int64_t amax_len, int terms, cudaStream_t st) {
     DDMP_REQUIRE(tc_aligned16(dH) && tc_aligned16(W) && tc_aligned16(gX), "tc_gemm_dx: pointers must be 16-byte aligned");
     DDMP_REQUIRE(workspace && tc_aligned16(workspace) && workspace_bytes >= tc_gemm_nt_workspace_bytes(Cin, Cout),
                  "tc_gemm_dx: workspace too small");
     if (amax && amax_len > 0 && Cout % tc::BK16 == 0 && Cin % 64 == 0 && tc::f16_split_enabled())
-        return tc::run_nt16(dH, nullptr, nullptr, nullptr, 0.f, W, 1, workspace, gX, n, Cin, Cout, amax, amax_len, st);
+        return tc::run_nt16(dH, nullptr, nullptr, nullptr, 0.f, W, 1, workspace, gX, n, Cin, Cout, amax, amax_len,
+                            terms, st);
     return tc::run_nt2(dH, nullptr, nullptr, nullptr, 0.f, W, 1, workspace, gX, n, Cin, Cout, st);
 }
 
@@ -2393,7 +2511,8 @@ int64_t tc_gemm_dw_workspace_bytes(int64_t n, int32_t Cin, int32_t Cout) {
 
 int tc_gemm_dw(const float* dH, const float* X, const int32_t* row_map, const float* scale, const float* shift,
                float slope, float* dW, void* workspace, int64_t workspace_bytes, int64_t n, int32_t Cin, int32_t Cout,
-               const float* amax_dh, int64_t amax_dh_len, const float* amax_x, int64_t amax_x_len, cudaStream_t st) {
+               const float* amax_dh, int64_t amax_dh_len, const float* amax_x, int64_t amax_x_len, int terms,
+               cudaStream_t st) {
     DDMP_REQUIRE(row_map == nullptr, "tc_gemm_dw: row_map is only supported by the FFMA path");
     DDMP_REQUIRE(workspace && workspace_bytes >= tc_gemm_dw_workspace_bytes(n, Cin, Cout),
                  "tc_gemm_dw: workspace too small (%lld bytes)", (long long)workspace_bytes);
@@ -2410,16 +2529,9 @@ int tc_gemm_dw(const float* dH, const float* X, const int32_t* row_map, const fl
         h.rows = n; h.M = Cout; h.N = Cin;
         h.tiles_m = (int)ceil_div(Cout, tc::BM);
         const int64_t segs16 = ceil_div(n, tc::kSegRows);
-        int rc16;
         static const bool tn_one_cta = [] { const char* e = getenv("DDMP_TC_2CTA"); return e && e[0] == '0'; }();
-        if (!tn_one_cta && Cout % 256 == 0 && Cin % 256 == 0) {
-            h.tiles_m = Cout / 256;
-            if (Cin % 512 == 0) { h.tiles_n = Cin / 512; h.num_items = segs16 * h.tiles_m * h.tiles_n; rc16 = tc::launch_tn16x2<2>(h, st); }
-            else { h.tiles_n = Cin / 256; h.num_items = segs16 * h.tiles_m * h.tiles_n; rc16 = tc::launch_tn16x2<1>(h, st); }
-        }
-        else if (Cin % 256 == 0) { h.tiles_n = Cin / 256; h.num_items = segs16 * h.tiles_m * h.tiles_n; rc16 = tc::launch_tn16<256, 2>(h, st); }
-        else if (Cin % 128 == 0) { h.tiles_n = Cin / 128; h.num_items = segs16 * h.tiles_m * h.tiles_n; rc16 = tc::launch_tn16<128, 3>(h, st); }
-        else { h.tiles_n = Cin / 64; h.num_items = segs16 * h.tiles_m * h.tiles_n; rc16 = tc::launch_tn16<64, 4>(h, st); }
+        const int rc16 = terms == 1 ? tc::launch_tn16_choice<1>(h, segs16, tn_one_cta, st)
+                                    : tc::launch_tn16_choice<3>(h, segs16, tn_one_cta, st);
         if (rc16) return rc16;
         tc::seg_reduce_kernel<<<(unsigned)ceil_div(count, 32), 256, 0, st>>>(h.P, dW, count, segs16);
         return check_launch("tc seg_reduce");

@@ -18,6 +18,10 @@ SLOPE = 0.01        # nn.LeakyReLU() default (reference util/networks.py:44,105)
 BN_EPS = 1e-5
 BN_MOMENTUM = 0.1
 GEMM_BACKEND = 0    # DDMP_GEMM_AUTO; tests may set 1 (FFMA) / 2 (tcgen05)
+# accuracy contract of the dense transforms, chosen per call / per network (include/ddmp_b200.h DDMP_GEMM_F16X1):
+# "fp32" = the fp16-split tensor-core kernels emulate fp32 with three products (default); "f16x1" = one fp16 product
+GEMM_F16X1 = 0x10   # DDMP_GEMM_F16X1, OR-ed into the backend argument
+DENSE_PRECISIONS = ("fp32", "f16x1")
 # backward: recompute dY inside the aggregation kernel (ddmp_spmm_bn_bwd) instead of materialising it.  OFF: measured
 # on B200 at 1M faces the doubled gather volume through L2 costs more than the two saved passes over dY (C=512:
 # 1.82 vs 1.37 ms vertex graph, 2.87 vs 2.52 ms face graph; scripts/bench_bn_spmm.py) -- kept for narrower graphs.
@@ -67,6 +71,16 @@ def spmm_gcn(graph: GcnGraph, H, bias=None, stats=False, transposed=False, out=N
     return (Y, partials) if stats else Y
 
 
+def check_dense_precision(dense_precision: str) -> str:
+    if dense_precision not in DENSE_PRECISIONS:
+        raise ValueError(f"dense_precision must be one of {DENSE_PRECISIONS}, got {dense_precision!r}")
+    return dense_precision
+
+
+def _with_precision(backend: int, dense_precision: str) -> int:
+    return backend | GEMM_F16X1 if check_dense_precision(dense_precision) == "f16x1" else backend
+
+
 def _gemm_ws(n, Cin, Cout, device, backend):
     if backend == 1:
         return None, 0
@@ -76,38 +90,42 @@ def _gemm_ws(n, Cin, Cout, device, backend):
     return torch.empty(nbytes // 4, dtype=torch.float32, device=device), nbytes
 
 
-def gemm_xw(X, W, row_map=None, scale=None, shift=None, out=None, n=None, backend=None, amax=None):
-    """``amax``: optional device tensor whose largest magnitude bounds |act(X)| -> fp16-split tensor-core kernel"""
+def gemm_xw(X, W, row_map=None, scale=None, shift=None, out=None, n=None, backend=None, amax=None,
+            dense_precision="fp32"):
+    """``amax``: optional device tensor whose largest magnitude bounds |act(X)| -> fp16-split tensor-core kernel.
+    ``dense_precision="f16x1"``: that kernel runs with one fp16 product instead of three (no effect elsewhere)"""
     n = X.shape[0] if n is None else n
     Cout, Cin = W.shape
     H = out if out is not None else torch.empty(n, Cout, dtype=torch.float32, device=X.device)
     backend = GEMM_BACKEND if backend is None else backend
     ws, ws_bytes = _gemm_ws(n, Cin, Cout, X.device, backend)
     lib.call("ddmp_gemm_xw", ptr(X), ptr(row_map), ptr(scale), ptr(shift), SLOPE, ptr(W), ptr(H), ptr(ws), ws_bytes,
-             n, Cin, Cout, ptr(amax), 0 if amax is None else amax.numel(), backend, stream_ptr(X.device))
+             n, Cin, Cout, ptr(amax), 0 if amax is None else amax.numel(), _with_precision(backend, dense_precision),
+             stream_ptr(X.device))
     return H
 
 
-def gemm_dx(dH, W, out=None, backend=None, amax=None):
+def gemm_dx(dH, W, out=None, backend=None, amax=None, dense_precision="fp32"):
     n = dH.shape[0]
     Cout, Cin = W.shape
     gX = out if out is not None else torch.empty(n, Cin, dtype=torch.float32, device=dH.device)
     backend = GEMM_BACKEND if backend is None else backend
     ws, ws_bytes = _gemm_ws(n, Cin, Cout, dH.device, backend)
     lib.call("ddmp_gemm_dx", ptr(dH), ptr(W), ptr(gX), ptr(ws), ws_bytes, n, Cin, Cout, ptr(amax),
-             0 if amax is None else amax.numel(), backend, stream_ptr(dH.device))
+             0 if amax is None else amax.numel(), _with_precision(backend, dense_precision), stream_ptr(dH.device))
     return gX
 
 
-def gemm_dw(dH, X, Cin, row_map=None, scale=None, shift=None, backend=None, amax_dh=None, amax_x=None):
+def gemm_dw(dH, X, Cin, row_map=None, scale=None, shift=None, backend=None, amax_dh=None, amax_x=None,
+            dense_precision="fp32"):
     n, Cout = dH.shape
     dW = torch.empty(Cout, Cin, dtype=torch.float32, device=dH.device)
     ws_bytes = int(lib.query("ddmp_gemm_dw_workspace_bytes", n, Cin, Cout))
     ws = torch.empty(max(ws_bytes, 16) // 4, dtype=torch.float32, device=dH.device)
     lib.call("ddmp_gemm_dw", ptr(dH), ptr(X), ptr(row_map), ptr(scale), ptr(shift), SLOPE, ptr(dW), ptr(ws),
              ws_bytes, n, Cin, Cout, ptr(amax_dh), 0 if amax_dh is None else amax_dh.numel(), ptr(amax_x),
-             0 if amax_x is None else amax_x.numel(), GEMM_BACKEND if backend is None else backend,
-             stream_ptr(dH.device))
+             0 if amax_x is None else amax_x.numel(),
+             _with_precision(GEMM_BACKEND if backend is None else backend, dense_precision), stream_ptr(dH.device))
     return dW
 
 
@@ -287,9 +305,11 @@ class GCNConvFunction(torch.autograd.Function):
 # whole network: 12 GCN layers + head
 # ---------------------------------------------------------------------------------------------------------------------
 class GcnNetFunction(torch.autograd.Function):
-    """forward(graph, kind, training, bn_buffers, taps, x_in, x_pos, *params)
+    """forward(graph, kind, training, bn_buffers, taps, x_in, x_pos, *params[, dense_precision])
 
     params = [W_1, b_1, gamma_1, beta_1, ..., W_12, b_12, gamma_12, beta_12, W_lin1, b_lin1, W_lin2, b_lin2]
+    dense_precision: optional trailing string, "fp32" (default) or "f16x1"; passed to every trunk GEMM of the forward
+    and the backward (the layers whose fp16-split tensor-core kernels it affects: DDMP_GEMM_F16X1).
     bn_buffers = [(running_mean_l, running_var_l)] updated in place (training) or read (eval).
     taps: optional list that receives (Y_l, stats_l) per layer, then (h_head, None), for the per-layer parity tests.
     """
@@ -298,6 +318,10 @@ class GcnNetFunction(torch.autograd.Function):
     def forward(ctx, graph: GcnGraph, kind: int, training: bool, bn_buffers, taps, x_in, x_pos, *params):
         dev = x_in.device
         set_device(dev)
+        ctx.has_precision = bool(params) and isinstance(params[-1], str)
+        dense = check_dense_precision(params[-1]) if ctx.has_precision else "fp32"
+        if ctx.has_precision:
+            params = params[:-1]
         n = graph.n
         x_in = _f32(x_in, "net input")
         L = (len(params) - 4) // 4
@@ -317,10 +341,10 @@ class GcnNetFunction(torch.autograd.Function):
             cout = Ws[l].shape[0]
             H = Hbuf[: n_ext * cout].view(n_ext, cout)               # [owned | halo] rows
             if l == 0:
-                gemm_xw(x_in, Ws[0], row_map=graph.perm, out=H, n=n)
+                gemm_xw(x_in, Ws[0], row_map=graph.perm, out=H, n=n, dense_precision=dense)
             else:
                 gemm_xw(Ys[l - 1], Ws[l], scale=stats[l - 1][2], shift=stats[l - 1][3], out=H,
-                        amax=act_bound(stats[l - 1]))
+                        amax=act_bound(stats[l - 1]), dense_precision=dense)
             if comm is not None:
                 comm.exchange(H)
             if training:
@@ -355,6 +379,7 @@ class GcnNetFunction(torch.autograd.Function):
         ctx.graph, ctx.kind, ctx.L = graph, kind, L
         ctx.Ys, ctx.stats, ctx.h_save, ctx.t_save = Ys, stats, h_save, t_save
         ctx.training = training
+        ctx.dense_precision = dense
         return out
 
     @staticmethod
@@ -363,7 +388,7 @@ class GcnNetFunction(torch.autograd.Function):
             raise RuntimeError("backward through eval-mode BatchNorm is not part of the Dual-DMP hot path")
         saved = ctx.saved_tensors
         x_in, Ws, W1, W2 = saved[0], saved[1:1 + ctx.L], saved[-2], saved[-1]
-        graph, L, kind = ctx.graph, ctx.L, ctx.kind
+        graph, L, kind, dense = ctx.graph, ctx.L, ctx.kind, ctx.dense_precision
         Ys, stats = ctx.Ys, ctx.stats
         dev = g_out.device
         set_device(dev)
@@ -411,12 +436,12 @@ class GcnNetFunction(torch.autograd.Function):
                 else:
                     spmm_gcn(graph, dY, transposed=True, out=dH, n_rows=n)
             if l == 0:
-                gW = gemm_dw(dH, x_in, cin, row_map=graph.perm)
+                gW = gemm_dw(dH, x_in, cin, row_map=graph.perm, dense_precision=dense)
             else:
                 gW = gemm_dw(dH, Ys[l - 1], cin, scale=stats[l - 1][2], shift=stats[l - 1][3], amax_dh=dh_max,
-                             amax_x=act_bound(stats[l - 1]) if dh_max is not None else None)
+                             amax_x=act_bound(stats[l - 1]) if dh_max is not None else None, dense_precision=dense)
                 gX = bufA[: n * cin].view(n, cin)
-                gemm_dx(dH, Ws[l], out=gX, amax=dh_max)
+                gemm_dx(dH, Ws[l], out=gX, amax=dh_max, dense_precision=dense)
             grads[4 * l: 4 * l + 4] = [gW, dbias, dgamma, dbeta]
         g_xpos = g_out if (kind == HEAD_POS and ctx.needs_input_grad[6]) else None
         ctx.Ys = ctx.stats = ctx.h_save = ctx.t_save = None
@@ -431,7 +456,7 @@ class GcnNetFunction(torch.autograd.Function):
                 k = all_grads[i].numel()
                 all_grads[i] = flat[off: off + k].view_as(all_grads[i])
                 off += k
-        return (None, None, None, None, None, None, g_xpos, *all_grads)
+        return (None, None, None, None, None, None, g_xpos, *all_grads) + ((None,) if ctx.has_precision else ())
 
 
 # ---------------------------------------------------------------------------------------------------------------------

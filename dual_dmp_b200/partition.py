@@ -273,7 +273,7 @@ class PartitionedNet(torch.nn.Module):
         bns = [getattr(net, f"bn{i}") for i in range(1, 13)]
         buffers = [(bn.running_mean, bn.running_var) for bn in bns]
         out_own = F_.GcnNetFunction.apply(pg, net.KIND, net.training, buffers, net.taps, x_own, xpos_own,
-                                          *net._params())
+                                          *net._params(), F_.check_dense_precision(net.dense_precision))
         net.last_graph = pg
         if net.training:
             torch._foreach_add_([bn.num_batches_tracked for bn in bns], 1)

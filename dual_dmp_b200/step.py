@@ -22,10 +22,13 @@ from .util import loss as L
 class DualStep:
     def __init__(self, posnet, normnet, dataset, n_mesh, k=(3.0, 4.0, 4.0, 4.0, 1.0), bnfloop=1, pos_lr=0.01,
                  norm_lr=0.01, grad_clip=0.8, bnf_warmup_epochs=100, capture=True, overlap=True,
-                 fused_optimizer=True, fused_loss=True):
+                 fused_optimizer=True, fused_loss=True, dense_precision=None):
+        """``dense_precision``: None keeps each network's ``dense_precision`` attribute; "fp32" or "f16x1" sets it on
+        both (util.networks: the accuracy contract of the dense transforms' tensor-core kernels)."""
         dev = torch.device(posnet.device)
         if dev.type != "cuda":
             raise RuntimeError("DualStep runs on CUDA only (dual_dmp_b200 has no CPU path)")
+        set_dense_precision((posnet, normnet), dense_precision)
         self.device = dev
         self.posnet, self.normnet, self.mesh = posnet, normnet, n_mesh
         self.k, self.bnfloop, self.grad_clip = tuple(float(x) for x in k), int(bnfloop), float(grad_clip)
@@ -174,6 +177,16 @@ class DualStep:
         return self._static_loss[bnf_off]
 
 
+def set_dense_precision(nets, dense_precision) -> None:
+    """set ``dense_precision`` ("fp32" | "f16x1") on every network; None leaves them as they are"""
+    if dense_precision is None:
+        return
+    from .functional import check_dense_precision
+    check_dense_precision(dense_precision)
+    for net in nets:
+        net.dense_precision = dense_precision
+
+
 class FusedAdam:
     """``clip_grad_norm_`` + ``torch.optim.Adam`` of one network as two library kernels over flat buffers
     (reference main.py:108-110; SURVEY.md §8f N1).  The parameters of ``module`` are re-pointed at views of one flat
@@ -307,7 +320,8 @@ class MultiDualStep(DualStep):
     per phase like ``DualStep``.  Every fit's numbers equal those of its own ``DualStep`` bit for bit.
 
     ``fits``: one dict per mesh with ``posnet``, ``normnet``, ``dataset``, ``n_mesh`` and optionally ``k``, ``pos_lr``,
-    ``norm_lr``, ``grad_clip`` and ``bnfloop`` (the defaults of ``DualStep``).  All fits share ``bnfloop``: a batch that
+    ``norm_lr``, ``grad_clip``, ``bnfloop`` and ``dense_precision`` (the defaults of ``DualStep``; fits may differ in
+    ``dense_precision``).  All fits share ``bnfloop``: a batch that
     mixes values is rejected, run it as two batches.  ``step(epoch)`` returns the per-fit totals ``[B]`` (float64);
     ``.pos[i]``, ``.norm[i]``, ``.parts[i]`` are fit ``i``'s outputs."""
 
@@ -326,6 +340,8 @@ class MultiDualStep(DualStep):
             raise ValueError(f"MultiDualStep: the fits are on several devices {sorted(map(str, devs))}; one batch "
                              "runs on one device")
         dev = devs.pop()
+        for f in fits:
+            set_dense_precision((f["posnet"], f["normnet"]), f.get("dense_precision"))
         self.device = dev
         self.bnfloop = loops.pop()
         self.bnf_warmup_epochs = int(bnf_warmup_epochs)

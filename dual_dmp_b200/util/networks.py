@@ -64,6 +64,9 @@ class _Net(nn.Module):
         self.reorder = True          # Morton-sort the graph (set False to keep the caller's numbering)
         self.taps = None             # set to a list to collect (Y_l, stats_l) of every layer (parity tests)
         self.last_graph = None       # GcnGraph used by the most recent forward (holds the row permutation)
+        # accuracy contract of the trunk's dense transforms: "fp32" (default; fp32-accurate products) or "f16x1" (one
+        # fp16 product on the tensor-core layers with operand bounds, DDMP_GEMM_F16X1 in include/ddmp_b200.h)
+        self.dense_precision = "fp32"
 
     def _params(self):
         p = []
@@ -82,7 +85,7 @@ class _Net(nn.Module):
         bns = [getattr(self, f"bn{i}") for i in range(1, 13)]
         buffers = [(bn.running_mean, bn.running_var) for bn in bns]
         out = F_.GcnNetFunction.apply(graph, self.KIND, self.training, buffers, self.taps, x_in.detach(), x_pos,
-                                      *self._params())
+                                      *self._params(), F_.check_dense_precision(self.dense_precision))
         if self.training:
             torch._foreach_add_([bn.num_batches_tracked for bn in bns], 1)
         return out

@@ -34,6 +34,16 @@ extern "C" {
 #define DDMP_GEMM_AUTO 0
 #define DDMP_GEMM_FFMA 1  /* fp32 FFMA kernel                                  */
 #define DDMP_GEMM_TC 2    /* tcgen05 tensor cores, 3xTF32 split, fp32 accumulate */
+/* Modifier bit, OR-ed into the `backend` argument of ddmp_gemm_xw / _dx / _dw: a lower-precision accuracy contract
+ * chosen per call.  Wherever the call would run a 3-term fp16-split tcgen05 kernel (hi*hi + hi*lo + lo*hi, i.e. on
+ * the tensor-core path and with operand bounds: `amax` for xw / dx, both `amax_dh` and `amax_x` for dw), it runs the
+ * 1-term kernel of the same shape choice instead: one fp16 product hi*hi per element pair, hi = fp16(s*x) with the
+ * same power-of-two scale s, fp32 accumulation.  Each product then has a relative error of at most 2^-10 + 2^-22
+ * (u = 2^-11 per rounding; plus 2^-25 / s absolute per operand element whose scaled magnitude is below 2^-14).
+ * Calls the bit does NOT affect (bitwise the same result with or without it): the FFMA kernels (widths < 64 under
+ * AUTO, DDMP_GEMM_FFMA, the narrow dW shapes, row_map in dW), the 3xTF32 tensor-core kernels (calls without an
+ * operand bound, e.g. the first layer, widths that are not multiples of 64, or DDMP_TC_SPLIT=tf32 set). */
+#define DDMP_GEMM_F16X1 0x10
 
 #define DDMP_HEAD_POS 0
 #define DDMP_HEAD_NORM 1

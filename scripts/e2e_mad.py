@@ -79,8 +79,9 @@ def run_oracle(case, k, bnfloop, iters, seed, threads, log):
             "seconds": time.perf_counter() - t0}
 
 
-def run_product(case, k, bnfloop, iters, seed, path, log, perturb=0):
-    """``perturb`` > 0: every initial weight is multiplied by (1 + 1e-7 * N(0,1)) drawn with that seed -- a rounding-level
+def run_product(case, k, bnfloop, iters, seed, path, log, perturb=0, dense_precision="fp32"):
+    """``dense_precision``: the networks' dense-transform accuracy contract ("fp32" | "f16x1", util.networks).
+    ``perturb`` > 0: every initial weight is multiplied by (1 + 1e-7 * N(0,1)) drawn with that seed -- a rounding-level
     perturbation, like the reduction-order changes that distinguish the oracle's own runs; the chaotic fit turns it into
     an independent trajectory, which gives the (otherwise bitwise deterministic) product an ensemble"""
     from dual_dmp_b200.step import DualStep
@@ -94,6 +95,7 @@ def run_product(case, k, bnfloop, iters, seed, path, log, perturb=0):
     posnet, normnet = PosNet(dev).to(dev), NormalNet(dev).to(dev)
     posnet.load_state_dict(pos_ref.state_dict())
     normnet.load_state_dict(nrm_ref.state_dict())
+    posnet.dense_precision = normnet.dense_precision = dense_precision
     if perturb:
         g = torch.Generator(device="cpu").manual_seed(1000 + int(perturb))
         with torch.no_grad():
@@ -140,7 +142,7 @@ def run_product(case, k, bnfloop, iters, seed, path, log, perturb=0):
                 if epoch % 100 == 0:
                     log(f"product epoch {epoch:4d} loss {float(loss):.6f} MAD {curve[-1]:.4f} "
                         f"normnet-MAD {norm_curve[-1]:.4f} ({time.perf_counter() - t0:.0f} s)")
-    return {"mad": curve, "normnet_mad": norm_curve, "loss": losses, "path": path,
+    return {"mad": curve, "normnet_mad": norm_curve, "loss": losses, "path": path, "dense_precision": dense_precision,
             "seconds": time.perf_counter() - t0}
 
 
@@ -163,6 +165,8 @@ def main():
     ap.add_argument("--threads", type=int, default=min(8, os.cpu_count() or 1))
     ap.add_argument("--path", default="dualstep", choices=["dualstep", "dropin"])
     ap.add_argument("--out", default=None)
+    ap.add_argument("--dense-precision", default="fp32", choices=["fp32", "f16x1"],
+                    help="product arm: accuracy contract of the dense transforms (DESIGN.md 4.2)")
     args = ap.parse_args()
     from tests.helpers import small_case
     case = small_case("ico", args.n)
@@ -174,7 +178,8 @@ def main():
     if args.arm in ("oracle", "both"):
         out["oracle"] = run_oracle(case, k, bnfloop, args.iters, args.seed, args.threads, log)
     if args.arm in ("product", "both"):
-        out["product"] = run_product(case, k, bnfloop, args.iters, args.seed, args.path, log)
+        out["product"] = run_product(case, k, bnfloop, args.iters, args.seed, args.path, log,
+                                     dense_precision=args.dense_precision)
     if args.arm == "both":
         out["compare"] = compare(out["product"], out["oracle"])
         log(json.dumps(out["compare"]))

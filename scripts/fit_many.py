@@ -40,6 +40,9 @@ def get_parser() -> argparse.ArgumentParser:
     p.add_argument("--grad_crip", type=float, default=0.8)
     p.add_argument("--bnfloop", type=int, default=1)
     p.add_argument("--batch", type=int, default=8, help=BATCH_HELP)
+    p.add_argument("--dense-precision", default="fp32", choices=["fp32", "f16x1"],
+                   help="accuracy contract of the networks' dense transforms: fp32 (default) or f16x1 (one fp16 product "
+                        "on the tensor-core layers; DESIGN.md 4.2)")
     return p
 
 
@@ -96,7 +99,8 @@ def fit_batch(dirs, args, device) -> list:
         out_dir = os.path.join(d, "output")
         os.makedirs(out_dir, exist_ok=True)
         fits.append(dict(posnet=PosNet(device).to(device), normnet=NormalNet(device).to(device), dataset=dataset,
-                         n_mesh=n_mesh, k=k, pos_lr=args.pos_lr, norm_lr=args.norm_lr, grad_clip=args.grad_crip))
+                         n_mesh=n_mesh, k=k, pos_lr=args.pos_lr, norm_lr=args.norm_lr, grad_clip=args.grad_crip,
+                         dense_precision=args.dense_precision))
         mad = Loss.mad(n_mesh.fn, gt.fn) if gt is not None else None
         meta.append(dict(input=d, out_dir=out_dir, gt=gt, o1=o1, initial_mad=mad, mad=mad))
     step = MultiDualStep(fits, bnfloop=args.bnfloop)
