@@ -108,11 +108,7 @@ int ddmp_rows_per_block(int32_t C) {
     // 128 rows per CTA for the wide layers, 256 for the narrow ones: >= 3,900 CTAs at 1M rows (a grid of 980 CTAs,
     // as with 1024 rows per block, leaves a mostly empty second wave: ncu, profiles/)
     // 128 rows per CTA from width 64 up (tile-staged kernel at C = 64: 32 KB tile, 5 CTAs per SM -- 2.6-2.9 / 4.2-4.8 TB/s
-    // on the vertex / face graph against 1.9 / 3.2 with 256 rows; DDMP_RPB64=256 restores the old block)
-    if (C == 64) {
-        static const int rpb64 = [] { const char* e = getenv("DDMP_RPB64"); return (e && atoi(e) == 256) ? 256 : 128; }();
-        return rpb64;
-    }
+    // on the vertex / face graph against 1.9 / 3.2 with 256 rows)
     return C <= 32 ? 256 : 128;
 }
 

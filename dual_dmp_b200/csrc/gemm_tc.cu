@@ -643,7 +643,7 @@ struct Nt16Args {
     const float* amax;       // bound of |act(A)|: max over this array
     int64_t amax_len;
     unsigned long long* trace;   // profiling only (DDMP_TC_TRACE=1): per-role cycle counters of CTA 0
-    int flags;               // DDMP_TC_F16_FLAGS. bit 0: prefetch the next tile's A rows into L2; bit 3: unstaged epilogue
+    int flags;               // ddmp_gemm_tc_flags: bit 3 unstaged epilogue, bit 4 staged epilogue, bit 5 register-fed A
     int64_t M;
     int N, K;
     int tiles_n;
@@ -659,19 +659,6 @@ constexpr int kProdNJ = BM * 16 / kProducerThreads;      // rows per thread per 
 constexpr int kProdRPP = kProducerThreads / 16;          // rows covered by one pass of the producer threads (16)
 __device__ __forceinline__ void sts64(uint32_t saddr, uint32_t x, uint32_t y) {
     asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(saddr), "r"(x), "r"(y) : "memory");
-}
-// A k-block touches 256 bytes of each of the tile's 128 rows (stride K*4), and the next 256 bytes of the same rows a
-// microsecond later: DRAM sees short scattered bursts (measured: every shape of the fp16-split kernel ran at
-// ~3.6 TB/s of operand + result traffic).  Pulling the NEXT tile's rows into L2 as whole rows while the current tile
-// is multiplied makes the DRAM reads long and sequential and turns the producers' loads into L2 hits.
-template <class Args>
-__device__ __forceinline__ void prefetch_tile_l2(const Args& g, int64_t m0) {
-    const int t = threadIdx.x;
-    if (t >= BM) return;
-    const int64_t m = m0 + t;
-    if (m >= g.M) return;
-    const int64_t r = g.a_map ? (int64_t)__ldg(g.a_map + m) : m;
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(g.A + r * g.K), "r"((uint32_t)g.K * 4u) : "memory");
 }
 // 16-byte read-only load the compiler may not move: the prefetch below depends on the loads of the NEXT k-block being
 // issued before the current one is transformed (plain __ldg loads get sunk below the transform to save registers).
@@ -709,8 +696,6 @@ __device__ __forceinline__ void produce_loop(const Args& g, int64_t first_tile, 
             const int64_t r = (m < g.M) ? (g.a_map ? (int64_t)__ldg(g.a_map + m) : m) : -1;
             rp[j] = r >= 0 ? g.A + r * g.K + c8 : nullptr;
         }
-        if ((g.flags & 1) && tile + tile_step < g.num_tiles)
-            prefetch_tile_l2(g, ((tile + tile_step) / g.tiles_n) * row_mul + row_add);
     };
     auto load = [&](float4 (&buf)[NJ], uint32_t& vmask, int& k0) {
         k0 = lc_kb * BK16;
@@ -1581,33 +1566,27 @@ static int launch_nt16x2(const Nt16Args& g0, cudaStream_t st) {
     return check_launch("tc_gemm_nt16x2");
 }
 
-// switches of the fp16-split NT kernels (environment DDMP_TC_F16_FLAGS, ddmp_gemm_tc_flags): bit 0 = prefetch the next
-// tile's A rows into L2, bit 1 = the same for K <= 256 only, bit 3 = unstaged epilogue, bit 4 = staged ld.shared + st.global
-// epilogue instead of TMA stores, bit 5 = the previous configuration (register-fed A operand everywhere, CTA pairs for
-// every N % 256 == 0)
+// switches of the fp16-split NT kernels (environment DDMP_TC_F16_FLAGS, ddmp_gemm_tc_flags): bit 3 = unstaged epilogue
+// (15-40 % slower), bit 4 = staged ld.shared + st.global epilogue instead of TMA stores, bit 5 = the previous
+// configuration (register-fed A operand everywhere, CTA pairs for every N % 256 == 0)
 int f16_flags(int set) {
     static std::atomic<int> v{-1};
     int cur = v.load(std::memory_order_relaxed);
     if (cur < 0) {
         const char* e = getenv("DDMP_TC_F16_FLAGS");
-        cur = e ? (atoi(e) & 0xffff) : 0;
+        cur = e ? (atoi(e) & 56) : 0;
         v.store(cur, std::memory_order_relaxed);
     }
-    if (set >= 0) v.store(set & 0xffff, std::memory_order_relaxed);
+    if (set >= 0) v.store(set & 56, std::memory_order_relaxed);
     return cur;
 }
 
-static bool f16_split_enabled() {
-    static const bool v = [] { const char* e = getenv("DDMP_TC_SPLIT"); return !(e && e[0] == 't'); }();   // "tf32"
-    return v;
-}
-
 // the shape choice of run_nt16 for one term count; TERMS = 1 halves a split stage, so the same shared memory holds
-// twice as many of them (a deeper pipeline; raw A slots, accumulator ring and staging unchanged)
+// twice as many of them (a deeper pipeline; raw A slots, accumulator ring and staging unchanged).  256-wide tiles run
+// on CTA pairs (half the weight stream per CTA; never slower than one CTA per 256-wide tile, profiles/README.md)
 template <int TERMS>
-static int launch_nt16_choice(const Nt16Args& g, int BN, bool tma_a, bool one_cta, cudaStream_t st) {
+static int launch_nt16_choice(const Nt16Args& g, int BN, bool tma_a, cudaStream_t st) {
     constexpr int D = TERMS == 3 ? 1 : 2;
-    if (BN == 256 && one_cta) return launch_nt16<256, 2 * D, 0, 2, TERMS>(g, st);
     if (tma_a) {                                     // one split stage traded for the raw fp32 slots
         if (BN == 256) return launch_nt16x2<2 * D, 2, TERMS>(g, st);
         if (BN == 128) return launch_nt16<128, 2 * D, 2, 4, TERMS>(g, st);
@@ -1622,8 +1601,7 @@ static int launch_nt16_choice(const Nt16Args& g, int BN, bool tma_a, bool one_ct
 static int run_nt16(const float* A, const int* a_map, const float* scale, const float* shift, float slope,
                     const float* W, int transposed, void* workspace, float* C, int64_t M, int N, int K,
                     const float* amax, int64_t amax_len, int terms, cudaStream_t st) {
-    int flags = f16_flags(-1);
-    if ((flags & 2) && K <= 256) flags |= 1;         // bit 1: the L2 prefetch only where it measured faster (K <= 256)
+    const int flags = f16_flags(-1);
     // (TMA tensor coordinates are 32-bit: row counts near 2^31 keep the register-fed producers)
     // TMA-fed A (DESIGN.md §4.2): at K <= 256, and at K = 512 when the BatchNorm + LeakyReLU prologue is fused (there
     // the transform makes the register-fed producers the bound); without the prologue the producers keep pace at
@@ -1671,9 +1649,8 @@ static int run_nt16(const float* A, const int* a_map, const float* scale, const 
     g.M = M; g.N = N; g.K = K; g.tiles_n = N / BN;
     g.num_tiles = ceil_div(M, BM) * g.tiles_n;
     DDMP_REQUIRE(g.num_tiles < (1ll << 31), "tc gemm: too many tiles");
-    static const bool one_cta = [] { const char* e = getenv("DDMP_TC_2CTA"); return e && e[0] == '0'; }();
-    if (terms == 1) return dump_trace(launch_nt16_choice<1>(g, BN, tma_a, one_cta, st));
-    return dump_trace(launch_nt16_choice<3>(g, BN, tma_a, one_cta, st));
+    if (terms == 1) return dump_trace(launch_nt16_choice<1>(g, BN, tma_a, st));
+    return dump_trace(launch_nt16_choice<3>(g, BN, tma_a, st));
 }
 
 // ---- TN kernel (dW) -------------------------------------------------------------------------------------------------
@@ -1903,8 +1880,11 @@ seg_reduce_kernel(const float* __restrict__ partials, float* __restrict__ out, i
     }
 }
 
-template <int BN, int STAGES, int PW>
-static int launch_tn_impl(const TnArgs& g, cudaStream_t st) {
+// producer warps: both operands are split in flight here, so the transform is issue-bound with 8 warps at BN >= 128
+// (ncu: 42 % issue utilisation, tensor pipe 45 %); 16 warps there
+template <int BN, int STAGES>
+static int launch_tn(const TnArgs& g, cudaStream_t st) {
+    constexpr int PW = BN >= 128 ? 16 : 8;
     constexpr size_t smem = (size_t)STAGES * (2 * BM * 128 + 2 * BN * 128) + 1024 + 256;
     static PerDeviceOnce configured;
     if (configured.need()) {
@@ -1915,14 +1895,6 @@ static int launch_tn_impl(const TnArgs& g, cudaStream_t st) {
     const int64_t grid = g.num_items < kNumSMs ? g.num_items : kNumSMs;
     tc_gemm_tn_kernel<BN, STAGES, PW><<<(unsigned)grid, PW * 32 + 32, smem, st>>>(g);
     return check_launch("tc_gemm_tn");
-}
-// producer warps: both operands are split in flight here, so the transform is issue-bound with 8 warps (ncu: 42 %
-// issue utilisation, tensor pipe 45 %); DDMP_TC_TN_WARPS=8 restores the narrow version for A/B runs
-template <int BN, int STAGES>
-static int launch_tn(const TnArgs& g, cudaStream_t st) {
-    static const int pw = [] { const char* e = getenv("DDMP_TC_TN_WARPS"); return (e && atoi(e) == 8) ? 8 : 16; }();
-    if (pw == 16 && BN >= 128) return launch_tn_impl<BN, STAGES, 16>(g, st);
-    return launch_tn_impl<BN, STAGES, 8>(g, st);
 }
 
 // ---- TN kernel (dW), fp16 split --------------------------------------------------------------------------------------
@@ -2446,10 +2418,10 @@ static int launch_tn16x2(const Tn16Args& g, cudaStream_t st) {
 // the tile choice of tc_gemm_dw's fp16-split path for one term count (h: shape fields set, tiles_m = ceil(Cout / 128));
 // TERMS = 1 doubles the split stages in the same shared memory
 template <int TERMS>
-static int launch_tn16_choice(Tn16Args& h, int64_t segs, bool one_cta, cudaStream_t st) {
+static int launch_tn16_choice(Tn16Args& h, int64_t segs, cudaStream_t st) {
     constexpr int D = TERMS == 3 ? 1 : 2;
     const int Cout = h.M, Cin = h.N;
-    if (!one_cta && Cout % 256 == 0 && Cin % 256 == 0) {
+    if (Cout % 256 == 0 && Cin % 256 == 0) {          // CTA pairs: 1.3-1.4x faster than one-CTA tiles
         h.tiles_m = Cout / 256;
         if (Cin % 512 == 0) { h.tiles_n = Cin / 512; h.num_items = segs * h.tiles_m * h.tiles_n; return launch_tn16x2<2, TERMS>(h, st); }
         h.tiles_n = Cin / 256; h.num_items = segs * h.tiles_m * h.tiles_n; return launch_tn16x2<1, TERMS>(h, st);
@@ -2487,7 +2459,7 @@ int tc_gemm_xw(const float* X, const int32_t* row_map, const float* scale, const
     DDMP_REQUIRE(tc_aligned16(X) && tc_aligned16(W) && tc_aligned16(H), "tc_gemm_xw: pointers must be 16-byte aligned");
     DDMP_REQUIRE(workspace && tc_aligned16(workspace) && workspace_bytes >= tc_gemm_nt_workspace_bytes(Cin, Cout),
                  "tc_gemm_xw: workspace too small");
-    if (amax && amax_len > 0 && Cin % tc::BK16 == 0 && Cout % 64 == 0 && tc::f16_split_enabled())
+    if (amax && amax_len > 0 && Cin % tc::BK16 == 0 && Cout % 64 == 0)
         return tc::run_nt16(X, row_map, scale, shift, slope, W, 0, workspace, H, n, Cout, Cin, amax, amax_len, terms,
                             st);
     return tc::run_nt2(X, row_map, scale, shift, slope, W, 0, workspace, H, n, Cout, Cin, st);
@@ -2499,7 +2471,7 @@ int tc_gemm_dx(const float* dH, const float* W, float* gX, void* workspace, int6
     DDMP_REQUIRE(tc_aligned16(dH) && tc_aligned16(W) && tc_aligned16(gX), "tc_gemm_dx: pointers must be 16-byte aligned");
     DDMP_REQUIRE(workspace && tc_aligned16(workspace) && workspace_bytes >= tc_gemm_nt_workspace_bytes(Cin, Cout),
                  "tc_gemm_dx: workspace too small");
-    if (amax && amax_len > 0 && Cout % tc::BK16 == 0 && Cin % 64 == 0 && tc::f16_split_enabled())
+    if (amax && amax_len > 0 && Cout % tc::BK16 == 0 && Cin % 64 == 0)
         return tc::run_nt16(dH, nullptr, nullptr, nullptr, 0.f, W, 1, workspace, gX, n, Cin, Cout, amax, amax_len,
                             terms, st);
     return tc::run_nt2(dH, nullptr, nullptr, nullptr, 0.f, W, 1, workspace, gX, n, Cin, Cout, st);
@@ -2519,19 +2491,15 @@ int tc_gemm_dw(const float* dH, const float* X, const int32_t* row_map, const fl
     DDMP_REQUIRE(tc_aligned16(dH) && tc_aligned16(X) && tc_aligned16(workspace), "tc_gemm_dw: 16-byte alignment");
     const int64_t count = (int64_t)Cin * Cout;
     // fp16 split: 10-30 % faster than 3xTF32 on every shape (1M rows: 512->512 2.39 vs 2.71 ms, 64->128 0.27 vs 0.36);
-    // both operands are split by the producer warps here, which bounds this kernel.  DDMP_TC_TN16=0 -> 3xTF32
-    static const bool tn16_off = [] { const char* e = getenv("DDMP_TC_TN16"); return e && e[0] == '0'; }();
-    if (amax_dh && amax_x && amax_dh_len > 0 && amax_x_len > 0 && Cout % 4 == 0 && tc::f16_split_enabled() &&
-        !tn16_off) {
+    // both operands are split by the producer warps here, which bounds this kernel
+    if (amax_dh && amax_x && amax_dh_len > 0 && amax_x_len > 0 && Cout % 4 == 0) {
         tc::Tn16Args h{};
         h.A = dH; h.B = X; h.P = reinterpret_cast<float*>(workspace); h.scale = scale; h.shift = shift; h.slope = slope;
         h.amax_a = amax_dh; h.amax_a_len = amax_dh_len; h.amax_b = amax_x; h.amax_b_len = amax_x_len;
         h.rows = n; h.M = Cout; h.N = Cin;
         h.tiles_m = (int)ceil_div(Cout, tc::BM);
         const int64_t segs16 = ceil_div(n, tc::kSegRows);
-        static const bool tn_one_cta = [] { const char* e = getenv("DDMP_TC_2CTA"); return e && e[0] == '0'; }();
-        const int rc16 = terms == 1 ? tc::launch_tn16_choice<1>(h, segs16, tn_one_cta, st)
-                                    : tc::launch_tn16_choice<3>(h, segs16, tn_one_cta, st);
+        const int rc16 = terms == 1 ? tc::launch_tn16_choice<1>(h, segs16, st) : tc::launch_tn16_choice<3>(h, segs16, st);
         if (rc16) return rc16;
         tc::seg_reduce_kernel<<<(unsigned)ceil_div(count, 32), 256, 0, st>>>(h.P, dW, count, segs16);
         return check_launch("tc seg_reduce");

@@ -498,7 +498,6 @@ int spmm_tile_launch(const int* rowptr, const int* col, const float* w, const fl
     tile::Args a{rowptr, col, w, H, bias, Y, partials, amax, n, C};
     const int rpb = ddmp_rows_per_block(C);               // the BatchNorm partials are laid out per row block
     if (C == 32 && rpb == 256) return tile::launch<32, 256>(a, st);
-    if (C == 64 && rpb == 256) return tile::launch<64, 256>(a, st);
     if (C == 64 && rpb == 128) return tile::launch<64, 128>(a, st);
     if (C >= 128 && rpb == 128) return tile::launch<128, 128>(a, st);
     set_error("spmm_tile: no instantiation for C=%d rows_per_block=%d", C, rpb);

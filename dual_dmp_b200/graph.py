@@ -39,45 +39,10 @@ def morton_order(coords: np.ndarray) -> np.ndarray:
     return np.argsort(code, kind="stable").astype(np.int64)
 
 
-def hilbert_order(coords: np.ndarray, bits: int = 20) -> np.ndarray:
-    """Permutation (new -> old) that sorts points along a 3-D Hilbert curve (``bits`` bits per axis, Skilling's
-    axes-to-transpose construction, vectorised); ties broken by original id.  Consecutive cells of a Hilbert curve are
-    always face-adjacent, so a run of consecutive rows is one connected patch -- a Morton run falls apart into distant
-    pieces wherever it crosses a high-order cell boundary, and the rows gathered across such a break miss L2."""
-    c = np.asarray(coords, dtype=np.float64)
-    lo, hi = c.min(axis=0), c.max(axis=0)
-    span = np.where(hi > lo, hi - lo, 1.0)
-    q = np.floor((c - lo) / span * float((1 << bits) - 1)).astype(np.uint64)
-    X = [q[:, 0].copy(), q[:, 1].copy(), q[:, 2].copy()]
-    one = np.uint64(1)
-    Q = one << np.uint64(bits - 1)
-    while Q > one:                                   # inverse undo
-        P = Q - one
-        for i in range(3):
-            hit = (X[i] & Q) != 0
-            t = np.where(hit, np.uint64(0), (X[0] ^ X[i]) & P)
-            X[0] = np.where(hit, X[0] ^ P, X[0] ^ t)
-            X[i] = X[i] ^ t
-        Q >>= one
-    X[1] ^= X[0]                                     # Gray encode
-    X[2] ^= X[1]
-    t = np.zeros_like(X[0])
-    Q = one << np.uint64(bits - 1)
-    while Q > one:
-        t = np.where((X[2] & Q) != 0, t ^ (Q - one), t)
-        Q >>= one
-    code = (_part1by2(X[0] ^ t) << np.uint64(2)) | (_part1by2(X[1] ^ t) << np.uint64(1)) | _part1by2(X[2] ^ t)
-    return np.argsort(code, kind="stable").astype(np.int64)
-
-
 def sfc_order(coords: np.ndarray) -> np.ndarray:
-    """Row order of the reordered graphs: Morton curve; ``DDMP_SFC=hilbert`` selects the Hilbert curve.  On the 1M-face
-    benchmark graphs the two are equivalent for the aggregation kernels (out-of-block references 14.8 / 15.1 % face,
-    18.0 / 18.3 % vertex graph; 4,036 vs 4,044 GB/s step-weighted, profiles/spmm_slice_ab_r2.txt), so the cheaper key
-    stays the default."""
-    import os
-    if os.environ.get("DDMP_SFC", "morton").lower() == "hilbert":
-        return hilbert_order(coords)
+    """Row order of the reordered graphs: Morton curve.  On the 1M-face benchmark graphs a Hilbert curve is equivalent
+    for the aggregation kernels (out-of-block references 14.8 / 15.1 % face, 18.0 / 18.3 % vertex graph; 4,036 vs 4,044
+    GB/s step-weighted, profiles/spmm_slice_ab_r2.txt) and its key costs more to build."""
     return morton_order(coords)
 
 

@@ -42,7 +42,7 @@ extern "C" {
  * (u = 2^-11 per rounding; plus 2^-25 / s absolute per operand element whose scaled magnitude is below 2^-14).
  * Calls the bit does NOT affect (bitwise the same result with or without it): the FFMA kernels (widths < 64 under
  * AUTO, DDMP_GEMM_FFMA, the narrow dW shapes, row_map in dW), the 3xTF32 tensor-core kernels (calls without an
- * operand bound, e.g. the first layer, widths that are not multiples of 64, or DDMP_TC_SPLIT=tf32 set). */
+ * operand bound, e.g. the first layer, or widths that are not multiples of 64). */
 #define DDMP_GEMM_F16X1 0x10
 
 #define DDMP_HEAD_POS 0
@@ -171,9 +171,11 @@ int ddmp_gemm_xw(const float* X, const int32_t* row_map, const float* scale, con
 /* scratch the tensor-core path of gemm_xw / gemm_dx needs for the pre-split, pre-swizzled weight image (0 when the
  * shape runs on the FFMA kernel; with workspace == NULL the FFMA kernel is used). */
 int64_t ddmp_gemm_workspace_bytes(int64_t n, int32_t Cin, int32_t Cout);
-/* A/B switches of the fp16-split tcgen05 kernels behind ddmp_gemm_xw / ddmp_gemm_dx (environment DDMP_TC_F16_FLAGS,
- * default 0): bit 0 = prefetch the next tile's rows into L2, bit 3 = unstaged epilogue, bit 4 = staged ld.shared +
- * st.global epilogue instead of TMA tensor stores.  flags < 0 only queries.  Returns the previous value. */
+/* Alternative configurations of the fp16-split tcgen05 kernels behind ddmp_gemm_xw / ddmp_gemm_dx (environment
+ * DDMP_TC_F16_FLAGS, default 0; bitwise the same results as the default): bit 3 (8) = unstaged thread-per-row
+ * epilogue; bit 4 (16) = staged ld.shared + st.global epilogue instead of TMA tensor stores; bit 5 (32) = A operand by
+ * the register-fed producers everywhere (no TMA A operand).  Other bits are ignored.  flags < 0 only queries.
+ * Returns the previous value. */
 int ddmp_gemm_tc_flags(int flags);
 /* gX[n,Cin] = dH[n,Cout] * W[Cout,Cin]. */
 int ddmp_gemm_dx(const float* dH, const float* W, float* gX, void* workspace, int64_t workspace_bytes, int64_t n,

@@ -1,5 +1,6 @@
 """A/B of the fp16-split NT kernels (X.W^T and dH.W) at the 1M-face shapes: ddmp_gemm_tc_flags settings given on the command
-line (default: 0 = TMA-store epilogue, 16 = staged epilogue), interleaved per shape in ONE process."""
+line (0 = the default configuration, 16 = staged epilogue instead of TMA stores, 32 = register-fed A operand everywhere;
+default: 0 16), interleaved per shape in ONE process."""
 import os, sys, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch

@@ -1,8 +1,9 @@
 """A/B of the two pipeline configurations of the fp16-split NT kernels (X.W^T and dH.W) at the 1M-face shapes.
 
   ab     [--flags F ...] [--reps R]   ddmp_gemm_tc_flags settings interleaved per shape and per repetition in ONE process
-                                     (default 32 = register-fed A operand everywhere, 0 = the selection of run_nt16); the L2
-                                     is overwritten before every timed call; median ms, and the share of the shape's floor
+                                     (0 = the selection of run_nt16, 16 = staged epilogue instead of TMA stores, 32 =
+                                     register-fed A operand everywhere; default: 32 0); the L2 is overwritten before
+                                     every timed call; median ms, and the share of the shape's floor
   trace  [--flags F]                 DDMP_TC_TRACE=1 cycle counters of CTA 0, one line per shape (stderr of the library)
 
 The floor of a call is the larger of its HBM bytes (A read + C written) / 6.55 TB/s (measured copy peak of the B200)

@@ -105,18 +105,14 @@ def test_reference_functions_outside_the_hot_path_refuse_loudly():
             getattr(L, name)(None, None)
 
 
-def test_space_filling_curve_orders():
-    """graph.hilbert_order (opt-in, DDMP_SFC=hilbert): consecutive cells of a full grid are face-adjacent (the defining
-    property of the Hilbert curve); graph.morton_order (default): the Z-order key; both are permutations with stable ties"""
+def test_morton_order():
+    """graph.morton_order (the row order of the reordered graphs): the Z-order key, a permutation with stable ties"""
     import numpy as np
-    from dual_dmp_b200.graph import hilbert_order, morton_order
+    from dual_dmp_b200.graph import morton_order
     b = 3
     g = np.stack(np.meshgrid(*[np.arange(1 << b)] * 3, indexing="ij"), -1).reshape(-1, 3).astype(float)
-    p = hilbert_order(g, bits=b)
-    assert sorted(p.tolist()) == list(range(len(g)))
-    assert (np.abs(np.diff(g[p], axis=0)).sum(1) == 1).all()
     q = morton_order(g)
     assert sorted(q.tolist()) == list(range(len(g)))
-    assert np.abs(np.diff(g[q], axis=0)).sum(1).max() > 1          # Z-order jumps, Hilbert does not
+    assert np.abs(np.diff(g[q], axis=0)).sum(1).max() > 1          # Z-order jumps between cells
     dup = np.concatenate([g[:5], g[:5]])
-    assert hilbert_order(dup, bits=b).tolist()[:2] == [0, 5] or set(hilbert_order(dup, bits=b)[:2].tolist()) == {0, 5}
+    assert morton_order(dup).tolist()[:2] == [0, 5]
