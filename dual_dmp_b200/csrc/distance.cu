@@ -25,6 +25,7 @@ namespace dist {
 
 constexpr int kT = 256;
 constexpr int kMaxBlocks = 1024;
+static_assert(kT == DDMP_DISTANCE_THREADS && kMaxBlocks == DDMP_DISTANCE_MAX_BLOCKS, "batched block counts (header)");
 // A root-to-leaf path visits internal nodes whose split prefix lengths strictly increase.  Keys use 63 of 64 bits (the
 // root's prefix is >= 1) and a tie between equal keys adds 64 + clz32(i ^ j) <= 95, so a path holds at most 95
 // internal nodes and a stack of 96 entries cannot overflow.
@@ -123,11 +124,44 @@ topology_kernel(const int64_t* __restrict__ keys, const int64_t* __restrict__ or
     parent[c1 < 0 ? F - 1 + ~c1 : c1] = (int)(i << 1 | 1);
 }
 
-// bottom-up refit, one thread per leaf; counters [F-1] are zero on entry and zero again on exit
-__global__ void __launch_bounds__(kT)
-refit_kernel(const double* __restrict__ vs, const int4* __restrict__ leaves, Node* nodes, const int* __restrict__ parent,
-             unsigned* counters, int64_t F) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+// Where a kernel body reads its block range.  A stand-alone kernel gives its one input the whole grid; a batched kernel
+// (one launch over the rows of a descriptor table) gives each row the blocks its stand-alone launch would have, and the
+// body sees row-local block ids and block count, so every partition and every order of summation stays the same.
+struct WholeGrid {
+    __device__ __forceinline__ unsigned blk() const { return blockIdx.x; }
+    __device__ __forceinline__ unsigned nblk() const { return gridDim.x; }
+};
+__shared__ unsigned s_range[2];          // batched kernels: the block's index within its row, the row's block count
+struct RowRange {
+    __device__ __forceinline__ unsigned blk() const { return s_range[0]; }
+    __device__ __forceinline__ unsigned nblk() const { return s_range[1]; }
+};
+
+// Batched kernels: rows of W int64 words in block order, word 0 = the row's first block, word 1 = its block count (a
+// row may own no block).  Thread 0 finds the row that owns this block (the last one whose first block is <= it) and
+// fills s_range; every thread gets the row after the barrier.
+template <int W>
+__device__ __forceinline__ const int64_t* claim_row(const int64_t* __restrict__ table, int n) {
+    __shared__ int s_row;
+    if (threadIdx.x == 0) {
+        int m = 0;
+        while (m + 1 < n && table[(int64_t)(m + 1) * W] <= (int64_t)blockIdx.x) ++m;
+        s_row = m;
+        s_range[0] = blockIdx.x - (unsigned)table[(int64_t)m * W];
+        s_range[1] = (unsigned)table[(int64_t)m * W + 1];
+    }
+    __syncthreads();
+    return table + (int64_t)s_row * W;
+}
+template <class T>
+__device__ __forceinline__ T* word_ptr(const int64_t* row, int k) { return reinterpret_cast<T*>(row[k]); }
+
+// bottom-up refit, one thread per leaf; counters [F-1] are zero on entry and zero again on exit.  Only the boxes change:
+// the leaves hold corner ids, so a tree built once refits to any new positions of the same mesh.
+template <class Range>
+__device__ __forceinline__ void refit_body(const Range rg, const double* __restrict__ vs, const int4* __restrict__ leaves,
+                                           Node* nodes, const int* __restrict__ parent, unsigned* counters, int64_t F) {
+    const int64_t i = (int64_t)rg.blk() * blockDim.x + threadIdx.x;
     if (i >= F) return;
     const int4 lf = leaves[i];
     float b[6];
@@ -155,6 +189,19 @@ refit_kernel(const double* __restrict__ vs, const int4* __restrict__ leaves, Nod
         if ((p >> 1) == 0) return;   // root: its own box is never read
         p = parent[p >> 1];
     }
+}
+
+__global__ void __launch_bounds__(kT)
+refit_kernel(const double* __restrict__ vs, const int4* __restrict__ leaves, Node* nodes, const int* __restrict__ parent,
+             unsigned* counters, int64_t F) {
+    refit_body(WholeGrid{}, vs, leaves, nodes, parent, counters, F);
+}
+
+__global__ void __launch_bounds__(kT)
+refit_multi_kernel(const int64_t* __restrict__ table, int n) {
+    const int64_t* r = claim_row<DDMP_BVH_REFIT_DESC_WORDS>(table, n);
+    refit_body(RowRange{}, word_ptr<const double>(r, 2), word_ptr<const int4>(r, 3), word_ptr<Node>(r, 4),
+               word_ptr<const int>(r, 5), word_ptr<unsigned>(r, 6), r[7]);
 }
 
 struct V3 {
@@ -238,10 +285,12 @@ __device__ __forceinline__ float box_lb2(const float* plo, const float* phi, con
     return s;
 }
 
-__global__ void __launch_bounds__(kT)
-query_kernel(const double* __restrict__ pts, int64_t P, const double* __restrict__ vs, const Node* __restrict__ nodes,
-             const int4* __restrict__ leaves, int64_t F, double* __restrict__ dist, int* __restrict__ face) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+template <class Range>
+__device__ __forceinline__ void query_body(const Range rg, const double* __restrict__ pts, int64_t P,
+                                           const double* __restrict__ vs, const Node* __restrict__ nodes,
+                                           const int4* __restrict__ leaves, int64_t F, double* __restrict__ dist,
+                                           int* __restrict__ face) {
+    const int64_t i = (int64_t)rg.blk() * blockDim.x + threadIdx.x;
     if (i >= P) return;
     const V3 p = {pts[3 * i], pts[3 * i + 1], pts[3 * i + 2]};
     double best = CUDART_INF;   // +inf
@@ -309,6 +358,19 @@ query_kernel(const double* __restrict__ pts, int64_t P, const double* __restrict
 }
 
 __global__ void __launch_bounds__(kT)
+query_kernel(const double* __restrict__ pts, int64_t P, const double* __restrict__ vs, const Node* __restrict__ nodes,
+             const int4* __restrict__ leaves, int64_t F, double* __restrict__ dist, int* __restrict__ face) {
+    query_body(WholeGrid{}, pts, P, vs, nodes, leaves, F, dist, face);
+}
+
+__global__ void __launch_bounds__(kT)
+query_multi_kernel(const int64_t* __restrict__ table, int n) {
+    const int64_t* r = claim_row<DDMP_DISTANCE_DESC_WORDS>(table, n);
+    query_body(RowRange{}, word_ptr<const double>(r, 2), r[3], word_ptr<const double>(r, 4), word_ptr<const Node>(r, 5),
+               word_ptr<const int4>(r, 6), r[7], word_ptr<double>(r, 8), word_ptr<int>(r, 9));
+}
+
+__global__ void __launch_bounds__(kT)
 exhaustive_kernel(const double* __restrict__ pts, int64_t P, const double* __restrict__ vs, const int* __restrict__ faces,
                   int64_t F, double* __restrict__ dist, int* __restrict__ face) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -324,11 +386,11 @@ exhaustive_kernel(const double* __restrict__ pts, int64_t P, const double* __res
 }
 
 // (min, max, sum, sum of squares) of dist[0..P); per-block partials, the last block combines them in block order
-__global__ void __launch_bounds__(kT)
-stats_kernel(const double* __restrict__ d, int64_t P, double* out, Scratch* sc) {
-    __shared__ double sm[4][kT / 32];
+template <class Range>
+__device__ __forceinline__ void stats_body(const Range rg, const double* __restrict__ d, int64_t P, double* out,
+                                           Scratch* sc, double (*sm)[kT / 32]) {
     double lo = CUDART_INF, hi = -CUDART_INF, s = 0.0, s2 = 0.0;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < P; i += (int64_t)gridDim.x * blockDim.x) {
+    for (int64_t i = (int64_t)rg.blk() * blockDim.x + threadIdx.x; i < P; i += (int64_t)rg.nblk() * blockDim.x) {
         const double x = d[i];
         lo = fmin(lo, x);
         hi = fmax(hi, x);
@@ -351,16 +413,76 @@ stats_kernel(const double* __restrict__ d, int64_t P, double* out, Scratch* sc) 
         const int q = threadIdx.x;
         double r = sm[q][0];
         for (int w = 1; w < kT / 32; ++w) r = q == 0 ? fmin(r, sm[q][w]) : q == 1 ? fmax(r, sm[q][w]) : r + sm[q][w];
-        sc->partials[q][blockIdx.x] = r;
+        sc->partials[q][rg.blk()] = r;
     }
-    if (publish_and_am_last(&sc->ticket, gridDim.x) && threadIdx.x < 4) {
+    if (publish_and_am_last(&sc->ticket, rg.nblk()) && threadIdx.x < 4) {
         const int q = threadIdx.x;
         double r = __ldcg(&sc->partials[q][0]);
-        for (unsigned b = 1; b < gridDim.x; ++b) {
+        for (unsigned b = 1; b < rg.nblk(); ++b) {
             const double x = __ldcg(&sc->partials[q][b]);
             r = q == 0 ? fmin(r, x) : q == 1 ? fmax(r, x) : r + x;
         }
         out[q] = r;
+    }
+}
+
+__global__ void __launch_bounds__(kT)
+stats_kernel(const double* __restrict__ d, int64_t P, double* out, Scratch* sc) {
+    __shared__ double sm[4][kT / 32];
+    stats_body(WholeGrid{}, d, P, out, sc, sm);
+}
+
+__global__ void __launch_bounds__(kT)
+stats_multi_kernel(const int64_t* __restrict__ table, int n) {
+    __shared__ double sm[4][kT / 32];
+    const int64_t* r = claim_row<DDMP_DISTANCE_STATS_DESC_WORDS>(table, n);
+    stats_body(RowRange{}, word_ptr<const double>(r, 2), r[3], word_ptr<double>(r, 4), word_ptr<Scratch>(r, 5), sm);
+}
+
+// Evaluation of one fit's positions (float32 [V,3]) against its clean mesh, run by the row's blocks:
+//   vs64 = the positions widened to float64 (the points and the vertex array of the fit's output tree);
+//   mad  = mean over faces of the angle in degrees between the face normal of the positions and the clean normal.
+// The face normal is the float32 arithmetic of util/mesh.py compute_face_normals on float32 positions: np.cross,
+// np.linalg.norm (squares summed in axis order, sqrt) + 1e-24, division; this file is compiled without multiply-add
+// contraction, so each product and difference rounds on its own as in numpy.  The angle is util/loss.py mad's float64
+// clip / arccos / rad2deg; the per-block partial sums are combined by the row's last block in block order.
+__global__ void __launch_bounds__(kT)
+eval_multi_kernel(const int64_t* __restrict__ table, int n) {
+    const int64_t* r = claim_row<DDMP_EVAL_DESC_WORDS>(table, n);
+    const float* __restrict__ pos = word_ptr<const float>(r, 2);
+    const int* __restrict__ faces = word_ptr<const int>(r, 3);
+    const double* __restrict__ gt_fn = word_ptr<const double>(r, 4);
+    double* __restrict__ vs64 = word_ptr<double>(r, 5);
+    Scratch* sc = word_ptr<Scratch>(r, 7);
+    const int64_t V = r[8], F = r[9];
+    const RowRange rg;
+    const int64_t tid = (int64_t)rg.blk() * kT + threadIdx.x, nth = (int64_t)rg.nblk() * kT;
+    for (int64_t e = tid; e < 3 * V; e += nth) vs64[e] = (double)pos[e];
+    double acc = 0.0;
+    for (int64_t f = tid; f < F; f += nth) {
+        float p[3][3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const int64_t v = faces[3 * f + c];
+#pragma unroll
+            for (int a = 0; a < 3; ++a) p[c][a] = pos[3 * v + a];
+        }
+        const float u[3] = {p[1][0] - p[0][0], p[1][1] - p[0][1], p[1][2] - p[0][2]};
+        const float w[3] = {p[2][0] - p[0][0], p[2][1] - p[0][1], p[2][2] - p[0][2]};
+        const float cx = u[1] * w[2] - u[2] * w[1], cy = u[2] * w[0] - u[0] * w[2], cz = u[0] * w[1] - u[1] * w[0];
+        const float len = sqrtf(cx * cx + cy * cy + cz * cz) + 1e-24f;
+        const float nx = cx / len, ny = cy / len, nz = cz / len;
+        double inner = (double)nx * gt_fn[3 * f] + (double)ny * gt_fn[3 * f + 1] + (double)nz * gt_fn[3 * f + 2];
+        inner = inner < -1.0 ? -1.0 : (inner > 1.0 ? 1.0 : inner);
+        acc += acos(inner) * (180.0 / 3.14159265358979323846);
+    }
+    __shared__ double sm[kT / 32];
+    const double b = block_sum<kT>(acc, sm);
+    if (threadIdx.x == 0) sc->partials[0][rg.blk()] = b;
+    if (publish_and_am_last(&sc->ticket, rg.nblk()) && threadIdx.x == 0) {
+        double t = 0.0;
+        for (unsigned k = 0; k < rg.nblk(); ++k) t += __ldcg(&sc->partials[0][k]);
+        *word_ptr<double>(r, 6) = t / (double)F;
     }
 }
 
@@ -418,6 +540,42 @@ int ddmp_distance_stats(const double* dist, int64_t P, double* out, void* scratc
     DDMP_REQUIRE(dist && out && scratch && P > 0, "distance_stats: bad arguments");
     dist::stats_kernel<<<dist::grid_for(P), dist::kT, 0, as_stream(stream)>>>(dist, P, out, (dist::Scratch*)scratch);
     return check_launch("distance_stats");
+}
+
+int ddmp_bvh_refit(const double* vs, const int32_t* leaves, void* nodes, const int32_t* parent, int32_t* counters,
+                   int64_t F, void* stream) {
+    using namespace ddmp;
+    DDMP_REQUIRE(vs && leaves && nodes && parent && counters && F > 0 && F < ((int64_t)1 << 30),
+                 "bvh_refit: bad arguments");
+    DDMP_REQUIRE(((uintptr_t)nodes & 63) == 0 && ((uintptr_t)leaves & 15) == 0, "bvh_refit: nodes / leaves misaligned");
+    if (F == 1) return DDMP_OK;   // a single leaf: no internal node holds a box
+    dist::refit_kernel<<<(unsigned)ceil_div(F, dist::kT), dist::kT, 0, as_stream(stream)>>>(
+        vs, (const int4*)leaves, (dist::Node*)nodes, parent, (unsigned*)counters, F);
+    return check_launch("bvh_refit");
+}
+
+static int launch_multi(void (*kernel)(const int64_t*, int), const int64_t* table, int32_t n, int64_t blocks,
+                        void* stream, const char* what) {
+    using namespace ddmp;
+    DDMP_REQUIRE(table && n > 0 && blocks > 0 && blocks < ((int64_t)1 << 31), "%s: bad arguments", what);
+    kernel<<<(unsigned)blocks, dist::kT, 0, as_stream(stream)>>>(table, n);
+    return check_launch(what);
+}
+
+int ddmp_bvh_refit_multi(const int64_t* table, int32_t n, int64_t blocks, void* stream) {
+    return launch_multi(ddmp::dist::refit_multi_kernel, table, n, blocks, stream, "bvh_refit_multi");
+}
+
+int ddmp_point_mesh_distance_multi(const int64_t* table, int32_t n, int64_t blocks, void* stream) {
+    return launch_multi(ddmp::dist::query_multi_kernel, table, n, blocks, stream, "point_mesh_distance_multi");
+}
+
+int ddmp_distance_stats_multi(const int64_t* table, int32_t n, int64_t blocks, void* stream) {
+    return launch_multi(ddmp::dist::stats_multi_kernel, table, n, blocks, stream, "distance_stats_multi");
+}
+
+int ddmp_eval_mad_multi(const int64_t* table, int32_t n, int64_t blocks, void* stream) {
+    return launch_multi(ddmp::dist::eval_multi_kernel, table, n, blocks, stream, "eval_mad_multi");
 }
 
 }  // extern "C"

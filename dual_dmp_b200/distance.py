@@ -103,10 +103,23 @@ class MeshBVH:
         n_int = max(self.F - 1, 1)
         self.nodes = torch.empty(n_int * _NODE_BYTES // 4, dtype=torch.int32, device=dev)
         self.leaves = torch.empty(self.F, 4, dtype=torch.int32, device=dev)
-        parent = torch.empty(2 * self.F - 1, dtype=torch.int32, device=dev)
-        counters = torch.zeros(n_int, dtype=torch.int32, device=dev)
+        self.parent = torch.empty(2 * self.F - 1, dtype=torch.int32, device=dev)
+        self.counters = torch.zeros(n_int, dtype=torch.int32, device=dev)        # kept zeroed for refit
         lib.call("ddmp_bvh_build", ptr(self.vs), ptr(self.faces), ptr(keys), ptr(order), ptr(self.nodes),
-                 ptr(self.leaves), ptr(parent), ptr(counters), self.F, st)
+                 ptr(self.leaves), ptr(self.parent), ptr(self.counters), self.F, st)
+
+    def refit(self, vs) -> None:
+        """Move the tree to new positions ``vs`` [V,3] of the same mesh: ``.vs`` and ``.bbox`` take the new values and
+        the node boxes are recomputed over the kept topology.  Queries stay exact; only their speed depends on how well
+        the topology, built for the first positions, fits the new ones."""
+        vs = _coords(vs, "vs")
+        if vs.shape[0] != self.V:
+            raise ValueError(f"refit: expected {self.V} vertices, got {vs.shape[0]}")
+        self.vs.copy_(_to64(vs, self.device))
+        st = self._stream()
+        lib.call("ddmp_prep_bbox", ptr(self.vs), ptr(self.bbox), ptr(self._scratch), self.V, st)
+        lib.call("ddmp_bvh_refit", ptr(self.vs), ptr(self.leaves), ptr(self.nodes), ptr(self.parent),
+                 ptr(self.counters), self.F, st)
 
     def _stream(self) -> int:
         set_device(self.device)
@@ -188,3 +201,137 @@ def hausdorff(a, b, device=None) -> dict:
     return {"a_to_b": ab, "b_to_a": ba, "hausdorff": h, "mean": mean, "diag": diag,
             "hausdorff_rel": h / diag if diag > 0 else float("nan"),
             "mean_rel": mean / diag if diag > 0 else float("nan")}
+
+
+# batched evaluation (include/ddmp_b200.h, "Batched evaluation of many fits"): table widths and block counts
+THREADS, MAX_BLOCKS = 256, 1024     # DDMP_DISTANCE_THREADS, DDMP_DISTANCE_MAX_BLOCKS
+EVAL_WORDS = 10                     # DDMP_EVAL_DESC_WORDS
+REFIT_WORDS = 8                     # DDMP_BVH_REFIT_DESC_WORDS
+QUERY_WORDS = 10                    # DDMP_DISTANCE_DESC_WORDS
+STATS_WORDS = 6                     # DDMP_DISTANCE_STATS_DESC_WORDS
+
+
+def _blocks(n: int, capped: bool) -> int:
+    b = -(-int(n) // THREADS)
+    return min(b, MAX_BLOCKS) if capped else b
+
+
+def block_table(rows, counts) -> tuple[np.ndarray, int]:
+    """rows [n, W] (words 2.. filled in) with words 0 / 1 set to each row's first block and block count; the total"""
+    t = np.array(rows, dtype=np.int64)
+    counts = np.asarray(counts, dtype=np.int64)
+    t[:, 1] = counts
+    t[:, 0] = np.concatenate([[0], np.cumsum(counts)[:-1]])
+    return t, int(counts.sum())
+
+
+class BatchEvaluator:
+    """Evaluation of B fits on one device in a fixed number of launches: per fit, the MAD of the current positions'
+    face normals against the clean mesh's (``Loss.mad`` of ``Mesh.compute_face_normals`` on the float32 positions) and
+    the two-sided distance of ``hausdorff(positions, clean)``.
+
+    ``meshes[i]``: fit i's mesh (``.vs``, ``.faces``: topology and starting positions); ``gts[i]``: its clean mesh
+    (``.vs``, ``.faces``, ``.fn`` float64 unit face normals, the same faces as ``meshes[i]``).  The clean meshes' trees
+    are built once; each fit's output tree is built once on its starting positions and refit at every evaluation.
+    ``evaluate`` needs no host synchronisation and does no per-fit host work beyond writing a table when the
+    positions' addresses change."""
+
+    def __init__(self, meshes, gts, device=None):
+        from .multi import DeviceTables
+        if len(meshes) != len(gts) or not meshes:
+            raise ValueError(f"BatchEvaluator: expected one clean mesh per fit, got {len(meshes)} fits and "
+                             f"{len(gts)} clean meshes")
+        self.device = dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        if dev.type != "cuda":
+            raise RuntimeError(f"BatchEvaluator runs on CUDA only (dual_dmp_b200 has no CPU path), got device {dev}")
+        self.B = B = len(meshes)
+        self.out = [MeshBVH(m.vs, m.faces, dev) for m in meshes]
+        self.gt = [MeshBVH(g.vs, g.faces, dev) for g in gts]
+        self.gt_fn = []
+        for i, (o, g, gm) in enumerate(zip(self.out, self.gt, gts)):
+            fn = np.asarray(gm.fn, dtype=np.float64)
+            if o.F != g.F or fn.shape != (g.F, 3):
+                raise ValueError(f"BatchEvaluator: fit {i} has {o.F} faces, its clean mesh {g.F} faces and "
+                                 f"{fn.shape[0]} normals")
+            self.gt_fn.append(torch.from_numpy(np.ascontiguousarray(fn)).to(dev))
+        # diag as hausdorff() computes it, on the host once
+        diag = []
+        for g in self.gt:
+            bb = g.bbox.tolist()
+            diag.append(math.sqrt(sum((bb[3 + k] - bb[k]) ** 2 for k in range(3))))
+        self.diag = torch.tensor(diag, dtype=torch.float64, device=dev)
+        slot = int(lib.query("ddmp_distance_scratch_bytes"))
+        slot = -(-slot // 256) * 256
+        self._scratch = torch.zeros(3 * B * slot // 8, dtype=torch.float64, device=dev)   # B eval slots, 2B stats slots
+        sc = lambda k: self._scratch.data_ptr() + k * slot                                 # noqa: E731
+        self.mad = torch.empty(B, dtype=torch.float64, device=dev)
+        self.stats = torch.empty(2 * B, 4, dtype=torch.float64, device=dev)     # rows 2i: a_to_b, 2i+1: b_to_a
+        P = [n for o, g in zip(self.out, self.gt) for n in (o.V, g.V)]
+        offs = np.concatenate([[0], np.cumsum(P)])
+        self._dist = torch.empty(int(offs[-1]), dtype=torch.float64, device=dev)
+        self._face = torch.empty(int(offs[-1]), dtype=torch.int32, device=dev)
+        #: per fit (dist a_to_b, face a_to_b, dist b_to_a, face b_to_a) of the last evaluation
+        self.distances = [(self._dist[offs[2 * i]:offs[2 * i + 1]], self._face[offs[2 * i]:offs[2 * i + 1]],
+                           self._dist[offs[2 * i + 1]:offs[2 * i + 2]], self._face[offs[2 * i + 1]:offs[2 * i + 2]])
+                          for i in range(B)]
+        self.counts = torch.tensor(P, dtype=torch.float64, device=dev).view(B, 2)
+        self._tables = DeviceTables(dev)
+        refit, q, s = [], [], []
+        for i, (o, g) in enumerate(zip(self.out, self.gt)):
+            refit.append([0, 0, ptr(o.vs), ptr(o.leaves), ptr(o.nodes), ptr(o.parent), ptr(o.counters), o.F])
+            d_ab, f_ab, d_ba, f_ba = self.distances[i]
+            q.append([0, 0, ptr(o.vs), o.V, ptr(g.vs), ptr(g.nodes), ptr(g.leaves), g.F, ptr(d_ab), ptr(f_ab)])
+            q.append([0, 0, ptr(g.vs), g.V, ptr(o.vs), ptr(o.nodes), ptr(o.leaves), o.F, ptr(d_ba), ptr(f_ba)])
+            s.append([0, 0, ptr(d_ab), o.V, ptr(self.stats[2 * i]), sc(B + 2 * i)])
+            s.append([0, 0, ptr(d_ba), g.V, ptr(self.stats[2 * i + 1]), sc(B + 2 * i + 1)])
+        rows, self._refit_blocks = block_table(refit, [_blocks(o.F, False) if o.F > 1 else 0 for o in self.out])
+        self._refit = self._tables.put("refit", rows)
+        rows, self._query_blocks = block_table(q, [_blocks(n, False) for n in P])
+        self._query = self._tables.put("query", rows)
+        rows, self._stats_blocks = block_table(s, [_blocks(n, True) for n in P])
+        self._stats_t = self._tables.put("stats", rows)
+        self._eval_rows = [[0, 0, 0, ptr(o.faces), ptr(fn), ptr(o.vs), ptr(self.mad[i]), sc(i), o.V, o.F]
+                           for i, (o, fn) in enumerate(zip(self.out, self.gt_fn))]
+        self._eval_blocks = [_blocks(max(o.V, o.F), True) for o in self.out]
+        self._eval_key = None
+
+    def evaluate(self, positions) -> dict:
+        """positions: B float32 CUDA tensors [V_i, 3] (e.g. ``MultiDualStep.pos``).  Returns device tensors [B]:
+        ``mad``; ``a_to_b`` / ``b_to_a``, each ``{min, max, mean, rms}``; ``hausdorff``, ``mean``, ``diag``,
+        ``hausdorff_rel``, ``mean_rel``, with the meanings of ``hausdorff(positions, clean)``."""
+        if len(positions) != self.B:
+            raise ValueError(f"evaluate: expected {self.B} position tensors, got {len(positions)}")
+        for i, (p, o) in enumerate(zip(positions, self.out)):
+            if not (isinstance(p, torch.Tensor) and p.is_cuda and p.dtype == torch.float32):
+                raise RuntimeError(f"evaluate: positions {i} must be a float32 CUDA tensor (dual_dmp_b200 has no CPU "
+                                   "path)")
+            if p.device != self.device or tuple(p.shape) != (o.V, 3) or not p.is_contiguous():
+                raise ValueError(f"evaluate: positions {i} must be a contiguous [{o.V}, 3] tensor on {self.device}, "
+                                 f"got {tuple(p.shape)} on {p.device}")
+        key = tuple(p.data_ptr() for p in positions)
+        if key != self._eval_key:
+            for row, k in zip(self._eval_rows, key):
+                row[2] = k
+            rows, self._eval_total = block_table(self._eval_rows, self._eval_blocks)
+            self._eval = self._tables.put("eval", rows)
+            self._eval_key = key
+        set_device(self.device)
+        st = stream_ptr(self.device)
+        B = self.B
+        lib.call("ddmp_eval_mad_multi", ptr(self._eval), B, self._eval_total, st)
+        if self._refit_blocks:
+            lib.call("ddmp_bvh_refit_multi", ptr(self._refit), B, self._refit_blocks, st)
+        lib.call("ddmp_point_mesh_distance_multi", ptr(self._query), 2 * B, self._query_blocks, st)
+        lib.call("ddmp_distance_stats_multi", ptr(self._stats_t), 2 * B, self._stats_blocks, st)
+        s = self.stats.view(B, 2, 4)
+        mean = s[:, :, 2] / self.counts
+        rms = torch.sqrt(s[:, :, 3] / self.counts)
+        side = [{"min": s[:, k, 0].clone(), "max": s[:, k, 1].clone(), "mean": mean[:, k], "rms": rms[:, k]}
+                for k in range(2)]
+        h = torch.maximum(side[0]["max"], side[1]["max"])
+        m = 0.5 * (mean[:, 0] + mean[:, 1])
+        ok = self.diag > 0
+        nan = torch.full_like(h, float("nan"))
+        return {"mad": self.mad.clone(), "a_to_b": side[0], "b_to_a": side[1], "hausdorff": h, "mean": m,
+                "diag": self.diag.clone(), "hausdorff_rel": torch.where(ok, h / self.diag, nan),
+                "mean_rel": torch.where(ok, m / self.diag, nan)}

@@ -282,6 +282,43 @@ int ddmp_point_mesh_distance_exhaustive(const double* points, int64_t P, const d
  * ddmp_distance_scratch_bytes() bytes, left zeroed. */
 int64_t ddmp_distance_scratch_bytes(void);
 int ddmp_distance_stats(const double* dist, int64_t P, double* out, void* scratch, void* stream);
+/* Recompute the boxes of a tree built by ddmp_bvh_build for new positions vs of the same mesh (same V, faces): the
+ * leaves hold corner ids, so the topology is kept and only the boxes change.  parent and counters are the arrays the
+ * build was given, kept with the tree (counters zero on entry and left zeroed).  Query results stay exact for any
+ * positions (the pruning needs only boxes rounded outward around their triangles); only their speed depends on how
+ * well the kept topology fits the new positions. */
+int ddmp_bvh_refit(const double* vs, const int32_t* leaves, void* nodes, const int32_t* parent, int32_t* counters,
+                   int64_t F, void* stream);
+
+/* Batched evaluation of many fits (csrc/distance.cu).  Each *_multi call is ONE launch of 256-thread blocks over the n
+ * rows of a DEVICE table of int64 words.  Word 0 of a row is its first block, word 1 its block count; rows own
+ * consecutive block ranges in table order and `blocks` is the sum of the counts.  A row's count is the grid of the
+ * stand-alone launch for its input (given below), and the row runs the stand-alone arithmetic with row-local block ids,
+ * so each row's results equal the stand-alone call bit for bit.  Pointers are device addresses stored as int64. */
+#define DDMP_DISTANCE_THREADS 256
+#define DDMP_DISTANCE_MAX_BLOCKS 1024
+/* ddmp_bvh_refit per row; blocks = ceil(F / 256) if F > 1, else 0.
+ *   2 vs   3 leaves   4 nodes   5 parent   6 counters   7 F */
+#define DDMP_BVH_REFIT_DESC_WORDS 8
+int ddmp_bvh_refit_multi(const int64_t* table, int32_t n, int64_t blocks, void* stream);
+/* ddmp_point_mesh_distance per row; blocks = ceil(P / 256).
+ *   2 points   3 P   4 vs   5 nodes   6 leaves   7 F   8 dist   9 face */
+#define DDMP_DISTANCE_DESC_WORDS 10
+int ddmp_point_mesh_distance_multi(const int64_t* table, int32_t n, int64_t blocks, void* stream);
+/* ddmp_distance_stats per row; blocks = min(ceil(P / 256), 1024); each row its own zeroed scratch of
+ * ddmp_distance_scratch_bytes() (left zeroed).
+ *   2 dist   3 P   4 out[4]   5 scratch */
+#define DDMP_DISTANCE_STATS_DESC_WORDS 6
+int ddmp_distance_stats_multi(const int64_t* table, int32_t n, int64_t blocks, void* stream);
+/* Evaluation of a fit's float32 positions pos [V,3] against its clean mesh's float64 unit face normals gt_fn [F,3]
+ * (same faces): vs64 [V,3] = pos widened to float64; *mad = mean over faces of
+ * rad2deg(arccos(clip(dot(fn, gt_fn), -1, 1))), float64, where fn is the face normal of pos in float32 arithmetic,
+ * cross(p1-p0, p2-p0) / (sqrt(x*x + y*y + z*z) + 1e-24f), as numpy computes it on float32 positions.  Per-block
+ * partial sums combined in block order.  blocks = min(ceil(max(V, F) / 256), 1024); scratch as for the stats.
+ * [ref: main.py:117-123 Mesh.compute_face_normals on the output positions, then util/loss.py:261-272 mad]
+ *   2 pos   3 faces   4 gt_fn   5 vs64   6 mad   7 scratch   8 V   9 F */
+#define DDMP_EVAL_DESC_WORDS 10
+int ddmp_eval_mad_multi(const int64_t* table, int32_t n, int64_t blocks, void* stream);
 /* ---- partitioned mode: BatchNorm reductions over NVLink peer memory (csrc/comm.cu) ------------------------- */
 /* Every rank owns one exchange buffer (ddmp_comm_buffer_bytes() bytes, allocated and zeroed by ddmp_comm_alloc) that all
  * peers of the box map through CUDA IPC (ddmp_comm_ipc_handle on the owner -> 64 opaque bytes -> ddmp_comm_ipc_open on

@@ -5,8 +5,11 @@ directories, with up to ``--batch`` fits sharing one GPU as one ``MultiDualStep`
     torchrun --nproc_per_node 8 scripts/fit_many.py data/* --batch 8      # directories sharded over the GPUs
 
 Each directory holds ``*_noise.obj`` and ``*_smooth.obj`` (and optionally ``*_gt.obj``), as for the single-mesh driver.
-Every 10 epochs the MAD against ``*_gt.obj`` is evaluated when it exists; every 100 epochs the current mesh is saved to
-``<input>/output/<epoch>_ddmp=<mad>.obj``.  At the end one JSON line per mesh is printed.
+Every 10 epochs the fits with a ``*_gt.obj`` are evaluated on the GPU (``distance.BatchEvaluator``: MAD and the
+two-sided distance to the clean mesh, all fits of the batch in a few launches, no host synchronisation); every 100
+epochs the current mesh is saved to ``<input>/output/<epoch>_ddmp=<mad>.obj`` by a writer thread while training goes on.
+At the end one JSON line per mesh is printed; fits with a clean mesh also report ``final_hausdorff``,
+``final_hausdorff_rel`` and ``final_mean_rel`` of the last evaluation (None before the first).
 """
 from __future__ import annotations
 
@@ -14,7 +17,9 @@ import argparse
 import glob
 import json
 import os
+import queue
 import sys
+import threading
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
@@ -82,13 +87,53 @@ def chunks(items, size: int):
     return [items[i: i + size] for i in range(0, len(items), size)]
 
 
+class SnapshotWriter:
+    """One thread that writes OBJ snapshots (``synth.write_obj``, the format of ``Mesh.save``) off the training thread.
+    ``put(event, jobs)``: once ``event`` (the device-to-host copies of the positions) has completed, write each
+    ``(path, vs, faces)``.  ``close()`` waits for every write and re-raises the first error."""
+
+    def __init__(self):
+        self._q: queue.Queue = queue.Queue()
+        self._error = None
+        self._thread = threading.Thread(target=self._run, name="fit_many-snapshots", daemon=True)
+        self._thread.start()
+
+    def _run(self) -> None:
+        from dual_dmp_b200.synth import write_obj
+        while True:
+            item = self._q.get()
+            if item is None:
+                return
+            event, jobs = item
+            if self._error is not None:
+                continue
+            try:
+                if event is not None:
+                    event.synchronize()
+                for path, vs, faces in jobs:
+                    write_obj(path, vs.numpy() if hasattr(vs, "numpy") else vs, faces)
+            except BaseException as e:      # re-raised on the training thread by close()
+                self._error = e
+
+    def put(self, event, jobs) -> None:
+        if self._error is not None:
+            raise self._error
+        self._q.put((event, jobs))
+
+    def close(self) -> None:
+        self._q.put(None)
+        self._thread.join()
+        if self._error is not None:
+            raise self._error
+
+
 def fit_batch(dirs, args, device) -> list:
     import torch
 
     import dual_dmp_b200.util.datamaker as Datamaker
     import dual_dmp_b200.util.loss as Loss
+    from dual_dmp_b200.distance import BatchEvaluator
     from dual_dmp_b200.step import MultiDualStep
-    from dual_dmp_b200.util.mesh import Mesh
     from dual_dmp_b200.util.networks import NormalNet, PosNet
 
     k = (args.k1, args.k2, args.k3, args.k4, args.k5)
@@ -104,23 +149,50 @@ def fit_batch(dirs, args, device) -> list:
         mad = Loss.mad(n_mesh.fn, gt.fn) if gt is not None else None
         meta.append(dict(input=d, out_dir=out_dir, gt=gt, o1=o1, initial_mad=mad, mad=mad))
     step = MultiDualStep(fits, bnfloop=args.bnfloop)
-    loss = None
-    for epoch in range(1, args.iter + 1):
-        loss = step.step(epoch)
-        if epoch % 10 == 0:
-            for i, m in enumerate(meta):
-                m["o1"].vs = step.pos[i].to("cpu").numpy().copy()
-                Mesh.compute_face_normals(m["o1"])
-                Mesh.compute_vert_normals(m["o1"])
-                if m["gt"] is not None:
-                    m["mad"] = Loss.mad(m["o1"].fn, m["gt"].fn)
-        if epoch % 100 == 0:
-            for m in meta:
-                mad = m["mad"] if m["mad"] is not None else float("nan")
-                Mesh.save(m["o1"], os.path.join(m["out_dir"], "{}_ddmp={:.3f}.obj".format(epoch, mad)))
+    with_gt = [i for i, m in enumerate(meta) if m["gt"] is not None]
+    evaluator = BatchEvaluator([meta[i]["o1"] for i in with_gt], [meta[i]["gt"] for i in with_gt], device) \
+        if with_gt else None
+    side = torch.cuda.Stream(device)
+    writer = SnapshotWriter()
+    loss = report = None
+    try:
+        for epoch in range(1, args.iter + 1):
+            loss = step.step(epoch)
+            if epoch % 10 == 0 and evaluator is not None:
+                report = evaluator.evaluate([step.pos[i] for i in with_gt])
+            if epoch % 100 == 0:
+                if report is not None:       # the file names need the MADs: one read for the batch
+                    for i, mad in zip(with_gt, report["mad"].tolist()):
+                        meta[i]["mad"] = mad
+                # positions to pinned host buffers on a side stream; the next step waits for the copies only
+                cur = torch.cuda.current_stream(device)
+                side.wait_stream(cur)
+                with torch.cuda.stream(side):
+                    host = [torch.empty(p.shape, dtype=p.dtype, pin_memory=True).copy_(p, non_blocking=True)
+                            for p in step.pos]
+                    done = torch.cuda.Event()
+                    done.record(side)
+                cur.wait_stream(side)
+                writer.put(done, [(os.path.join(m["out_dir"], "{}_ddmp={:.3f}.obj".format(
+                    epoch, m["mad"] if m["mad"] is not None else float("nan"))), h, m["o1"].faces)
+                    for m, h in zip(meta, host)])
+    finally:
+        writer.close()
     final = loss.to("cpu").tolist()
-    return [dict(input=m["input"], iters=args.iter, final_loss=final[i], initial_mad=m["initial_mad"],
-                 final_mad=m["mad"]) for i, m in enumerate(meta)]
+    finals = {}
+    if report is not None:
+        mads, h, hr, mr = (report[k].tolist() for k in ("mad", "hausdorff", "hausdorff_rel", "mean_rel"))
+        for j, i in enumerate(with_gt):
+            meta[i]["mad"] = mads[j]
+            finals[i] = dict(final_hausdorff=h[j], final_hausdorff_rel=hr[j], final_mean_rel=mr[j])
+    out = []
+    for i, m in enumerate(meta):
+        r = dict(input=m["input"], iters=args.iter, final_loss=final[i], initial_mad=m["initial_mad"],
+                 final_mad=m["mad"])
+        if m["gt"] is not None:
+            r.update(finals.get(i, dict(final_hausdorff=None, final_hausdorff_rel=None, final_mean_rel=None)))
+        out.append(r)
+    return out
 
 
 def main(argv=None) -> None:
