@@ -486,6 +486,177 @@ eval_multi_kernel(const int64_t* __restrict__ table, int n) {
     }
 }
 
+// ---- area-weighted surface samples and the normal angle across a correspondence (DESIGN.md §4.9) ----------------
+// w_f = |(b-a) x (c-a)| (twice the area), float64, the cross product in tri_d2's component order, squares summed in
+// axis order.  q_f = rint(w_f / w_max * 2^32) as int64 (0 where that is not positive, NaN included) and P_f its
+// inclusive prefix.  Integer sums are exact in any order, so the prefix does not depend on the block partition.
+constexpr int kScanItems = 4;                    // consecutive faces per thread in the prefix kernels
+constexpr int kScanTile = kT * kScanItems;       // faces per block
+constexpr uint64_t kGolden = 0x9E3779B97F4A7C15ull;
+
+__host__ __device__ __forceinline__ uint64_t splitmix64(uint64_t z) {   // the output function of splitmix64
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+
+__device__ __forceinline__ V3 cross3(V3 u, V3 w) {
+    return {u.y * w.z - u.z * w.y, u.z * w.x - u.x * w.z, u.x * w.y - u.y * w.x};
+}
+
+__device__ __forceinline__ V3 face_cross(const double* __restrict__ vs, const int* __restrict__ faces, int64_t f) {
+    const V3 a = load3(vs, __ldg(faces + 3 * f));
+    return cross3(sub(load3(vs, __ldg(faces + 3 * f + 1)), a), sub(load3(vs, __ldg(faces + 3 * f + 2)), a));
+}
+
+__device__ __forceinline__ double face_weight(const double* __restrict__ vs, const int* __restrict__ faces, int64_t f) {
+    const V3 n = face_cross(vs, faces, f);
+    return sqrt(dot(n, n));
+}
+
+// exclusive prefix of v over the block's threads in thread order; total = the block's sum
+__device__ __forceinline__ long long block_excl_scan(long long v, long long& total) {
+    __shared__ long long warp_total[kT / 32];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    long long incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const long long y = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += y;
+    }
+    if (lane == 31) warp_total[w] = incl;
+    __syncthreads();
+    long long off = 0;
+    total = 0;
+#pragma unroll
+    for (int k = 0; k < kT / 32; ++k) {
+        const long long t = warp_total[k];
+        if (k < w) off += t;
+        total += t;
+    }
+    return off + incl - v;
+}
+
+// *wmax = bits of max_f w_f (zero on entry; non-negative doubles order like their bit patterns)
+__global__ void __launch_bounds__(kT)
+weight_max_kernel(const double* __restrict__ vs, const int* __restrict__ faces, int64_t F,
+                  unsigned long long* wmax) {
+    double m = 0.0;
+    for (int64_t f = (int64_t)blockIdx.x * kT + threadIdx.x; f < F; f += (int64_t)gridDim.x * kT)
+        m = fmax(m, face_weight(vs, faces, f));
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if ((threadIdx.x & 31) == 0 && m > 0.0) atomicMax(wmax, (unsigned long long)__double_as_longlong(m));
+}
+
+// prefix[f] = q_f; tile_sum[block] = the sum of the block's q_f
+__global__ void __launch_bounds__(kT)
+weight_quant_kernel(const double* __restrict__ vs, const int* __restrict__ faces, int64_t F,
+                    const unsigned long long* __restrict__ wmax, int64_t* __restrict__ prefix,
+                    int64_t* __restrict__ tile_sum) {
+    const double wm = __longlong_as_double((long long)*wmax);
+    const int64_t base = (int64_t)blockIdx.x * kScanTile + (int64_t)threadIdx.x * kScanItems;
+    long long s = 0;
+#pragma unroll
+    for (int k = 0; k < kScanItems; ++k) {
+        if (base + k >= F) break;
+        const double x = rint(face_weight(vs, faces, base + k) / wm * 4294967296.0);
+        const long long q = x > 0.0 ? (long long)x : 0;
+        prefix[base + k] = q;
+        s += q;
+    }
+    long long total;
+    block_excl_scan(s, total);
+    if (threadIdx.x == 0) tile_sum[blockIdx.x] = total;
+}
+
+// tile_sum[0..nb) -> its exclusive prefix, one block; thread t scans the contiguous run [t*per, (t+1)*per)
+__global__ void __launch_bounds__(kT)
+tile_scan_kernel(int64_t* __restrict__ tile_sum, int64_t nb) {
+    const int64_t per = (nb + kT - 1) / kT, lo = (int64_t)threadIdx.x * per, hi = lo + per < nb ? lo + per : nb;
+    long long s = 0;
+    for (int64_t k = lo; k < hi; ++k) s += tile_sum[k];
+    long long total;
+    long long run = block_excl_scan(s, total);
+    for (int64_t k = lo; k < hi; ++k) {
+        const long long x = tile_sum[k];
+        tile_sum[k] = run;
+        run += x;
+    }
+}
+
+// prefix[f] = q_f -> P_f, the block's inclusive scan plus the tiles before it
+__global__ void __launch_bounds__(kT)
+prefix_apply_kernel(int64_t* __restrict__ prefix, const int64_t* __restrict__ tile_off, int64_t F) {
+    const int64_t base = (int64_t)blockIdx.x * kScanTile + (int64_t)threadIdx.x * kScanItems;
+    long long q[kScanItems], s = 0;
+#pragma unroll
+    for (int k = 0; k < kScanItems; ++k) {
+        q[k] = base + k < F ? prefix[base + k] : 0;
+        s += q[k];
+    }
+    long long total;
+    long long run = block_excl_scan(s, total) + tile_off[blockIdx.x];
+#pragma unroll
+    for (int k = 0; k < kScanItems; ++k) {
+        run += q[k];
+        if (base + k < F) prefix[base + k] = run;
+    }
+}
+
+// Sample i: words k = 0, 1, 2 are splitmix64(key + (3i + k + 1) * golden); u0 = word 0 >> 32, r = (word >> 11) * 2^-53.
+// Target T = ((i * 2^32 + u0) * Q) div (n * 2^32) < Q, face = the first f with P_f > T (a face with q_f = 0 is never
+// first), point = (1 - s) a + s (1 - r2) b + s r2 c with s = sqrt(r1), per component ((wa a + wb b) + wc c).
+__global__ void __launch_bounds__(kT)
+sample_kernel(const double* __restrict__ vs, const int* __restrict__ faces, const int64_t* __restrict__ prefix,
+              int64_t F, int64_t n, uint64_t key, double* __restrict__ pts, int* __restrict__ face) {
+    const int64_t i = (int64_t)blockIdx.x * kT + threadIdx.x;
+    if (i >= n) return;
+    const uint64_t Q = (uint64_t)__ldg(prefix + F - 1);
+    const uint64_t w0 = key + (uint64_t)(3 * i + 1) * kGolden;
+    const uint64_t u0 = splitmix64(w0) >> 32;
+    // s = sqrt(r1) first: sqrt's slow path is a called routine, and taken here no value lives across the call (taken
+    // after the search, it costs a spill)
+    const double s = sqrt((double)(splitmix64(w0 + kGolden) >> 11) * 0x1p-53);
+    const double r2 = (double)(splitmix64(w0 + 2 * kGolden) >> 11) * 0x1p-53;
+    // T = ((i * 2^32 + u0) * Q) div (n * 2^32): the product is below 2^125
+    const unsigned __int128 x = (unsigned __int128)(((uint64_t)i << 32) | u0);
+    const uint64_t T = (uint64_t)(x * Q / ((unsigned __int128)(uint64_t)n << 32));
+    int64_t lo = 0, hi = F - 1;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if ((uint64_t)__ldg(prefix + mid) > T) hi = mid;
+        else lo = mid + 1;
+    }
+    const V3 a = load3(vs, __ldg(faces + 3 * lo)), b = load3(vs, __ldg(faces + 3 * lo + 1)),
+             c = load3(vs, __ldg(faces + 3 * lo + 2));
+    const double wa = 1.0 - s, wb = s * (1.0 - r2), wc = s * r2;
+    pts[3 * i] = (wa * a.x + wb * b.x) + wc * c.x;
+    pts[3 * i + 1] = (wa * a.y + wb * b.y) + wc * c.y;
+    pts[3 * i + 2] = (wa * a.z + wb * b.z) + wc * c.z;
+    face[i] = (int)lo;
+}
+
+// deg[i] = rad2deg(arccos(clip(n_A(fa[i]) . n_B(fb[i]), -1, 1))), n = cross / (|cross| + 1e-24) as
+// Mesh.compute_face_normals computes it in float64
+__device__ __forceinline__ V3 unit_normal(const double* __restrict__ vs, const int* __restrict__ faces, int64_t f) {
+    const V3 n = face_cross(vs, faces, f);
+    const double len = sqrt(dot(n, n)) + 1e-24;
+    return {n.x / len, n.y / len, n.z / len};
+}
+
+__global__ void __launch_bounds__(kT)
+normal_angle_kernel(const double* __restrict__ vs_a, const int* __restrict__ faces_a, const int* __restrict__ fa,
+                    const double* __restrict__ vs_b, const int* __restrict__ faces_b, const int* __restrict__ fb,
+                    int64_t n, double* __restrict__ deg) {
+    const int64_t i = (int64_t)blockIdx.x * kT + threadIdx.x;
+    if (i >= n) return;
+    const V3 na = unit_normal(vs_a, faces_a, __ldg(fa + i)), nb = unit_normal(vs_b, faces_b, __ldg(fb + i));
+    double c = dot(na, nb);
+    c = c < -1.0 ? -1.0 : (c > 1.0 ? 1.0 : c);
+    deg[i] = acos(c) * (180.0 / 3.14159265358979323846);
+}
+
 }  // namespace dist
 }  // namespace ddmp
 
@@ -576,6 +747,53 @@ int ddmp_distance_stats_multi(const int64_t* table, int32_t n, int64_t blocks, v
 
 int ddmp_eval_mad_multi(const int64_t* table, int32_t n, int64_t blocks, void* stream) {
     return launch_multi(ddmp::dist::eval_multi_kernel, table, n, blocks, stream, "eval_mad_multi");
+}
+
+int64_t ddmp_surface_prefix_workspace_bytes(int64_t F) {
+    return 8 * (1 + ddmp::ceil_div(F > 0 ? F : 1, ddmp::dist::kScanTile));
+}
+
+int ddmp_surface_prefix(const double* vs, const int32_t* faces, int64_t F, int64_t* prefix, void* workspace,
+                        void* stream) {
+    using namespace ddmp;
+    DDMP_REQUIRE(vs && faces && prefix && workspace && F > 0 && F < ((int64_t)1 << 30), "surface_prefix: bad arguments");
+    const cudaStream_t st = as_stream(stream);
+    unsigned long long* wmax = (unsigned long long*)workspace;
+    int64_t* tile = (int64_t*)workspace + 1;
+    const unsigned nb = (unsigned)ceil_div(F, dist::kScanTile);
+    DDMP_REQUIRE(cudaMemsetAsync(wmax, 0, sizeof(*wmax), st) == cudaSuccess, "surface_prefix: memset failed");
+    dist::weight_max_kernel<<<dist::grid_for(F), dist::kT, 0, st>>>(vs, faces, F, wmax);
+    int rc = check_launch("surface_prefix max");
+    if (rc != 0) return rc;
+    dist::weight_quant_kernel<<<nb, dist::kT, 0, st>>>(vs, faces, F, wmax, prefix, tile);
+    if ((rc = check_launch("surface_prefix quantise")) != 0) return rc;
+    dist::tile_scan_kernel<<<1, dist::kT, 0, st>>>(tile, nb);
+    if ((rc = check_launch("surface_prefix tiles")) != 0) return rc;
+    dist::prefix_apply_kernel<<<nb, dist::kT, 0, st>>>(prefix, tile, F);
+    return check_launch("surface_prefix scan");
+}
+
+int ddmp_surface_sample(const double* vs, const int32_t* faces, const int64_t* prefix, int64_t F, int64_t n,
+                        int64_t seed, int32_t side, double* points, int32_t* face, void* stream) {
+    using namespace ddmp;
+    DDMP_REQUIRE(vs && faces && prefix && points && face && F > 0 && F < ((int64_t)1 << 30) && n > 0 &&
+                     n < ((int64_t)1 << 31) && seed >= 0 && side >= 0,
+                 "surface_sample: bad arguments");
+    using dist::kGolden;
+    using dist::splitmix64;
+    const uint64_t key = splitmix64(splitmix64((uint64_t)seed + kGolden) + ((uint64_t)side + 1) * kGolden);
+    dist::sample_kernel<<<(unsigned)ceil_div(n, dist::kT), dist::kT, 0, as_stream(stream)>>>(vs, faces, prefix, F, n,
+                                                                                           key, points, face);
+    return check_launch("surface_sample");
+}
+
+int ddmp_normal_angle(const double* vs_a, const int32_t* faces_a, const int32_t* face_a, const double* vs_b,
+                      const int32_t* faces_b, const int32_t* face_b, int64_t n, double* deg, void* stream) {
+    using namespace ddmp;
+    DDMP_REQUIRE(vs_a && faces_a && face_a && vs_b && faces_b && face_b && deg && n > 0, "normal_angle: bad arguments");
+    dist::normal_angle_kernel<<<(unsigned)ceil_div(n, dist::kT), dist::kT, 0, as_stream(stream)>>>(
+        vs_a, faces_a, face_a, vs_b, faces_b, face_b, n, deg);
+    return check_launch("normal_angle");
 }
 
 }  // extern "C"

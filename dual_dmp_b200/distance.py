@@ -9,6 +9,10 @@ meshes are apart, sampled at their vertices, the quantity upstream Dual-DMP repo
     gt = MeshBVH(gt_mesh.vs, gt_mesh.faces)              # the reference mesh's tree, built once per fit
     report = hausdorff(o1_mesh, gt)                       # report["hausdorff_rel"], report["mean_rel"]
 
+``surface_distance(a, b, samples)`` does the same on area-weighted surface samples of both meshes, so the result does
+not depend on how either mesh is triangulated, and adds the normal error across the nearest-face correspondence, which
+needs no shared faces.
+
 Contract (DESIGN.md "Point-to-mesh distance"): float64 triangle tests; a zero-area face counts as the segment or point
 it spans; ties go to the lowest face id; results are deterministic and equal bit for bit those of an exhaustive scan.
 """
@@ -107,6 +111,7 @@ class MeshBVH:
         self.counters = torch.zeros(n_int, dtype=torch.int32, device=dev)        # kept zeroed for refit
         lib.call("ddmp_bvh_build", ptr(self.vs), ptr(self.faces), ptr(keys), ptr(order), ptr(self.nodes),
                  ptr(self.leaves), ptr(self.parent), ptr(self.counters), self.F, st)
+        self._prefix = None            # the sampler's face-weight prefix, built by the first sample_surface
 
     def refit(self, vs) -> None:
         """Move the tree to new positions ``vs`` [V,3] of the same mesh: ``.vs`` and ``.bbox`` take the new values and
@@ -116,6 +121,7 @@ class MeshBVH:
         if vs.shape[0] != self.V:
             raise ValueError(f"refit: expected {self.V} vertices, got {vs.shape[0]}")
         self.vs.copy_(_to64(vs, self.device))
+        self._prefix = None
         st = self._stream()
         lib.call("ddmp_prep_bbox", ptr(self.vs), ptr(self.bbox), ptr(self._scratch), self.V, st)
         lib.call("ddmp_bvh_refit", ptr(self.vs), ptr(self.leaves), ptr(self.nodes), ptr(self.parent),
@@ -150,6 +156,39 @@ class MeshBVH:
             lib.call("ddmp_point_mesh_distance_exhaustive", ptr(pts), P, ptr(self.vs), ptr(self.faces), self.F,
                      ptr(dist), ptr(face), self._stream())
         return dist, face
+
+    def sample_surface(self, n: int, seed: int = 0, side: int = 0) -> tuple[torch.Tensor, torch.Tensor]:
+        """(points float64 [n,3], face int32 [n]) on the tree's device: ``n`` deterministic points on the surface,
+        stratified by area (each face gets ``n`` times its share of the area in samples, to within less than 2), in face
+        order, uniform inside each face.  ``(seed, side)`` select the random numbers; ``surface_distance`` draws mesh a
+        with side 0 and mesh b with side 1.  The first call reads the total weight back from the device once and raises
+        ``ValueError`` when the mesh has zero total area."""
+        n = _check_int(n, "samples", 1, 1 << 31)
+        seed = _check_int(seed, "seed", 0, 1 << 63)
+        side = _check_int(side, "side", 0, 1 << 31)
+        st = self._stream()
+        if self._prefix is None:
+            ws = torch.empty(int(lib.query("ddmp_surface_prefix_workspace_bytes", self.F)) // 8, dtype=torch.int64,
+                             device=self.device)
+            prefix = torch.empty(self.F, dtype=torch.int64, device=self.device)
+            lib.call("ddmp_surface_prefix", ptr(self.vs), ptr(self.faces), self.F, ptr(prefix), ptr(ws), st)
+            if int(prefix[-1]) == 0:
+                raise ValueError("sample_surface: the mesh has zero total area (no surface to sample)")
+            self._prefix = prefix
+        pts = torch.empty(n, 3, dtype=torch.float64, device=self.device)
+        face = torch.empty(n, dtype=torch.int32, device=self.device)
+        lib.call("ddmp_surface_sample", ptr(self.vs), ptr(self.faces), ptr(self._prefix), self.F, n, seed, side,
+                 ptr(pts), ptr(face), st)
+        return pts, face
+
+
+def _check_int(x, what: str, lo: int, hi: int | None = None) -> int:
+    if isinstance(x, (bool, np.bool_)) or not isinstance(x, (int, np.integer)):
+        raise ValueError(f"{what}: expected an int, got {type(x).__name__}")
+    x = int(x)
+    if x < lo or (hi is not None and x >= hi):
+        raise ValueError(f"{what}: expected an int in [{lo}, {'inf' if hi is None else hi}), got {x}")
+    return x
 
 
 def distance_stats(dist: torch.Tensor) -> dict:
@@ -192,8 +231,11 @@ def hausdorff(a, b, device=None) -> dict:
     ta, tb = _as_bvh(a, device), _as_bvh(b, device)
     if ta.device != tb.device:
         raise ValueError(f"hausdorff: meshes on different devices ({ta.device}, {tb.device})")
-    ab = distance_stats(tb.query(ta.vs)[0])
-    ba = distance_stats(ta.query(tb.vs)[0])
+    return _two_sided(distance_stats(tb.query(ta.vs)[0]), distance_stats(ta.query(tb.vs)[0]), tb)
+
+
+def _two_sided(ab: dict, ba: dict, tb: MeshBVH) -> dict:
+    """the report of ``hausdorff`` from the statistics of both directions; diag from b's box"""
     bb = tb.bbox.tolist()
     diag = math.sqrt(sum((bb[3 + k] - bb[k]) ** 2 for k in range(3)))
     h = max(ab["max"], ba["max"])
@@ -201,6 +243,45 @@ def hausdorff(a, b, device=None) -> dict:
     return {"a_to_b": ab, "b_to_a": ba, "hausdorff": h, "mean": mean, "diag": diag,
             "hausdorff_rel": h / diag if diag > 0 else float("nan"),
             "mean_rel": mean / diag if diag > 0 else float("nan")}
+
+
+def _normal_angles(ta: MeshBVH, face_a: torch.Tensor, tb: MeshBVH, face_b: torch.Tensor) -> torch.Tensor:
+    """degrees between the normal of ta's face face_a[i] and of tb's face face_b[i], float64 [n]"""
+    n = int(face_a.shape[0])
+    deg = torch.empty(n, dtype=torch.float64, device=ta.device)
+    lib.call("ddmp_normal_angle", ptr(ta.vs), ptr(ta.faces), ptr(face_a), ptr(tb.vs), ptr(tb.faces), ptr(face_b), n,
+             ptr(deg), ta._stream())
+    return deg
+
+
+def surface_distance(a, b, samples: int, seed: int = 0, device=None) -> dict:
+    """Two-sided distance and normal error between meshes ``a`` and ``b`` of any topologies, sampled on their surfaces:
+    ``samples`` area-weighted points per mesh (``MeshBVH.sample_surface``, a with side 0 and b with side 1, both with
+    ``seed``), each queried against the other mesh's surface.  ``a`` and ``b`` take what ``hausdorff`` takes (a reused
+    ``MeshBVH`` keeps its tree and its sampling prefix).  The report:
+
+    * ``a_to_b`` / ``b_to_a``, ``hausdorff``, ``mean``, ``diag``, ``hausdorff_rel``, ``mean_rel``: as in ``hausdorff``,
+      over the surface samples instead of the vertices, ``diag`` taken from b;
+    * ``normal_a_to_b`` / ``normal_b_to_a``: ``{min, max, mean, rms, n}`` of the angle in degrees between the normal of
+      a sample's face and the normal of its nearest face on the other mesh (``Loss.mad``'s angle, across that
+      correspondence; a flipped face reads 180, a zero-area nearest face 90);
+    * ``normal_mean = (normal_a_to_b.mean + normal_b_to_a.mean) / 2``; ``samples``, ``seed``.
+
+    A mesh of zero total area raises ``ValueError``."""
+    samples = _check_int(samples, "samples", 1, 1 << 31)
+    seed = _check_int(seed, "seed", 0, 1 << 63)
+    if device is None:
+        device = next((m.device for m in (a, b) if isinstance(m, MeshBVH)), None)
+    ta, tb = _as_bvh(a, device), _as_bvh(b, device)
+    if ta.device != tb.device:
+        raise ValueError(f"surface_distance: meshes on different devices ({ta.device}, {tb.device})")
+    pa, fa = ta.sample_surface(samples, seed, 0)
+    pb, fb = tb.sample_surface(samples, seed, 1)
+    d_ab, g_ab = tb.query(pa)
+    d_ba, g_ba = ta.query(pb)
+    nab, nba = distance_stats(_normal_angles(ta, fa, tb, g_ab)), distance_stats(_normal_angles(tb, fb, ta, g_ba))
+    return {**_two_sided(distance_stats(d_ab), distance_stats(d_ba), tb), "normal_a_to_b": nab, "normal_b_to_a": nba,
+            "normal_mean": 0.5 * (nab["mean"] + nba["mean"]), "samples": samples, "seed": seed}
 
 
 # batched evaluation (include/ddmp_b200.h, "Batched evaluation of many fits"): table widths and block counts

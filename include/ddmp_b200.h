@@ -319,6 +319,33 @@ int ddmp_distance_stats_multi(const int64_t* table, int32_t n, int64_t blocks, v
  *   2 pos   3 faces   4 gt_fn   5 vs64   6 mad   7 scratch   8 V   9 F */
 #define DDMP_EVAL_DESC_WORDS 10
 int ddmp_eval_mad_multi(const int64_t* table, int32_t n, int64_t blocks, void* stream);
+
+/* Area-weighted surface samples of a mesh (vs [V,3] float64, faces [F,3], F < 2^30), deterministic (csrc/distance.cu,
+ * DESIGN.md §4.9).  Face weight w_f = |(b-a) x (c-a)| in float64 (cross product in the component order of the point-to-
+ * triangle routine, squares summed in axis order); w_max = max_f w_f; q_f = rint(w_f / w_max * 2^32) as int64, 0 where
+ * that is not positive (zero-area faces, slivers below 2^-33 of the largest face, NaN); prefix [F] int64 = inclusive
+ * prefix P_f of q_f, so Q = P_{F-1} < 2^62.  Q = 0: no surface to sample (the caller checks before sampling).
+ * workspace: ddmp_surface_prefix_workspace_bytes(F) bytes, contents irrelevant on entry. */
+int64_t ddmp_surface_prefix_workspace_bytes(int64_t F);
+int ddmp_surface_prefix(const double* vs, const int32_t* faces, int64_t F, int64_t* prefix, void* workspace,
+                        void* stream);
+/* n samples (1 <= n < 2^31) over the prefix of ddmp_surface_prefix (Q > 0), seed >= 0, side >= 0:
+ *   mix(z)  = splitmix64's output function: z = (z ^ z>>30) * 0xBF58476D1CE4E5B9; z = (z ^ z>>27) * 0x94D049BB133111EB;
+ *             z ^ z>>31  (uint64 arithmetic, mod 2^64);  G = 0x9E3779B97F4A7C15
+ *   key     = mix(mix(seed + G) + (side + 1) * G)
+ *   word k of sample i (k = 0, 1, 2) = mix(key + (3i + k + 1) * G);  u0 = word 0 >> 32;  r1, r2 = (word 1, 2 >> 11) * 2^-53
+ *   T_i     = ((i * 2^32 + u0) * Q) div (n * 2^32)  (exact, 128-bit);  face[i] = the first f with P_f > T_i
+ *   s = sqrt(r1), wa = 1 - s, wb = s * (1 - r2), wc = s * r2;  points[i] = (wa*a + wb*b) + wc*c per component.
+ * Every face gets n*q_f/Q samples to within less than 2, and face[] is non-decreasing in i.
+ * points [n,3] float64, face [n] int32. */
+int ddmp_surface_sample(const double* vs, const int32_t* faces, const int64_t* prefix, int64_t F, int64_t n,
+                        int64_t seed, int32_t side, double* points, int32_t* face, void* stream);
+/* deg[i] = rad2deg(arccos(clip(dot(n_A(face_a[i]), n_B(face_b[i])), -1, 1))), float64, with the face normal
+ * n = cross(p1-p0, p2-p0) / (|cross| + 1e-24) of Mesh.compute_face_normals (a zero-area face: n = 0, 90 degrees).
+ * face_a / face_b: valid face ids of (vs_a, faces_a) / (vs_b, faces_b), e.g. a sample's face and its nearest face.
+ * [ref: util/loss.py:261-272 mad, across a correspondence instead of equal face ids] */
+int ddmp_normal_angle(const double* vs_a, const int32_t* faces_a, const int32_t* face_a, const double* vs_b,
+                      const int32_t* faces_b, const int32_t* face_b, int64_t n, double* deg, void* stream);
 /* ---- partitioned mode: BatchNorm reductions over NVLink peer memory (csrc/comm.cu) ------------------------- */
 /* Every rank owns one exchange buffer (ddmp_comm_buffer_bytes() bytes, allocated and zeroed by ddmp_comm_alloc) that all
  * peers of the box map through CUDA IPC (ddmp_comm_ipc_handle on the owner -> 64 opaque bytes -> ddmp_comm_ipc_open on
