@@ -108,8 +108,6 @@ int make_tensor_map_2d(void* map, const float* base, int64_t outer, int64_t inne
 
 // tile-staged aggregation kernel (spmm_tile.cu)
 bool spmm_tile_supported(int64_t n, int C);
-int spmm_tile_set(int setting);   // mode | flags << 4, see spmm_tile.cu
-int spmm_flags();
 int spmm_bn_bwd_tile_rows(int C);
 int spmm_bn_bwd_tile_launch(const int* rowptr, const int* col, const float* w, const float* gX, const float* Y,
                             const float* mean, const float* rstd, const float* scale, const float* shift,

@@ -1566,17 +1566,12 @@ static int launch_nt16x2(const Nt16Args& g0, cudaStream_t st) {
     return check_launch("tc_gemm_nt16x2");
 }
 
-// switches of the fp16-split NT kernels (environment DDMP_TC_F16_FLAGS, ddmp_gemm_tc_flags): bit 3 = unstaged epilogue
-// (15-40 % slower), bit 4 = staged ld.shared + st.global epilogue instead of TMA stores, bit 5 = the previous
-// configuration (register-fed A operand everywhere, CTA pairs for every N % 256 == 0)
+// switches of the fp16-split NT kernels (ddmp_gemm_tc_flags): bit 3 = unstaged epilogue (15-40 % slower), bit 4 = staged
+// ld.shared + st.global epilogue instead of TMA stores, bit 5 = the previous configuration (register-fed A operand
+// everywhere, CTA pairs for every N % 256 == 0)
 int f16_flags(int set) {
-    static std::atomic<int> v{-1};
-    int cur = v.load(std::memory_order_relaxed);
-    if (cur < 0) {
-        const char* e = getenv("DDMP_TC_F16_FLAGS");
-        cur = e ? (atoi(e) & 56) : 0;
-        v.store(cur, std::memory_order_relaxed);
-    }
+    static std::atomic<int> v{0};
+    const int cur = v.load(std::memory_order_relaxed);
     if (set >= 0) v.store(set & 56, std::memory_order_relaxed);
     return cur;
 }

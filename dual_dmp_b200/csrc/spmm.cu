@@ -19,7 +19,7 @@ __global__ void __launch_bounds__(256, (STATS || C >= 512) ? 3 : 4)
 spmm_gcn_kernel(const int* __restrict__ rowptr, const int* __restrict__ col, const float* __restrict__ w,
                 const float* __restrict__ H, const float* __restrict__ bias, float* __restrict__ Y,
                 float* __restrict__ partials, float* __restrict__ amax_blocks, int64_t n, int rows_per_block,
-                int blocks_per_cta, int flags) {
+                int blocks_per_cta) {
     constexpr int G = (C / 4 < 32) ? (C / 4) : 32;
     constexpr int NV = C / (4 * G);
     constexpr int GROUPS = 256 / G;
@@ -149,9 +149,11 @@ spmm_gcn_kernel(const int* __restrict__ rowptr, const int* __restrict__ col, con
             if (BIAS) {
                 o.x += bsum[v].x; o.y += bsum[v].y; o.z += bsum[v].z; o.w += bsum[v].w;
             }
-            if (flags & 2) __stcs(reinterpret_cast<float4*>(yp + (v * G + lg) * 4), o);   // streaming: Y is not re-read from L2
-            else st4(yp + (v * G + lg) * 4, o);
-            amx = fmaxf(fmaxf(amx, fmaxf(fabsf(o.x), fabsf(o.y))), fmaxf(fabsf(o.z), fabsf(o.w)));
+            // streaming (evict-first) store: this kernel never re-reads Y, and keeping it out of L2 leaves the cache to the
+            // gathered rows (+1 % on the wide layers)
+            __stcs(reinterpret_cast<float4*>(yp + (v * G + lg) * 4), o);
+            // only when requested: without this condition ptxas spills the row loop's state in the plain flavour
+            if (amax_blocks) amx = fmaxf(fmaxf(amx, fmaxf(fabsf(o.x), fabsf(o.y))), fmaxf(fabsf(o.z), fabsf(o.w)));
             if (STATS) {                            // Welford: running mean and M2 of this group's rows (see bn.cu)
                 float4 s = *reinterpret_cast<float4*>(myred + (v * G + lg) * 4);
                 float4 q = *reinterpret_cast<float4*>(myred + C + (v * G + lg) * 4);
@@ -589,7 +591,7 @@ __global__ void gcn_edge_weights_kernel(const int* __restrict__ rowptr, const in
 
 template <int C>
 static int launch_spmm(const int* rowptr, const int* col, const float* w, const float* H, const float* bias,
-                       float* Y, float* partials, float* amax_blocks, int64_t n, cudaStream_t st) {
+                       float* Y, float* partials, float* amax_blocks, int64_t n, bool reference, cudaStream_t st) {
     const int rpb = ddmp_rows_per_block(C);
     const int64_t nblk = ceil_div(n, rpb);
     // consecutive row blocks per CTA (DDMP_SPMM_CHUNK).  Default 1: walking 4 or 8 neighbouring blocks per CTA to
@@ -599,26 +601,27 @@ static int launch_spmm(const int* rowptr, const int* col, const float* w, const 
     int bpc = chunk_env < 1 ? 1 : chunk_env;
     while (bpc > 1 && ceil_div(nblk, bpc) < 8 * kNumSMs) --bpc;
     const unsigned grid = (unsigned)ceil_div(nblk, bpc);
-    const int fl = spmm_flags();
-    if (partials && !amax_blocks && (fl & 4) && (C == 512 || (C == 256 && (fl & 8))) && bpc == 1) {
-        // wide forward flavour: Welford state in tensor memory (spmm_gcn_stats_tmem_kernel; flag 4: C = 512, flag 8:
-        // C = 256).  1M-row graphs, vertex / face: C = 512 0.592 -> 0.525 / 0.938 -> 0.862 ms; C = 256 0.331 -> 0.296 /
-        // 0.483 -> 0.449 ms once the kernel runs 4 CTAs per SM (at 3 it measured the same as the 16 KB shared-memory
-        // state): profiles/spmm_tmem_ab_r2.txt
+    if (!reference && partials && !amax_blocks && (C == 256 || C == 512) && bpc == 1) {
+        // wide forward flavour: Welford state in tensor memory (spmm_gcn_stats_tmem_kernel).  1M-row graphs, vertex /
+        // face: C = 512 0.592 -> 0.525 / 0.938 -> 0.862 ms; C = 256 0.331 -> 0.296 / 0.483 -> 0.449 ms once the kernel
+        // runs 4 CTAs per SM (at 3 it measured the same as the 16 KB shared-memory state): profiles/spmm_tmem_ab_r2.txt
         constexpr int CT = (C == 256 || C == 512) ? C : 256;
         if (bias) spmm_gcn_stats_tmem_kernel<CT, true><<<(unsigned)nblk, 256, 0, st>>>(rowptr, col, w, H, bias, Y, partials, n, rpb);
         else spmm_gcn_stats_tmem_kernel<CT, false><<<(unsigned)nblk, 256, 0, st>>>(rowptr, col, w, H, bias, Y, partials, n, rpb);
         return check_launch("spmm_gcn_stats_tmem");
     }
     if (partials) {
-        if (bias) spmm_gcn_kernel<C, true, true><<<grid, 256, 0, st>>>(rowptr, col, w, H, bias, Y, partials, amax_blocks, n, rpb, bpc, fl);
-        else spmm_gcn_kernel<C, true, false><<<grid, 256, 0, st>>>(rowptr, col, w, H, bias, Y, partials, amax_blocks, n, rpb, bpc, fl);
+        if (bias) spmm_gcn_kernel<C, true, true><<<grid, 256, 0, st>>>(rowptr, col, w, H, bias, Y, partials, amax_blocks, n, rpb, bpc);
+        else spmm_gcn_kernel<C, true, false><<<grid, 256, 0, st>>>(rowptr, col, w, H, bias, Y, partials, amax_blocks, n, rpb, bpc);
     } else {
-        if (bias) spmm_gcn_kernel<C, false, true><<<grid, 256, 0, st>>>(rowptr, col, w, H, bias, Y, partials, amax_blocks, n, rpb, bpc, fl);
-        else spmm_gcn_kernel<C, false, false><<<grid, 256, 0, st>>>(rowptr, col, w, H, bias, Y, partials, amax_blocks, n, rpb, bpc, fl);
+        if (bias) spmm_gcn_kernel<C, false, true><<<grid, 256, 0, st>>>(rowptr, col, w, H, bias, Y, partials, amax_blocks, n, rpb, bpc);
+        else spmm_gcn_kernel<C, false, false><<<grid, 256, 0, st>>>(rowptr, col, w, H, bias, Y, partials, amax_blocks, n, rpb, bpc);
     }
     return check_launch("spmm_gcn");
 }
+
+// ddmp_spmm_reference_kernel: the gather kernel with shared-memory statistics at every width
+static std::atomic<int> g_reference_kernel{0};
 
 }  // namespace ddmp
 
@@ -638,13 +641,15 @@ int ddmp_spmm_gcn(const int32_t* rowptr, const int32_t* col, const float* w, con
     if (n == 0) return DDMP_OK;
     DDMP_REQUIRE(rowptr && col && w && H && Y, "spmm_gcn: null pointer");
     cudaStream_t st = as_stream(stream);
-    if (spmm_tile_supported(n, C)) return spmm_tile_launch(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, C, st);
+    const bool ref = g_reference_kernel.load(std::memory_order_relaxed) != 0;
+    if (!ref && spmm_tile_supported(n, C))
+        return spmm_tile_launch(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, C, st);
     switch (C) {
-        case 32: return launch_spmm<32>(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, st);
-        case 64: return launch_spmm<64>(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, st);
-        case 128: return launch_spmm<128>(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, st);
-        case 256: return launch_spmm<256>(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, st);
-        case 512: return launch_spmm<512>(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, st);
+        case 32: return launch_spmm<32>(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, ref, st);
+        case 64: return launch_spmm<64>(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, ref, st);
+        case 128: return launch_spmm<128>(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, ref, st);
+        case 256: return launch_spmm<256>(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, ref, st);
+        case 512: return launch_spmm<512>(rowptr, col, w, H, bias, Y, stats_partials, amax_blocks, n, ref, st);
         default: break;
     }
     if (stats_partials || amax_blocks) {
@@ -679,12 +684,9 @@ int ddmp_spmm_bn_bwd_tile(const int32_t* rowptr, const int32_t* col, const float
                                    amax_blocks, n, C, as_stream(stream));
 }
 
-int ddmp_spmm_use_tile_kernel(int mode) { return ddmp::spmm_tile_set(mode); }
+int ddmp_spmm_reference_kernel(int on) { return ddmp::g_reference_kernel.exchange(on != 0, std::memory_order_relaxed); }
 
-int64_t ddmp_spmm_amax_len(int64_t n, int32_t C) {
-    const int64_t nblk = ddmp_num_row_blocks(n, C);
-    return ddmp::spmm_tile_supported(n, C) && C > 128 ? nblk * (C / 128) : nblk;
-}
+int64_t ddmp_spmm_amax_len(int64_t n, int32_t C) { return ddmp_num_row_blocks(n, C); }
 
 int ddmp_spmm_bn_bwd(const int32_t* rowptr, const int32_t* col, const float* w, const float* gX, const float* Y,
                      const float* mean, const float* rstd, const float* scale, const float* shift, const float* c1,

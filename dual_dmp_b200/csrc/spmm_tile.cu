@@ -5,16 +5,16 @@
 // leave the block go to L1/L2.  Replaces torch_geometric GCNConv.propagate (index_select -> mul -> scatter_add,
 // reference util/networks.py:51-62,112-123) like spmm.cu; same epilogues (bias, BatchNorm partial sums, max|Y|).
 //
-// Mapping: CTA = (row block of R rows) x (channel slice of CS <= 128 channels), 256 threads.  A group of G = CS/4
-// lanes owns one output row at a time (one float4 per lane); the 256/G groups walk the block's rows.  No global
-// dependent-load chain is left in the loop: rowptr / col / w come from shared memory, in-block rows from the tile.
-//   C = 32, 64  : CS = C,   R = 256  (tile 32 / 64 KB)
-//   C >= 128    : CS = 128, R = 128  (tile 64 KB), C/128 CTAs per row block (neighbouring block indices, so the
-//                 slices of one row are fetched from DRAM at about the same time)
+// Mapping: CTA = row block of R rows, all C <= 128 channels, 256 threads.  A group of G = C/4 lanes owns one output
+// row at a time (one float4 per lane); the 256/G groups walk the block's rows.  No global dependent-load chain is left
+// in the loop: rowptr / col / w come from shared memory, in-block rows from the tile.
+//   C = 32      : R = 256  (tile 32 KB)
+//   C = 64, 128 : R = 128  (tile 32 / 64 KB)
+// The wider layers run the gather kernel (spmm.cu): there a TMA tile of whole rows does not fit, and a 128-channel
+// slice per CTA measured slower (DESIGN.md §4.1).
 // Deterministic: no atomics; per-CTA BatchNorm partials are combined in group order.
 // Roofline: HBM; algorithmic bytes 4*[(n+1) + 2*nnz + 2*n*C] (SURVEY.md §8d).
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -59,32 +59,29 @@ struct Args {
     const float* bias;
     float* Y;
     float* partials;      // [nblk][2][C] or null
-    float* amax;          // [nblk * slices] or null
+    float* amax;          // [nblk] or null
     int64_t n;
-    int C;
 };
 
-template <int CS, int R, bool STATS, bool BIAS>
+template <int C, int R, bool STATS, bool BIAS>
 __global__ void __launch_bounds__(kThreads)
 spmm_tile_kernel(const __grid_constant__ CUtensorMap hmap, const Args a) {
-    constexpr int G = CS / 4;
+    constexpr int G = C / 4;
     constexpr int GROUPS = kThreads / G;
     constexpr int kMetaCap = R * kMetaPerRow;
-    static_assert(GROUPS * 2 * CS * 4 <= R * CS * 4, "the statistics scratch aliases the tile");
+    static_assert(GROUPS * 2 * C * 4 <= R * C * 4, "the statistics scratch aliases the tile");
     extern __shared__ unsigned char smem_raw[];
     unsigned char* base = smem_raw + ((128u - (smem_u32(smem_raw) & 127u)) & 127u);    // TMA destination: 128 B aligned
-    float* tile = reinterpret_cast<float*>(base);                                       // [R][CS]
-    float* red = tile;                                                                  // [GROUPS][2*CS], after the loop
-    int* scol = reinterpret_cast<int*>(base + (size_t)R * CS * 4);                      // [kMetaCap]
+    float* tile = reinterpret_cast<float*>(base);                                       // [R][C]
+    float* red = tile;                                                                  // [GROUPS][2*C], after the loop
+    int* scol = reinterpret_cast<int*>(base + (size_t)R * C * 4);                       // [kMetaCap]
     float* sw = reinterpret_cast<float*>(scol + kMetaCap);                              // [kMetaCap]
     int* srow = reinterpret_cast<int*>(sw + kMetaCap);                                  // [R + 1]
     uint64_t* barp = reinterpret_cast<uint64_t*>(srow + R + 2 + ((R & 1) ? 1 : 0));     // 8 B aligned
     float* wmax = reinterpret_cast<float*>(barp + 1);                                   // [kThreads / 32]
     uint64_t& bar = *barp;
 
-    const int slices = a.C / CS;
-    const int64_t blk = blockIdx.x / slices;
-    const int ch0 = (blockIdx.x % slices) * CS;
+    const int64_t blk = blockIdx.x;
     const int64_t row0 = blk * R;
     const int rows = (int)((row0 + R <= a.n) ? R : (a.n - row0));
     const int lane = threadIdx.x & 31;
@@ -94,8 +91,8 @@ spmm_tile_kernel(const __grid_constant__ CUtensorMap hmap, const Args a) {
     if (threadIdx.x == 0) {
         mbar_init(&bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        mbar_expect_tx(&bar, (uint32_t)(R * CS * 4));            // rows past n are zero-filled and still counted
-        tma_load_2d(tile, &hmap, ch0, (int)row0, &bar);
+        mbar_expect_tx(&bar, (uint32_t)(R * C * 4));             // rows past n are zero-filled and still counted
+        tma_load_2d(tile, &hmap, 0, (int)row0, &bar);
     }
     // (rowptr, col, w) of the block -> shared memory, while the tile is in flight
     for (int i = threadIdx.x; i <= rows; i += kThreads) srow[i] = __ldg(a.rowptr + row0 + i);
@@ -110,14 +107,14 @@ spmm_tile_kernel(const __grid_constant__ CUtensorMap hmap, const Args a) {
         }
     }
     float4 bsum = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (BIAS) bsum = ldg4(a.bias + ch0 + lg * 4);
+    if (BIAS) bsum = ldg4(a.bias + lg * 4);
     float4 ssum = make_float4(0.f, 0.f, 0.f, 0.f), qsum = make_float4(0.f, 0.f, 0.f, 0.f);     // running mean, M2
     float cnt = 0.f;
     float amx = 0.f;
     __syncthreads();
     mbar_wait(&bar, 0);
 
-    const float* Hs = a.H + ch0 + lg * 4;
+    const float* Hs = a.H + lg * 4;
     for (int r = gid; r < rows; r += GROUPS) {
         const int s = srow[r] - kb, e = srow[r + 1] - kb;
         float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -135,8 +132,8 @@ spmm_tile_kernel(const __grid_constant__ CUtensorMap hmap, const Args a) {
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 const int64_t lc = (int64_t)c[u] - row0;
-                if ((uint64_t)lc < (uint64_t)rows) x[u] = *reinterpret_cast<const float4*>(tile + (int)lc * CS + lg * 4);
-                else x[u] = ldg4(Hs + (int64_t)c[u] * a.C);
+                if ((uint64_t)lc < (uint64_t)rows) x[u] = *reinterpret_cast<const float4*>(tile + (int)lc * C + lg * 4);
+                else x[u] = ldg4(Hs + (int64_t)c[u] * C);
             }
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
@@ -149,13 +146,13 @@ spmm_tile_kernel(const __grid_constant__ CUtensorMap hmap, const Args a) {
             const float w1 = meta_in_smem ? sw[k] : __ldg(a.w + kb + k);
             const int64_t lc = (int64_t)c1 - row0;
             float4 x;
-            if ((uint64_t)lc < (uint64_t)rows) x = *reinterpret_cast<const float4*>(tile + (int)lc * CS + lg * 4);
-            else x = ldg4(Hs + (int64_t)c1 * a.C);
+            if ((uint64_t)lc < (uint64_t)rows) x = *reinterpret_cast<const float4*>(tile + (int)lc * C + lg * 4);
+            else x = ldg4(Hs + (int64_t)c1 * C);
             acc.x = fmaf(w1, x.x, acc.x); acc.y = fmaf(w1, x.y, acc.y);
             acc.z = fmaf(w1, x.z, acc.z); acc.w = fmaf(w1, x.w, acc.w);
         }
         if (BIAS) { acc.x += bsum.x; acc.y += bsum.y; acc.z += bsum.z; acc.w += bsum.w; }
-        st4(a.Y + (row0 + r) * a.C + ch0 + lg * 4, acc);
+        st4(a.Y + (row0 + r) * C + lg * 4, acc);
         amx = fmaxf(fmaxf(amx, fmaxf(fabsf(acc.x), fabsf(acc.y))), fmaxf(fabsf(acc.z), fabsf(acc.w)));
         if (STATS) {                                // Welford: running mean and M2 of this thread's rows (see bn.cu)
             cnt += 1.f;
@@ -172,17 +169,17 @@ spmm_tile_kernel(const __grid_constant__ CUtensorMap hmap, const Args a) {
         // per-group (mean, M2) -> shared memory (over the tile, which is dead now); then one thread per channel merges the
         // groups in group order (Chan et al.) and writes the block's (sum, M2 about the block mean)
         __syncthreads();
-        st4(red + gid * 2 * CS + lg * 4, ssum);
-        st4(red + gid * 2 * CS + CS + lg * 4, qsum);
+        st4(red + gid * 2 * C + lg * 4, ssum);
+        st4(red + gid * 2 * C + C + lg * 4, qsum);
         __syncthreads();
-        float* outp = a.partials + blk * 2 * a.C;
-        for (int ch = threadIdx.x; ch < CS; ch += kThreads) {
+        float* outp = a.partials + blk * 2 * C;
+        for (int ch = threadIdx.x; ch < C; ch += kThreads) {
             float n_a = 0.f, mean = 0.f, m2 = 0.f;
 #pragma unroll 4
             for (int g = 0; g < GROUPS; ++g) {
                 const float n_b = (float)((rows - g + GROUPS - 1) / GROUPS);      // rows g, g+GROUPS, ... of this block
                 if (g < rows) {
-                    const float mb = red[g * 2 * CS + ch], qb = red[g * 2 * CS + CS + ch];
+                    const float mb = red[g * 2 * C + ch], qb = red[g * 2 * C + C + ch];
                     const float n = n_a + n_b;
                     const float d = mb - mean;
                     mean = fmaf(d, n_b / n, mean);
@@ -190,8 +187,8 @@ spmm_tile_kernel(const __grid_constant__ CUtensorMap hmap, const Args a) {
                     n_a = n;
                 }
             }
-            outp[ch0 + ch] = mean * n_a;
-            outp[a.C + ch0 + ch] = m2;
+            outp[ch] = mean * n_a;
+            outp[C + ch] = m2;
         }
     }
     if (a.amax) {
@@ -203,7 +200,7 @@ spmm_tile_kernel(const __grid_constant__ CUtensorMap hmap, const Args a) {
             float m = wmax[0];
 #pragma unroll
             for (int i = 1; i < kThreads / 32; ++i) m = fmaxf(m, wmax[i]);
-            a.amax[blockIdx.x] = m;
+            a.amax[blk] = m;
         }
     }
 }
@@ -389,30 +386,29 @@ static int make_map(CUtensorMap* map, const float* H, int64_t n, int C, int CS, 
     return make_tensor_map_2d(map, H, n, C, R, CS, false, "spmm_tile");
 }
 
-template <int CS, int R>
+template <int C, int R>
 static int launch(const Args& a, cudaStream_t st) {
     CUtensorMap map;
-    int rc = make_map(&map, a.H, a.n, a.C, CS, R);
+    int rc = make_map(&map, a.H, a.n, C, C, R);
     if (rc != DDMP_OK) return rc;
     const int64_t nblk = ceil_div(a.n, R);
-    const unsigned grid = (unsigned)(nblk * (a.C / CS));
     const bool stats = a.partials != nullptr, bias = a.bias != nullptr;
-    const size_t smem = smem_bytes<CS, R>();
+    const size_t smem = smem_bytes<C, R>();
     static PerDeviceOnce configured;
     if (configured.need()) {
         const int mx = (int)smem;
-        DDMP_CUDA(cudaFuncSetAttribute(spmm_tile_kernel<CS, R, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
-        DDMP_CUDA(cudaFuncSetAttribute(spmm_tile_kernel<CS, R, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
-        DDMP_CUDA(cudaFuncSetAttribute(spmm_tile_kernel<CS, R, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
-        DDMP_CUDA(cudaFuncSetAttribute(spmm_tile_kernel<CS, R, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
+        DDMP_CUDA(cudaFuncSetAttribute(spmm_tile_kernel<C, R, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
+        DDMP_CUDA(cudaFuncSetAttribute(spmm_tile_kernel<C, R, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
+        DDMP_CUDA(cudaFuncSetAttribute(spmm_tile_kernel<C, R, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
+        DDMP_CUDA(cudaFuncSetAttribute(spmm_tile_kernel<C, R, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
         configured.mark();
     }
     if (stats) {
-        if (bias) spmm_tile_kernel<CS, R, true, true><<<grid, kThreads, smem, st>>>(map, a);
-        else spmm_tile_kernel<CS, R, true, false><<<grid, kThreads, smem, st>>>(map, a);
+        if (bias) spmm_tile_kernel<C, R, true, true><<<(unsigned)nblk, kThreads, smem, st>>>(map, a);
+        else spmm_tile_kernel<C, R, true, false><<<(unsigned)nblk, kThreads, smem, st>>>(map, a);
     } else {
-        if (bias) spmm_tile_kernel<CS, R, false, true><<<grid, kThreads, smem, st>>>(map, a);
-        else spmm_tile_kernel<CS, R, false, false><<<grid, kThreads, smem, st>>>(map, a);
+        if (bias) spmm_tile_kernel<C, R, false, true><<<(unsigned)nblk, kThreads, smem, st>>>(map, a);
+        else spmm_tile_kernel<C, R, false, false><<<(unsigned)nblk, kThreads, smem, st>>>(map, a);
     }
     return check_launch("spmm_tile");
 }
@@ -456,50 +452,19 @@ int spmm_bn_bwd_tile_launch(const int* rowptr, const int* col, const float* w, c
     return tile::launch_bwd<128, 64>(a, st);
 }
 
-// Kernel choice (ddmp_spmm_use_tile_kernel(v) / environment DDMP_SPMM_TILE; v = mode | flags << 4):
-//   mode 0 = gather kernel for every width
-//        1 = tile-staged kernel for C <= 128, gather kernel above (default: measured fastest on B200, 1M-face graphs,
-//            profiles/spmm_tile_ab_r2.txt, profiles/spmm_pipe_ab_r2.txt)
-//        2 = tile-staged kernel for every supported width
-//   flags bit 1 = streaming (evict-first) stores of Y in the gather kernel (default on: Y is never re-read from L2 by this
-//   kernel, and keeping it out leaves the cache to the gathered rows: +1 % on the wide layers).  -1: not decided yet.
-static std::atomic<int> g_tile_mode{-1};
-constexpr int kDefaultSetting = 1 | ((2 | 4 | 8) << 4);  // tile kernel for C <= 128, streaming stores, TMEM Welford state at C = 256 / 512
-
-static int tile_setting() {
-    int v = g_tile_mode.load(std::memory_order_relaxed);
-    if (v < 0) {
-        const char* e = getenv("DDMP_SPMM_TILE");
-        v = e ? atoi(e) : kDefaultSetting;
-        if (v < 0 || (v & 15) > 2) v = kDefaultSetting;
-        g_tile_mode.store(v, std::memory_order_relaxed);
-    }
-    return v;
-}
-static int tile_mode() { return tile_setting() & 15; }
-int spmm_flags() { return tile_setting() >> 4; }
-
-int spmm_tile_set(int v) {
-    const int prev = tile_setting();
-    if (v < 0 || (v & 15) > 2) v = kDefaultSetting;
-    g_tile_mode.store(v, std::memory_order_relaxed);
-    return prev;
-}
-
+// the widths where this kernel beats the gather kernel on B200 (1M-face graphs, profiles/spmm_tile_ab_r2.txt); the TMA
+// row coordinate is a 32-bit int
 bool spmm_tile_supported(int64_t n, int C) {
-    const int mode = tile_mode();
-    if (mode == 0 || n >= (1ll << 31)) return false;
-    if (C == 32 || C == 64 || C == 128) return true;
-    return mode == 2 && C > 128 && C <= 512 && C % 128 == 0;
+    return n < (1ll << 31) && (C == 32 || C == 64 || C == 128);
 }
 
 int spmm_tile_launch(const int* rowptr, const int* col, const float* w, const float* H, const float* bias, float* Y,
                      float* partials, float* amax, int64_t n, int C, cudaStream_t st) {
-    tile::Args a{rowptr, col, w, H, bias, Y, partials, amax, n, C};
+    tile::Args a{rowptr, col, w, H, bias, Y, partials, amax, n};
     const int rpb = ddmp_rows_per_block(C);               // the BatchNorm partials are laid out per row block
     if (C == 32 && rpb == 256) return tile::launch<32, 256>(a, st);
     if (C == 64 && rpb == 128) return tile::launch<64, 128>(a, st);
-    if (C >= 128 && rpb == 128) return tile::launch<128, 128>(a, st);
+    if (C == 128 && rpb == 128) return tile::launch<128, 128>(a, st);
     set_error("spmm_tile: no instantiation for C=%d rows_per_block=%d", C, rpb);
     return DDMP_ERR_UNSUPPORTED;
 }

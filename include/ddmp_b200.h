@@ -75,22 +75,21 @@ int ddmp_gcn_edge_weights(const int32_t* rowptr, const int32_t* col, float* w, i
 /* Y[i,:] = sum_k w[k] * H[col[k],:] (+ bias).  Optional epilogue statistics: stats_partials[b][0][c] = sum of
  * Y[:,c] over row block b, [b][1][c] = sum of Y^2 (BatchNorm partials).  The same call is the backward pass
  * (A_hat is symmetric): dH = spmm(dY) with bias = stats = NULL.  C must be a multiple of 4.
- * amax_blocks (optional, [ddmp_spmm_amax_len(n,C)]): max |Y| of every (row block, channel slice) a CTA produced, the
- * `amax` input of the dense transforms that consume Y.
- * Mesh widths (32, 64, multiples of 128 up to 512) run the tile-staged kernel: the row block's own rows of H arrive in
- * shared memory by one TMA tensor copy, its (rowptr, col, w) stream by coalesced loads (csrc/spmm_tile.cu).
+ * amax_blocks (optional, [ddmp_spmm_amax_len(n,C)]): max |Y| of every row block, the `amax` input of the dense
+ * transforms that consume Y.
+ * C = 32, 64, 128 run the tile-staged kernel: the row block's own rows of H arrive in shared memory by one TMA tensor
+ * copy, its (rowptr, col, w) stream by coalesced loads (csrc/spmm_tile.cu).  Wider rows run the gather kernel; its
+ * forward flavour (statistics without amax_blocks) at C = 256 / 512 keeps the Welford state in tensor memory.
  * [ref: GCNConv.propagate + bias at util/networks.py:51-62,112-123; torch_scatter.scatter_add] */
 int ddmp_spmm_gcn(const int32_t* rowptr, const int32_t* col, const float* w, const float* H, const float* bias,
                   float* Y, float* stats_partials, float* amax_blocks, int64_t n, int32_t C, void* stream);
-/* number of floats ddmp_spmm_gcn writes to amax_blocks for this shape */
+/* number of floats ddmp_spmm_gcn writes to amax_blocks for this shape: the row-block count, ddmp_num_row_blocks(n, C) */
 int64_t ddmp_spmm_amax_len(int64_t n, int32_t C);
-/* Kernel choice of ddmp_spmm_gcn (environment DDMP_SPMM_TILE, default 225).  setting = mode | flags << 4.
- * mode: 0 = gather-only kernel for every width, 1 = tile-staged kernel for C <= 128 (where it measures faster on B200),
- * 2 = tile-staged kernel for every mesh width (A/B measurements, bit-exactness test between the two kernels).
- * flags: 2 = streaming stores of Y in the gather kernel; 4 = forward flavour (bias + BatchNorm moments) at C = 512 with the
- * per-warp Welford state in tensor memory instead of shared memory (bitwise-equal results); 8 = the same at C = 256.
- * Returns the previous setting. */
-int ddmp_spmm_use_tile_kernel(int mode);
+/* Test and A/B hook, process-wide, default 0.  on != 0: ddmp_spmm_gcn runs the gather kernel with the Welford state in
+ * shared memory at every width, instead of the tile-staged kernel (C <= 128) and the tensor-memory flavour (C = 256 /
+ * 512).  Its results are bitwise those of the default kernels, which the tests check against it.  Returns the previous
+ * value (0 or 1). */
+int ddmp_spmm_reference_kernel(int on);
 
 /* Backward aggregation fused with ddmp_bn_bwd_apply:  dH = A_hat * dY  with dY recomputed on the fly from the gathered
  * rows of gX and Y (dY is never materialised); optional colsum_partials[b][0][c] = column sums of dY (conv bias
@@ -171,11 +170,10 @@ int ddmp_gemm_xw(const float* X, const int32_t* row_map, const float* scale, con
 /* scratch the tensor-core path of gemm_xw / gemm_dx needs for the pre-split, pre-swizzled weight image (0 when the
  * shape runs on the FFMA kernel; with workspace == NULL the FFMA kernel is used). */
 int64_t ddmp_gemm_workspace_bytes(int64_t n, int32_t Cin, int32_t Cout);
-/* Alternative configurations of the fp16-split tcgen05 kernels behind ddmp_gemm_xw / ddmp_gemm_dx (environment
- * DDMP_TC_F16_FLAGS, default 0; bitwise the same results as the default): bit 3 (8) = unstaged thread-per-row
- * epilogue; bit 4 (16) = staged ld.shared + st.global epilogue instead of TMA tensor stores; bit 5 (32) = A operand by
- * the register-fed producers everywhere (no TMA A operand).  Other bits are ignored.  flags < 0 only queries.
- * Returns the previous value. */
+/* Alternative configurations of the fp16-split tcgen05 kernels behind ddmp_gemm_xw / ddmp_gemm_dx (default 0; bitwise
+ * the same results as the default): bit 3 (8) = unstaged thread-per-row epilogue; bit 4 (16) = staged ld.shared +
+ * st.global epilogue instead of TMA tensor stores; bit 5 (32) = A operand by the register-fed producers everywhere (no
+ * TMA A operand).  Other bits are ignored.  flags < 0 only queries.  Returns the previous value. */
 int ddmp_gemm_tc_flags(int flags);
 /* gX[n,Cin] = dH[n,Cout] * W[Cout,Cin]. */
 int ddmp_gemm_dx(const float* dH, const float* W, float* gX, void* workspace, int64_t workspace_bytes, int64_t n,

@@ -1,6 +1,7 @@
 """Micro-benchmark of the GCN aggregation kernels on the 1M-face graphs (both flavours, every width).
-usage: bench_spmm.py [setting ...]   setting = mode | flags << 4 of ddmp_spmm_use_tile_kernel (include/ddmp_b200.h);
-default: the library's default.  All settings are measured in ONE process on the same graphs, interleaved per shape."""
+usage: bench_spmm.py [setting ...]   setting = 0: the default kernels, 1: the reference gather kernel
+(ddmp_spmm_reference_kernel, include/ddmp_b200.h); default: both.  All settings are measured in ONE process on the same
+graphs, interleaved per shape."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -9,8 +10,7 @@ from dual_dmp_b200._lib import lib
 from dual_dmp_b200.graph import GcnGraph
 from dual_dmp_b200.util.mesh import Mesh
 dev = "cuda:0"
-default = int(lib.query("ddmp_spmm_use_tile_kernel", 0)); lib.query("ddmp_spmm_use_tile_kernel", default)
-settings = [int(a) for a in sys.argv[1:]] or [default]
+settings = [int(a) for a in sys.argv[1:]] or [0, 1]
 vs, faces = synth.icosphere(224)
 m = Mesh(vs=vs * 100, faces=faces)
 F, V = len(faces), len(vs)
@@ -25,7 +25,7 @@ for name, g in (("vertex", vg), ("face", fg)):
         for flav, fn in (("fwd(stats+bias)", lambda: F_.spmm_gcn(g, H, bias=b, stats=True)), ("bwd(plain)", lambda: F_.spmm_gcn(g, H, amax=True))):
             line = f"{name:6s} C={C:3d} {flav:16s}"
             for s in settings:
-                lib.query("ddmp_spmm_use_tile_kernel", s)
+                lib.query("ddmp_spmm_reference_kernel", s)
                 fn(); torch.cuda.synchronize()
                 ms = 0.0
                 for _ in range(5):
@@ -40,4 +40,4 @@ for name, g in (("vertex", vg), ("face", fg)):
         del H
 for s in settings:
     print(f"setting {s}: step-weighted {tot_b[s] / tot_t[s] / 1e6:.0f} GB/s, {2 * tot_t[s]:.2f} ms per step (48 launches)")
-lib.query("ddmp_spmm_use_tile_kernel", default)
+lib.query("ddmp_spmm_reference_kernel", 0)

@@ -22,9 +22,9 @@ DEV = "cuda:0"
 U32 = 2.0 ** -24
 U64 = 2.0 ** -53
 WIDTHS = [32, 64, 128, 256, 512]
-# ddmp_spmm_use_tile_kernel settings: mode (0 gather, 1 tile-staged for C <= 128, 2 tile-staged everywhere) | flags << 4
-# (2: streaming stores, 4|8: Welford state in tensor memory at C = 512 / 256)
-SETTINGS = [mode | (flags << 4) for mode in (0, 1, 2) for flags in (2, 4 | 8)]
+# ddmp_spmm_reference_kernel: 0 = the default kernels (tile-staged at C <= 128, Welford state in tensor memory at C = 256 /
+# 512), 1 = the gather kernel with shared-memory statistics at every width
+SETTINGS = [0, 1]
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -92,18 +92,17 @@ def _check_partials(partials, ref, C):
 
 def _set(setting):
     from dual_dmp_b200._lib import lib
-    lib.query("ddmp_spmm_use_tile_kernel", setting)
+    lib.query("ddmp_spmm_reference_kernel", setting)
 
 
 @pytest.fixture
 def restore_setting():
     from dual_dmp_b200._lib import lib
-    prev = lib.query("ddmp_spmm_use_tile_kernel", -1)
-    lib.query("ddmp_spmm_use_tile_kernel", prev)
+    prev = lib.query("ddmp_spmm_reference_kernel", 0)
     try:
         yield
     finally:
-        lib.query("ddmp_spmm_use_tile_kernel", prev)
+        lib.query("ddmp_spmm_reference_kernel", prev)
 
 
 def test_long_row_graph_csr_and_weights(agg):
@@ -122,7 +121,7 @@ def test_long_row_graph_csr_and_weights(agg):
 
 
 @pytest.mark.parametrize("C", WIDTHS + [12])
-def test_aggregation_is_exact_on_long_rows(agg, C, restore_setting):
+def test_aggregation_is_exact_on_long_rows_default_and_reference(agg, C, restore_setting):
     """power-of-two weights, integer H in [-64, 64], power-of-two bias: every product and partial sum is exact in fp32,
     so Y and max|Y| must EQUAL the float64 reference on every kernel setting -- a dropped, doubled or misplaced (col, w)
     entry of any chunk fails here with no tolerance involved"""
@@ -152,7 +151,7 @@ def test_aggregation_is_exact_on_long_rows(agg, C, restore_setting):
 
 
 @pytest.mark.parametrize("C", WIDTHS + [12])
-def test_aggregation_with_gcn_weights_within_a_priori_bound(agg, C, restore_setting):
+def test_aggregation_with_gcn_weights_within_a_priori_bound_default_and_reference(agg, C, restore_setting):
     """real GCN weights (the graph's own fp32 w), random H and bias, against float64 index_add_ on the device, per row:
     |Y_i - ref_i| <= 2 (L_i + 1) 2^-24 (sum_k |w_k H_ck| + |b|)   (recursive fp32 summation of L_i products + bias)"""
     from dual_dmp_b200 import functional as F_
@@ -179,9 +178,9 @@ def test_aggregation_with_gcn_weights_within_a_priori_bound(agg, C, restore_sett
 
 
 @pytest.mark.parametrize("C", WIDTHS)
-def test_aggregation_kernels_bitwise_equal_on_long_rows(agg, C, restore_setting):
-    """tile-staged (shared-memory and global (col, w) streams), gather, gather with streaming stores, and the TMEM
-    statistics flavour all accumulate every row in CSR order: Y, the block partials and max|Y| are IDENTICAL"""
+def test_aggregation_default_kernels_equal_reference_on_long_rows(agg, C, restore_setting):
+    """the default kernels (tile-staged with shared-memory and global (col, w) streams, the TMEM statistics flavour) and
+    the reference gather kernel all accumulate every row in CSR order: Y, the block partials and max|Y| are IDENTICAL"""
     from dual_dmp_b200 import functional as F_
     n = agg["n"]
     torch.manual_seed(200 + C)
@@ -190,7 +189,7 @@ def test_aggregation_kernels_bitwise_equal_on_long_rows(agg, C, restore_setting)
     for name, (rowptr, col, w, _, n_rows) in agg["variants"].items():
         g = _sub(rowptr, col, w, n_rows)
         res = {}
-        for setting in [0] + SETTINGS:
+        for setting in SETTINGS:
             _set(setting)
             y1, p1 = F_.spmm_gcn(g, H, bias=b, stats=True, n_rows=n_rows)
             y2, p2 = F_.spmm_gcn(g, H, stats=True, n_rows=n_rows)
@@ -199,7 +198,7 @@ def test_aggregation_kernels_bitwise_equal_on_long_rows(agg, C, restore_setting)
             assert float(ab.max()) == float(y3.abs().max())
             res[setting] = (y1, p1, y2, p2, y3, y4, ab.max())
         for setting, out in res.items():
-            for i, (x, x0) in enumerate(zip(out, res[0])):
+            for i, (x, x0) in enumerate(zip(out, res[1])):
                 assert torch.equal(x, x0), (name, setting, i)
     report(f"long rows: aggregation kernels bitwise equal C={C}", len(res))
 

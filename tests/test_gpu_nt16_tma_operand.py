@@ -106,7 +106,6 @@ def test_register_operand_where_tma_does_not_pay():
     gather; K = 512 without the prologue, the fused row gather (a_map) and flags bit 5 keep the register-fed
     producers.  Read from the kernels' cycle-trace lines (DDMP_TC_TRACE=1)."""
     env = dict(os.environ, DDMP_TC_TRACE="1")
-    env.pop("DDMP_TC_F16_FLAGS", None)
     p = subprocess.run([sys.executable, "-c", _PROBE, ROOT], env=env, capture_output=True, text=True, timeout=600)
     assert p.returncode == 0, p.stderr
     lines = p.stderr.splitlines()

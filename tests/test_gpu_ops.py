@@ -201,11 +201,12 @@ def test_batchnorm_lrelu_forward_backward(C, n):
 
 @pytest.mark.parametrize("ratio", [0.0, 100.0, 1000.0, 1.0e4])
 @pytest.mark.parametrize("C,n", [(32, 70001), (256, 33333), (512, 1001)])
-def test_batchnorm_statistics_with_large_mean_over_sigma(C, n, ratio):
+def test_batchnorm_statistics_with_large_mean_over_sigma_default_and_reference(C, n, ratio):
     """the variance must not be formed as E[y^2] - E[y]^2 in float32 (SURVEY.md §7 hard part 3): the aggregation epilogue
     emits per-block (sum, M2 about the block mean) (Welford per thread, Chan merge per block) and the finalize combines
     them in float64, so the relative error of var / rstd grows like |mean|/sigma * 1e-7, not (mean/sigma)^2 * 1e-7.
-    Also the partitioned-mode route (rank sums in float64 -> finalize_sums) and the tile-staged / gather kernels"""
+    Also the partitioned-mode route (rank sums in float64 -> finalize_sums), on the default kernels and the reference
+    kernel (gather kernel, shared-memory statistics)"""
     from dual_dmp_b200 import functional as F_
     from dual_dmp_b200._lib import lib
     from dual_dmp_b200.graph import GcnGraph
@@ -218,20 +219,20 @@ def test_batchnorm_statistics_with_large_mean_over_sigma(C, n, ratio):
     ref_var = Yd.double().var(0, unbiased=False)
     gamma, beta = torch.ones(C, device=DEV), torch.zeros(C, device=DEV)
     tol = 2e-6 + 4e-7 * ratio
-    prev = lib.query("ddmp_spmm_use_tile_kernel", 0)
+    prev = lib.query("ddmp_spmm_reference_kernel", 0)
     try:
-        for mode in (2, 0, 2 | (2 << 4), 2 << 4):    # tile-staged / gather kernel, without and with streaming stores
-            lib.query("ddmp_spmm_use_tile_kernel", mode)
+        for ref in (0, 1):
+            lib.query("ddmp_spmm_reference_kernel", ref)
             _, partials = F_.spmm_gcn(graph, Yd, stats=True)
             st = F_.bn_stats_finalize(partials, n, gamma, beta)
             e_mean = float((st[0].double() - ref_mean).abs().max() / ref_mean.abs().max().clamp_min(1.0))
             e_rstd = rel_err(st[1], torch.rsqrt(ref_var + 1e-5))
             st2 = F_.bn_stats_finalize_sums(F_.bn_rank_sums(partials, n), n, gamma, beta)
-            report(f"bn stats |mean|/sigma={ratio:g} C={C} n={n} kernel setting {mode}", (e_mean, e_rstd))
-            assert e_mean < 2e-7 and e_rstd < tol, (mode, e_mean, e_rstd, tol)
+            report(f"bn stats |mean|/sigma={ratio:g} C={C} n={n} reference kernel {ref}", (e_mean, e_rstd))
+            assert e_mean < 2e-7 and e_rstd < tol, (ref, e_mean, e_rstd, tol)
             assert torch.equal(st, st2)
     finally:
-        lib.query("ddmp_spmm_use_tile_kernel", prev)
+        lib.query("ddmp_spmm_reference_kernel", prev)
 
 
 @pytest.mark.parametrize("cin,cout", [(64, 128), (128, 256), (256, 256), (512, 512), (512, 256), (256, 64), (128, 64)])
@@ -543,9 +544,10 @@ def GcnGraphIdentity(n):
 
 @pytest.mark.parametrize("C", [32, 64, 128, 256, 512])
 @pytest.mark.parametrize("kind,n", [("ico", 3), ("ico", 10), ("open", 9), ("ico", 40)])
-def test_spmm_tile_kernel_equals_gather_kernel_bitwise(kind, n, C):
-    """csrc/spmm_tile.cu (TMA-staged row block + shared-memory index stream) against csrc/spmm.cu (gathers only): the
-    two accumulate every row in the same CSR order, so Y, the BatchNorm partial sums and max|Y| must be IDENTICAL --
+def test_spmm_default_kernels_equal_reference_kernel_bitwise(kind, n, C):
+    """the default kernels (csrc/spmm_tile.cu, TMA-staged row block + shared-memory index stream, at C <= 128) against
+    the reference kernel (csrc/spmm.cu, gathers only, ddmp_spmm_reference_kernel): both accumulate every row in the same
+    CSR order, so Y, the BatchNorm partial sums and max|Y| must be IDENTICAL --
     closed and open meshes, Morton-ordered and caller-ordered graphs, row counts below / not a multiple of the row
     block, and the partitioned layout (H = [owned | halo] rows, only the owned rows computed)."""
     from dual_dmp_b200 import functional as F_
@@ -559,43 +561,42 @@ def test_spmm_tile_kernel_equals_gather_kernel_bitwise(kind, n, C):
                GcnGraph(ds.face_index, F, DEV, coords=ds.z2.detach()[:, :3], reorder=True),
                GcnGraph(ds.face_index, F, DEV, reorder=False)]
     torch.manual_seed(C + n)
-    prev = lib.query("ddmp_spmm_use_tile_kernel", 0)
+    prev = lib.query("ddmp_spmm_reference_kernel", 0)
     try:
         for graph in graphs_:
             H = torch.randn(graph.n, C, device=DEV)
             b = torch.randn(C, device=DEV)
             res = {}
-            for on in (2, 0, 2 << 4):                # tile-staged, gather, gather with streaming stores
-                lib.query("ddmp_spmm_use_tile_kernel", on)
+            for ref in (0, 1):
+                lib.query("ddmp_spmm_reference_kernel", ref)
                 Y, partials, ab = F_.spmm_gcn(graph, H, bias=b, stats=True, amax=True)
                 Yp = F_.spmm_gcn(graph, H)
-                res[on] = (Y, partials, ab.max(), Yp)
-            assert torch.equal(res[2][0], res[0][0]) and torch.equal(res[2][3], res[0][3])
-            assert torch.equal(res[2][1], res[0][1])
-            assert torch.equal(res[32][0], res[0][0]) and torch.equal(res[32][3], res[0][3]) and torch.equal(res[32][1], res[0][1])
-            assert float(res[2][2]) == float(res[0][2]) == float(res[0][0].abs().max())
+                res[ref] = (Y, partials, ab.max(), Yp)
+            assert torch.equal(res[0][0], res[1][0]) and torch.equal(res[0][3], res[1][3])
+            assert torch.equal(res[0][1], res[1][1])
+            assert float(res[0][2]) == float(res[1][2]) == float(res[1][0].abs().max())
             # partitioned layout: the last rows of H are "halo" rows that are only read
             n_own = graph.n - max(1, graph.n // 7)
             rp = graph.rowptr[: n_own + 1].contiguous()
             sub = type("G", (), dict(rowptr=rp, col=graph.col, w=graph.w, rowptr_t=rp, col_t=graph.col, w_t=graph.w))
             outs = []
-            for on in (2, 0):
-                lib.query("ddmp_spmm_use_tile_kernel", on)
+            for ref in (0, 1):
+                lib.query("ddmp_spmm_reference_kernel", ref)
                 outs.append(F_.spmm_gcn(sub, H, bias=b, n_rows=n_own))
             assert outs[0].shape == (n_own, C) and torch.equal(outs[0], outs[1])
-            assert torch.equal(outs[0], res[0][0][:n_own])
+            assert torch.equal(outs[0], res[1][0][:n_own])
     finally:
-        lib.query("ddmp_spmm_use_tile_kernel", prev)
+        lib.query("ddmp_spmm_reference_kernel", prev)
 
 
 @pytest.mark.parametrize("C", [256, 512])
 @pytest.mark.parametrize("kind,n", [("ico", 3), ("open", 9), ("ico", 40)])
-def test_spmm_tensor_memory_statistics_kernel_equals_shared_memory_kernel_bitwise(kind, n, C):
+def test_spmm_tensor_memory_statistics_kernel_equals_reference_kernel_bitwise(kind, n, C):
     """spmm_gcn_stats_tmem_kernel (forward flavour of the wide layers: per-warp Welford state in TMEM through
-    tcgen05.ld / tcgen05.st instead of 32 KB of shared memory; flag 4 of ddmp_spmm_use_tile_kernel) keeps the warp -> row
-    assignment, the per-element accumulation order and the Chan merge of spmm_gcn_kernel: Y and the (sum, M2) block
-    partials must be IDENTICAL -- with and without bias, ragged last block, partitioned layout, repeated launches (TMEM
-    allocation / release)."""
+    tcgen05.ld / tcgen05.st instead of 32 KB of shared memory; the default) keeps the warp -> row assignment, the
+    per-element accumulation order and the Chan merge of spmm_gcn_kernel (ddmp_spmm_reference_kernel): Y and the
+    (sum, M2) block partials must be IDENTICAL -- with and without bias, ragged last block, partitioned layout, repeated
+    launches (TMEM allocation / release)."""
     from dual_dmp_b200 import functional as F_
     from dual_dmp_b200._lib import lib
     from dual_dmp_b200.graph import GcnGraph
@@ -606,7 +607,7 @@ def test_spmm_tensor_memory_statistics_kernel_equals_shared_memory_kernel_bitwis
     graphs_ = [GcnGraph(ds.edge_index, V, DEV, coords=ds.x_pos, reorder=True),
                GcnGraph(ds.face_index, F, DEV, coords=ds.z2.detach()[:, :3], reorder=True)]
     torch.manual_seed(C + n)
-    prev = lib.query("ddmp_spmm_use_tile_kernel", 0)
+    prev = lib.query("ddmp_spmm_reference_kernel", 0)
     try:
         for graph in graphs_:
             H = torch.randn(graph.n, C, device=DEV)
@@ -615,18 +616,17 @@ def test_spmm_tensor_memory_statistics_kernel_equals_shared_memory_kernel_bitwis
             rp = graph.rowptr[: n_own + 1].contiguous()
             sub = type("G", (), dict(rowptr=rp, col=graph.col, w=graph.w, rowptr_t=rp, col_t=graph.col, w_t=graph.w))
             res = {}
-            for flags in (2, 2 | 4 | 8, 4 | 8):
-                lib.query("ddmp_spmm_use_tile_kernel", 1 | (flags << 4))
+            for ref in (1, 0):
+                lib.query("ddmp_spmm_reference_kernel", ref)
                 out = []
                 for _ in range(3):
                     out += [*F_.spmm_gcn(graph, H, bias=b, stats=True), *F_.spmm_gcn(graph, H, stats=True),
                             *F_.spmm_gcn(sub, H, bias=b, stats=True, n_rows=n_own)]
-                res[flags] = out
-            for flags in (2 | 4 | 8, 4 | 8):
-                for i, (x, x0) in enumerate(zip(res[flags], res[2])):
-                    assert torch.equal(x, x0), (flags, i, graph.n, C)
+                res[ref] = out
+            for i, (x, x0) in enumerate(zip(res[0], res[1])):
+                assert torch.equal(x, x0), (i, graph.n, C)
     finally:
-        lib.query("ddmp_spmm_use_tile_kernel", prev)
+        lib.query("ddmp_spmm_reference_kernel", prev)
 
 
 @pytest.mark.parametrize("C", [32, 64, 128, 256, 512])
