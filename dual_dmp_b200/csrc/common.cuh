@@ -108,11 +108,6 @@ int make_tensor_map_2d(void* map, const float* base, int64_t outer, int64_t inne
 
 // tile-staged aggregation kernel (spmm_tile.cu)
 bool spmm_tile_supported(int64_t n, int C);
-int spmm_bn_bwd_tile_rows(int C);
-int spmm_bn_bwd_tile_launch(const int* rowptr, const int* col, const float* w, const float* gX, const float* Y,
-                            const float* mean, const float* rstd, const float* scale, const float* shift,
-                            const float* c1, const float* c2, float slope, float* dH, float* colsum, float* amax,
-                            int64_t n, int C, cudaStream_t st);
 int spmm_tile_launch(const int* rowptr, const int* col, const float* w, const float* H, const float* bias, float* Y,
                      float* partials, float* amax, int64_t n, int C, cudaStream_t st);
 

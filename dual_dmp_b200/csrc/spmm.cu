@@ -423,142 +423,6 @@ spmm_gcn_stats_tmem_kernel(const int* __restrict__ rowptr, const int* __restrict
     }
 }
 
-// Backward aggregation fused with the BatchNorm/LeakyReLU backward "apply":
-//     dH[i,:] = sum_k w[k] * dY[col[k],:],   dY = scale*(gZ - c1 - xhat*c2),  gZ = gX * lrelu'(scale*Y+shift)
-// dY is never written: it is recomputed from the gathered rows of gX and Y as  dY = scale*gZ + A - B*Y  with the
-// per-channel constants A = scale*(c2*rstd*mean - c1), B = scale*c2*rstd (built once per launch in shared memory).
-// This removes the separate apply pass (read gX, read Y, write dY) and the read of dY: 3 passes instead of 5 over
-// [n, C]; the gather volume through L2 doubles.  The conv-bias gradient (column sums of dY over the rows) comes
-// from each row's own dY.  Channels are processed in halves of at most 2 float4 per lane to bound the registers.
-template <int C>
-__global__ void __launch_bounds__(256, 3)
-spmm_bn_bwd_kernel(const int* __restrict__ rowptr, const int* __restrict__ col, const float* __restrict__ w,
-                   const float* __restrict__ gX, const float* __restrict__ Y, const float* __restrict__ mean,
-                   const float* __restrict__ rstd, const float* __restrict__ scale, const float* __restrict__ shift,
-                   const float* __restrict__ c1, const float* __restrict__ c2, float slope, float* __restrict__ dH,
-                   float* __restrict__ partials, int64_t n, int rows_per_block) {
-    constexpr int G = (C / 4 < 32) ? (C / 4) : 32;
-    constexpr int NV = C / (4 * G);
-    constexpr int HV = NV < 2 ? NV : 2;
-    constexpr int GROUPS = 256 / G;
-    __shared__ __align__(16) float cst[4 * C];          // scale | shift | A | B
-    __shared__ __align__(16) float red[GROUPS * C];     // per-group column sums of dY (bias gradient)
-    for (int c = threadIdx.x; c < C; c += 256) {
-        const float sc = scale[c], k1 = c1[c], k2 = c2[c], rs = rstd[c], mu = mean[c];
-        cst[c] = sc;
-        cst[C + c] = shift[c];
-        cst[2 * C + c] = sc * (k2 * rs * mu - k1);
-        cst[3 * C + c] = sc * k2 * rs;
-    }
-    const int lane = threadIdx.x & 31;
-    const int lg = lane % G;
-    const int gid = threadIdx.x / G;
-    const unsigned gmask = (G == 32) ? 0xffffffffu : (((1u << G) - 1u) << ((lane / G) * G));
-    float* myred = red + gid * C;
-#pragma unroll
-    for (int v = 0; v < NV; ++v) st4(myred + (v * G + lg) * 4, make_float4(0.f, 0.f, 0.f, 0.f));
-    __syncthreads();
-
-    const int64_t row0 = (int64_t)blockIdx.x * rows_per_block;
-    const int64_t row_end = (row0 + rows_per_block < n) ? (row0 + rows_per_block) : n;
-    auto dy4 = [&](const float4& g, const float4& y, const float4& sc, const float4& sh, const float4& A,
-                   const float4& B) {
-        float4 d;
-        d.x = fmaf(sc.x, (fmaf(y.x, sc.x, sh.x) > 0.f) ? g.x : g.x * slope, fmaf(-B.x, y.x, A.x));
-        d.y = fmaf(sc.y, (fmaf(y.y, sc.y, sh.y) > 0.f) ? g.y : g.y * slope, fmaf(-B.y, y.y, A.y));
-        d.z = fmaf(sc.z, (fmaf(y.z, sc.z, sh.z) > 0.f) ? g.z : g.z * slope, fmaf(-B.z, y.z, A.z));
-        d.w = fmaf(sc.w, (fmaf(y.w, sc.w, sh.w) > 0.f) ? g.w : g.w * slope, fmaf(-B.w, y.w, A.w));
-        return d;
-    };
-    for (int64_t r = row0 + gid; r < row_end; r += GROUPS) {
-        const int start = __ldg(rowptr + r), end = __ldg(rowptr + r + 1);
-#pragma unroll
-        for (int h = 0; h < NV; h += HV) {
-            float4 sc[HV], sh[HV], A[HV], B[HV], acc[HV];
-#pragma unroll
-            for (int v = 0; v < HV; ++v) {
-                const int c = ((h + v) * G + lg) * 4;
-                sc[v] = *reinterpret_cast<const float4*>(cst + c);
-                sh[v] = *reinterpret_cast<const float4*>(cst + C + c);
-                A[v] = *reinterpret_cast<const float4*>(cst + 2 * C + c);
-                B[v] = *reinterpret_cast<const float4*>(cst + 3 * C + c);
-                acc[v] = make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-            for (int k0 = start; k0 < end; k0 += G) {
-                const int kk = k0 + lg;
-                const int myc = (kk < end) ? __ldg(col + kk) : 0;
-                const float myw = (kk < end) ? __ldg(w + kk) : 0.f;
-                const int cnt = (end - k0 < G) ? (end - k0) : G;
-                int j = 0;
-                for (; j + 2 <= cnt; j += 2) {
-                    const int ca = __shfl_sync(gmask, myc, j, G), cb = __shfl_sync(gmask, myc, j + 1, G);
-                    const float wa = __shfl_sync(gmask, myw, j, G), wb = __shfl_sync(gmask, myw, j + 1, G);
-                    float4 ga[HV], ya[HV], gb[HV], yb[HV];
-#pragma unroll
-                    for (int v = 0; v < HV; ++v) {
-                        const int c = ((h + v) * G + lg) * 4;
-                        ga[v] = ldg4(gX + (int64_t)ca * C + c); ya[v] = ldg4(Y + (int64_t)ca * C + c);
-                        gb[v] = ldg4(gX + (int64_t)cb * C + c); yb[v] = ldg4(Y + (int64_t)cb * C + c);
-                    }
-#pragma unroll
-                    for (int v = 0; v < HV; ++v) {
-                        const float4 da = dy4(ga[v], ya[v], sc[v], sh[v], A[v], B[v]);
-                        const float4 db = dy4(gb[v], yb[v], sc[v], sh[v], A[v], B[v]);
-                        acc[v].x = fmaf(wa, da.x, acc[v].x); acc[v].y = fmaf(wa, da.y, acc[v].y);
-                        acc[v].z = fmaf(wa, da.z, acc[v].z); acc[v].w = fmaf(wa, da.w, acc[v].w);
-                        acc[v].x = fmaf(wb, db.x, acc[v].x); acc[v].y = fmaf(wb, db.y, acc[v].y);
-                        acc[v].z = fmaf(wb, db.z, acc[v].z); acc[v].w = fmaf(wb, db.w, acc[v].w);
-                    }
-                }
-                for (; j < cnt; ++j) {
-                    const int ca = __shfl_sync(gmask, myc, j, G);
-                    const float wa = __shfl_sync(gmask, myw, j, G);
-#pragma unroll
-                    for (int v = 0; v < HV; ++v) {
-                        const int c = ((h + v) * G + lg) * 4;
-                        const float4 da = dy4(ldg4(gX + (int64_t)ca * C + c), ldg4(Y + (int64_t)ca * C + c), sc[v], sh[v],
-                                              A[v], B[v]);
-                        acc[v].x = fmaf(wa, da.x, acc[v].x); acc[v].y = fmaf(wa, da.y, acc[v].y);
-                        acc[v].z = fmaf(wa, da.z, acc[v].z); acc[v].w = fmaf(wa, da.w, acc[v].w);
-                    }
-                }
-            }
-#pragma unroll
-            for (int v = 0; v < HV; ++v) {
-                const int c = ((h + v) * G + lg) * 4;
-                st4(dH + r * C + c, acc[v]);
-                if (partials) {      // own row's dY -> bias-gradient partial sums
-                    const float4 d = dy4(ldg4(gX + r * C + c), ldg4(Y + r * C + c), sc[v], sh[v], A[v], B[v]);
-                    float4 t = *reinterpret_cast<float4*>(myred + c);
-                    t.x += d.x; t.y += d.y; t.z += d.z; t.w += d.w;
-                    st4(myred + c, t);
-                }
-            }
-        }
-    }
-    if (partials) {
-        __syncthreads();
-        float* outp = partials + (int64_t)blockIdx.x * C;
-        for (int i = threadIdx.x; i < C; i += 256) {
-            float t = 0.f;
-#pragma unroll 8
-            for (int g = 0; g < GROUPS; ++g) t += red[g * C + i];
-            outp[i] = t;
-        }
-    }
-}
-
-template <int C>
-static int launch_spmm_bn_bwd(const int* rowptr, const int* col, const float* w, const float* gX, const float* Y,
-                              const float* mean, const float* rstd, const float* scale, const float* shift,
-                              const float* c1, const float* c2, float slope, float* dH, float* partials, int64_t n,
-                              cudaStream_t st) {
-    const int rpb = ddmp_rows_per_block(C);
-    spmm_bn_bwd_kernel<C><<<(unsigned)ceil_div(n, rpb), 256, 0, st>>>(rowptr, col, w, gX, Y, mean, rstd, scale, shift,
-                                                                      c1, c2, slope, dH, partials, n, rpb);
-    return check_launch("spmm_bn_bwd");
-}
-
 // Any width: one warp per row, lanes stride over channels (operator-level GCNConv with unusual widths).
 __global__ void __launch_bounds__(256)
 spmm_gcn_generic_kernel(const int* __restrict__ rowptr, const int* __restrict__ col, const float* __restrict__ w,
@@ -660,54 +524,8 @@ int ddmp_spmm_gcn(const int32_t* rowptr, const int32_t* col, const float* w, con
     return check_launch("spmm_gcn_generic");
 }
 
-int64_t ddmp_spmm_bn_bwd_tile_blocks(int64_t n, int32_t C) {
-    const int r = ddmp::spmm_bn_bwd_tile_rows(C);
-    return n <= 0 ? 0 : (n + r - 1) / r;
-}
-
-int64_t ddmp_spmm_bn_bwd_tile_amax_len(int64_t n, int32_t C) {
-    return ddmp_spmm_bn_bwd_tile_blocks(n, C) * (C > 128 ? C / 128 : 1);
-}
-
-int ddmp_spmm_bn_bwd_tile(const int32_t* rowptr, const int32_t* col, const float* w, const float* gX, const float* Y,
-                          const float* mean, const float* rstd, const float* scale, const float* shift,
-                          const float* c1, const float* c2, float slope, float* dH, float* colsum_partials,
-                          float* amax_blocks, int64_t n, int32_t C, void* stream) {
-    using namespace ddmp;
-    DDMP_REQUIRE(n >= 0 && n < (1ll << 31), "spmm_bn_bwd_tile: bad row count");
-    DDMP_REQUIRE(C == 32 || C == 64 || (C >= 128 && C <= 512 && C % 128 == 0),
-                 "spmm_bn_bwd_tile: C must be 32, 64 or a multiple of 128 up to 512 (got %d)", C);
-    if (n == 0) return DDMP_OK;
-    DDMP_REQUIRE(rowptr && col && w && gX && Y && mean && rstd && scale && shift && c1 && c2 && dH,
-                 "spmm_bn_bwd_tile: null pointer");
-    return spmm_bn_bwd_tile_launch(rowptr, col, w, gX, Y, mean, rstd, scale, shift, c1, c2, slope, dH, colsum_partials,
-                                   amax_blocks, n, C, as_stream(stream));
-}
-
 int ddmp_spmm_reference_kernel(int on) { return ddmp::g_reference_kernel.exchange(on != 0, std::memory_order_relaxed); }
 
 int64_t ddmp_spmm_amax_len(int64_t n, int32_t C) { return ddmp_num_row_blocks(n, C); }
-
-int ddmp_spmm_bn_bwd(const int32_t* rowptr, const int32_t* col, const float* w, const float* gX, const float* Y,
-                     const float* mean, const float* rstd, const float* scale, const float* shift, const float* c1,
-                     const float* c2, float slope, float* dH, float* colsum_partials, int64_t n, int32_t C,
-                     void* stream) {
-    using namespace ddmp;
-    DDMP_REQUIRE(n >= 0 && C > 0, "spmm_bn_bwd: bad shape");
-    if (n == 0) return DDMP_OK;
-    DDMP_REQUIRE(rowptr && col && w && gX && Y && mean && rstd && scale && shift && c1 && c2 && dH,
-                 "spmm_bn_bwd: null pointer");
-    cudaStream_t st = as_stream(stream);
-    switch (C) {
-        case 32: return launch_spmm_bn_bwd<32>(rowptr, col, w, gX, Y, mean, rstd, scale, shift, c1, c2, slope, dH, colsum_partials, n, st);
-        case 64: return launch_spmm_bn_bwd<64>(rowptr, col, w, gX, Y, mean, rstd, scale, shift, c1, c2, slope, dH, colsum_partials, n, st);
-        case 128: return launch_spmm_bn_bwd<128>(rowptr, col, w, gX, Y, mean, rstd, scale, shift, c1, c2, slope, dH, colsum_partials, n, st);
-        case 256: return launch_spmm_bn_bwd<256>(rowptr, col, w, gX, Y, mean, rstd, scale, shift, c1, c2, slope, dH, colsum_partials, n, st);
-        case 512: return launch_spmm_bn_bwd<512>(rowptr, col, w, gX, Y, mean, rstd, scale, shift, c1, c2, slope, dH, colsum_partials, n, st);
-        default: break;
-    }
-    set_error("spmm_bn_bwd: supports C in {32,64,128,256,512}, got %d", C);
-    return DDMP_ERR_UNSUPPORTED;
-}
 
 }  // extern "C"

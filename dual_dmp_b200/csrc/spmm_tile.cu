@@ -205,191 +205,15 @@ spmm_tile_kernel(const __grid_constant__ CUtensorMap hmap, const Args a) {
     }
 }
 
-// Backward aggregation fused with the BatchNorm / LeakyReLU backward "apply" (replaces ddmp_bn_bwd_apply + ddmp_spmm_gcn
-// on the backward pass; reference: autograd of nn.BatchNorm1d + nn.LeakyReLU + GCNConv.propagate,
-// util/networks.py:51-62):
-//     dY = scale * (gZ - c1 - xhat * c2),  gZ = gX * lrelu'(scale*Y + shift),  xhat = (Y - mean) * rstd
-//     dH[i,:] = sum_k w[k] * dY[col[k],:]          colsum[c] = sum_i dY[i,c]   (conv-bias gradient)
-// The block's own rows of gX and Y arrive by two TMA tensor copies; dY of those rows is formed ONCE in shared memory
-// (in place over the gX tile) and the in-block gathers read it from there; a reference that leaves the block recomputes
-// dY from the two global rows.  dY is never written to HBM: per layer the pass reads gX and Y and writes dH (3 tensor
-// passes + halo) instead of 5 (apply: read gX, Y, write dY; aggregate: read dY, write dH).
-struct BwdArgs {
-    const int* rowptr;
-    const int* col;
-    const float* w;
-    const float* gX;
-    const float* Y;
-    const float* mean;
-    const float* rstd;
-    const float* scale;
-    const float* shift;
-    const float* c1;
-    const float* c2;
-    float slope;
-    float* dH;
-    float* colsum;        // [nblk][C] or null
-    float* amax;          // [nblk * slices] or null
-    int64_t n;
-    int C;
-};
-
-template <int CS, int R>
-__global__ void __launch_bounds__(kThreads)
-spmm_bn_bwd_tile_kernel(const __grid_constant__ CUtensorMap gmap, const __grid_constant__ CUtensorMap ymap,
-                        const BwdArgs a) {
-    constexpr int G = CS / 4;
-    constexpr int GROUPS = kThreads / G;
-    constexpr int kMetaCap = R * kMetaPerRow;
-    static_assert(GROUPS * CS * 4 <= R * CS * 4, "the column-sum scratch aliases the Y tile");
-    extern __shared__ unsigned char smem_raw[];
-    unsigned char* base = smem_raw + ((128u - (smem_u32(smem_raw) & 127u)) & 127u);
-    float* tg = reinterpret_cast<float*>(base);                                         // gX tile, then dY  [R][CS]
-    float* ty = tg + R * CS;                                                            // Y tile, then scratch
-    int* scol = reinterpret_cast<int*>(ty + R * CS);
-    float* sw = reinterpret_cast<float*>(scol + kMetaCap);
-    int* srow = reinterpret_cast<int*>(sw + kMetaCap);
-    uint64_t* barp = reinterpret_cast<uint64_t*>(srow + R + 2 + ((R & 1) ? 1 : 0));
-    float* wmax = reinterpret_cast<float*>(barp + 1);
-    uint64_t& bar = *barp;
-
-    const int slices = a.C / CS;
-    const int64_t blk = blockIdx.x / slices;
-    const int ch0 = (blockIdx.x % slices) * CS;
-    const int64_t row0 = blk * R;
-    const int rows = (int)((row0 + R <= a.n) ? R : (a.n - row0));
-    const int lane = threadIdx.x & 31;
-    const int lg = threadIdx.x % G;
-    const int gid = threadIdx.x / G;
-
-    if (threadIdx.x == 0) {
-        mbar_init(&bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        mbar_expect_tx(&bar, (uint32_t)(2 * R * CS * 4));
-        tma_load_2d(tg, &gmap, ch0, (int)row0, &bar);
-        tma_load_2d(ty, &ymap, ch0, (int)row0, &bar);
-    }
-    for (int i = threadIdx.x; i <= rows; i += kThreads) srow[i] = __ldg(a.rowptr + row0 + i);
-    // per-lane channel constants (this lane's four channels of the slice)
-    const int c = ch0 + lg * 4;
-    const float4 mu = ldg4(a.mean + c), rs = ldg4(a.rstd + c), sc = ldg4(a.scale + c), sh = ldg4(a.shift + c);
-    const float4 k1 = ldg4(a.c1 + c), k2 = ldg4(a.c2 + c);
-    const float slope = a.slope;
-    auto dy4 = [&](const float4& g, const float4& y) {          // same arithmetic as bn.cu rowblock_kernel<1>
-        float4 d;
-        const float gzx = (fmaf(y.x, sc.x, sh.x) > 0.f) ? g.x : g.x * slope;
-        const float gzy = (fmaf(y.y, sc.y, sh.y) > 0.f) ? g.y : g.y * slope;
-        const float gzz = (fmaf(y.z, sc.z, sh.z) > 0.f) ? g.z : g.z * slope;
-        const float gzw = (fmaf(y.w, sc.w, sh.w) > 0.f) ? g.w : g.w * slope;
-        d.x = sc.x * (gzx - k1.x - ((y.x - mu.x) * rs.x) * k2.x);
-        d.y = sc.y * (gzy - k1.y - ((y.y - mu.y) * rs.y) * k2.y);
-        d.z = sc.z * (gzz - k1.z - ((y.z - mu.z) * rs.z) * k2.z);
-        d.w = sc.w * (gzw - k1.w - ((y.w - mu.w) * rs.w) * k2.w);
-        return d;
-    };
-    __syncthreads();
-    const int kb = srow[0];
-    const int nk = srow[rows] - kb;
-    const bool meta_in_smem = nk <= kMetaCap;
-    if (meta_in_smem) {
-        for (int i = threadIdx.x; i < nk; i += kThreads) {
-            scol[i] = __ldg(a.col + kb + i);
-            sw[i] = __ldg(a.w + kb + i);
-        }
-    }
-    mbar_wait(&bar, 0);
-    // dY of the block's own rows, in place over the gX tile; column sums of dY (rows of this block only)
-    float4 csum = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int r = gid; r < rows; r += GROUPS) {
-        float4* pg = reinterpret_cast<float4*>(tg + r * CS + lg * 4);
-        const float4 d = dy4(*pg, *reinterpret_cast<const float4*>(ty + r * CS + lg * 4));
-        *pg = d;
-        csum.x += d.x; csum.y += d.y; csum.z += d.z; csum.w += d.w;
-    }
-    __syncthreads();
-    if (a.colsum) {
-        float* red = ty;                                        // the Y tile is dead now
-        st4(red + gid * CS + lg * 4, csum);
-        __syncthreads();
-        for (int i = threadIdx.x; i < CS; i += kThreads) {
-            float t = 0.f;
-#pragma unroll 8
-            for (int g = 0; g < GROUPS; ++g) t += red[g * CS + i];
-            a.colsum[blk * a.C + ch0 + i] = t;
-        }
-    }
-
-    float amx = 0.f;
-    const float* Gs = a.gX + c;
-    const float* Ys = a.Y + c;
-    for (int r = gid; r < rows; r += GROUPS) {
-        const int s = srow[r] - kb, e = srow[r + 1] - kb;
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-        int k = s;
-        for (; k + 4 <= e; k += 4) {
-            int cc[4];
-            float wv[4];
-            float4 x[4], y[4];
-            bool in[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                cc[u] = meta_in_smem ? scol[k + u] : __ldg(a.col + kb + k + u);
-                wv[u] = meta_in_smem ? sw[k + u] : __ldg(a.w + kb + k + u);
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int64_t lc = (int64_t)cc[u] - row0;
-                in[u] = (uint64_t)lc < (uint64_t)rows;
-                if (in[u]) x[u] = *reinterpret_cast<const float4*>(tg + (int)lc * CS + lg * 4);
-                else { x[u] = ldg4(Gs + (int64_t)cc[u] * a.C); y[u] = ldg4(Ys + (int64_t)cc[u] * a.C); }
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const float4 d = in[u] ? x[u] : dy4(x[u], y[u]);
-                acc.x = fmaf(wv[u], d.x, acc.x); acc.y = fmaf(wv[u], d.y, acc.y);
-                acc.z = fmaf(wv[u], d.z, acc.z); acc.w = fmaf(wv[u], d.w, acc.w);
-            }
-        }
-        for (; k < e; ++k) {
-            const int c1_ = meta_in_smem ? scol[k] : __ldg(a.col + kb + k);
-            const float w1 = meta_in_smem ? sw[k] : __ldg(a.w + kb + k);
-            const int64_t lc = (int64_t)c1_ - row0;
-            float4 d;
-            if ((uint64_t)lc < (uint64_t)rows) d = *reinterpret_cast<const float4*>(tg + (int)lc * CS + lg * 4);
-            else d = dy4(ldg4(Gs + (int64_t)c1_ * a.C), ldg4(Ys + (int64_t)c1_ * a.C));
-            acc.x = fmaf(w1, d.x, acc.x); acc.y = fmaf(w1, d.y, acc.y);
-            acc.z = fmaf(w1, d.z, acc.z); acc.w = fmaf(w1, d.w, acc.w);
-        }
-        st4(a.dH + (row0 + r) * a.C + c, acc);
-        amx = fmaxf(fmaxf(amx, fmaxf(fabsf(acc.x), fabsf(acc.y))), fmaxf(fabsf(acc.z), fabsf(acc.w)));
-    }
-    if (a.amax) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) amx = fmaxf(amx, __shfl_xor_sync(0xffffffffu, amx, o));
-        if (lane == 0) wmax[threadIdx.x >> 5] = amx;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            float m = wmax[0];
-#pragma unroll
-            for (int i = 1; i < kThreads / 32; ++i) m = fmaxf(m, wmax[i]);
-            a.amax[blockIdx.x] = m;
-        }
-    }
-}
-
-template <int CS, int R>
+template <int C, int R>
 constexpr size_t smem_bytes() {
-    return 128 + (size_t)R * CS * 4 + (size_t)R * kMetaPerRow * 8 + (size_t)(R + 4) * 4 + 8 + (kThreads / 32) * 4 + 16;
-}
-
-static int make_map(CUtensorMap* map, const float* H, int64_t n, int C, int CS, int R) {
-    return make_tensor_map_2d(map, H, n, C, R, CS, false, "spmm_tile");
+    return 128 + (size_t)R * C * 4 + (size_t)R * kMetaPerRow * 8 + (size_t)(R + 4) * 4 + 8 + (kThreads / 32) * 4 + 16;
 }
 
 template <int C, int R>
 static int launch(const Args& a, cudaStream_t st) {
     CUtensorMap map;
-    int rc = make_map(&map, a.H, a.n, C, C, R);
+    int rc = make_tensor_map_2d(&map, a.H, a.n, C, R, C, false, "spmm_tile");
     if (rc != DDMP_OK) return rc;
     const int64_t nblk = ceil_div(a.n, R);
     const bool stats = a.partials != nullptr, bias = a.bias != nullptr;
@@ -413,44 +237,7 @@ static int launch(const Args& a, cudaStream_t st) {
     return check_launch("spmm_tile");
 }
 
-template <int CS, int R>
-constexpr size_t bwd_smem_bytes() {
-    return 128 + (size_t)2 * R * CS * 4 + (size_t)R * kMetaPerRow * 8 + (size_t)(R + 4) * 4 + 8 + (kThreads / 32) * 4 + 16;
-}
-
-template <int CS, int R>
-static int launch_bwd(const BwdArgs& a, cudaStream_t st) {
-    CUtensorMap gmap, ymap;
-    int rc = make_map(&gmap, a.gX, a.n, a.C, CS, R);
-    if (rc != DDMP_OK) return rc;
-    rc = make_map(&ymap, a.Y, a.n, a.C, CS, R);
-    if (rc != DDMP_OK) return rc;
-    const int64_t nblk = ceil_div(a.n, R);
-    const unsigned grid = (unsigned)(nblk * (a.C / CS));
-    const size_t smem = bwd_smem_bytes<CS, R>();
-    static PerDeviceOnce configured;
-    if (configured.need()) {
-        DDMP_CUDA(cudaFuncSetAttribute(spmm_bn_bwd_tile_kernel<CS, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured.mark();
-    }
-    spmm_bn_bwd_tile_kernel<CS, R><<<grid, kThreads, smem, st>>>(gmap, ymap, a);
-    return check_launch("spmm_bn_bwd_tile");
-}
-
 }  // namespace tile
-
-// rows per CTA of the fused backward kernel (two tiles per CTA, so half the forward kernel's block)
-int spmm_bn_bwd_tile_rows(int C) { return C == 32 ? 256 : (C == 64 ? 128 : 64); }
-
-int spmm_bn_bwd_tile_launch(const int* rowptr, const int* col, const float* w, const float* gX, const float* Y,
-                            const float* mean, const float* rstd, const float* scale, const float* shift,
-                            const float* c1, const float* c2, float slope, float* dH, float* colsum, float* amax,
-                            int64_t n, int C, cudaStream_t st) {
-    tile::BwdArgs a{rowptr, col, w, gX, Y, mean, rstd, scale, shift, c1, c2, slope, dH, colsum, amax, n, C};
-    if (C == 32) return tile::launch_bwd<32, 256>(a, st);
-    if (C == 64) return tile::launch_bwd<64, 128>(a, st);
-    return tile::launch_bwd<128, 64>(a, st);
-}
 
 // the widths where this kernel beats the gather kernel on B200 (1M-face graphs, profiles/spmm_tile_ab_r2.txt); the TMA
 // row coordinate is a 32-bit int

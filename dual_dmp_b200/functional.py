@@ -7,8 +7,6 @@ activated tensors are recomputed on load by the consumers (SURVEY.md §7 hard pa
 """
 from __future__ import annotations
 
-import os
-
 import torch
 
 from ._lib import lib, ptr, require_cuda, set_device, stream_ptr
@@ -22,15 +20,6 @@ GEMM_BACKEND = 0    # DDMP_GEMM_AUTO; tests may set 1 (FFMA) / 2 (tcgen05)
 # "fp32" = the fp16-split tensor-core kernels emulate fp32 with three products (default); "f16x1" = one fp16 product
 GEMM_F16X1 = 0x10   # DDMP_GEMM_F16X1, OR-ed into the backend argument
 DENSE_PRECISIONS = ("fp32", "f16x1")
-# backward: recompute dY inside the aggregation kernel (ddmp_spmm_bn_bwd) instead of materialising it.  OFF: measured
-# on B200 at 1M faces the doubled gather volume through L2 costs more than the two saved passes over dY (C=512:
-# 1.82 vs 1.37 ms vertex graph, 2.87 vs 2.52 ms face graph; scripts/bench_bn_spmm.py) -- kept for narrower graphs.
-FUSE_BN_SPMM = False
-# backward: BatchNorm/LeakyReLU "apply" folded into the TILE-staged aggregation kernel (ddmp_spmm_bn_bwd_tile): dY of a row
-# block is formed once in shared memory from the TMA-staged gX / Y tiles, so the gather volume does not double and dY
-# never goes to HBM (3 tensor passes per layer instead of 5).  Single-GPU path only (the partitioned mode exchanges dY).
-FUSE_BN_SPMM_TILE = os.environ.get("DDMP_FUSE_BN_TILE", "0") != "0"
-TILE_WIDTHS = (32, 64, 128, 256, 384, 512)
 
 HEAD_POS, HEAD_NORM = 0, 1
 
@@ -223,54 +212,7 @@ def bn_lrelu_backward(gX, Y, stats, dY_out=None, comm=None):
     return dY, small[0], small[1], small[4]
 
 
-def bn_bwd_spmm_fused(graph, gX, Y, stats, dH_out=None):
-    """BatchNorm/LeakyReLU backward + backward aggregation with dY never materialised:
-    reduce (sum gZ, sum gZ*xhat) -> finalize -> ddmp_spmm_bn_bwd.  Returns (dH, dgamma, dbeta, dbias)."""
-    n, C = Y.shape
-    dev = Y.device
-    st = stream_ptr(dev)
-    nblk = num_elem_blocks(n, C)
-    partials = torch.empty(nblk, 2, C, dtype=torch.float32, device=dev)
-    nblk_s = num_row_blocks(n, C)                                          # row blocks of the aggregation kernel
-    colsum_p = torch.empty(nblk_s, 1, C, dtype=torch.float32, device=dev)
-    small = torch.empty(5, C, dtype=torch.float32, device=dev)             # dgamma, dbeta, c1, c2, dbias
-    mean, rstd, scale, shift = stats[0], stats[1], stats[2], stats[3]
-    lib.call("ddmp_bn_bwd_reduce", ptr(gX), ptr(Y), ptr(mean), ptr(rstd), ptr(scale), ptr(shift), SLOPE,
-             ptr(partials), n, C, st)
-    lib.call("ddmp_bn_bwd_finalize", ptr(partials), nblk, n, C, ptr(small[0]), ptr(small[1]), ptr(small[2]),
-             ptr(small[3]), st)
-    dH = dH_out if dH_out is not None else torch.empty_like(Y)
-    lib.call("ddmp_spmm_bn_bwd", ptr(graph.rowptr), ptr(graph.col), ptr(graph.w), ptr(gX), ptr(Y), ptr(mean),
-             ptr(rstd), ptr(scale), ptr(shift), ptr(small[2]), ptr(small[3]), SLOPE, ptr(dH), ptr(colsum_p), n, C, st)
-    lib.call("ddmp_colsum_finalize", ptr(colsum_p), nblk_s, 1, C, ptr(small[4]), st)
-    return dH, small[0], small[1], small[4]
-
-
-def bn_bwd_spmm_tile(graph, gX, Y, stats, dH_out=None, amax=False):
-    """BatchNorm/LeakyReLU backward + backward aggregation on the tile-staged kernel: reduce (sum gZ, sum gZ*xhat) ->
-    finalize -> ddmp_spmm_bn_bwd_tile (dY formed in shared memory, never written).  Returns
-    (dH, dgamma, dbeta, dbias, amax_blocks or None)."""
-    n, C = Y.shape
-    dev = Y.device
-    st = stream_ptr(dev)
-    nblk = num_elem_blocks(n, C)
-    partials = torch.empty(nblk, 2, C, dtype=torch.float32, device=dev)
-    small = torch.empty(5, C, dtype=torch.float32, device=dev)             # dgamma, dbeta, c1, c2, dbias
-    mean, rstd, scale, shift = stats[0], stats[1], stats[2], stats[3]
-    lib.call("ddmp_bn_bwd_reduce", ptr(gX), ptr(Y), ptr(mean), ptr(rstd), ptr(scale), ptr(shift), SLOPE,
-             ptr(partials), n, C, st)
-    lib.call("ddmp_bn_bwd_finalize", ptr(partials), nblk, n, C, ptr(small[0]), ptr(small[1]), ptr(small[2]),
-             ptr(small[3]), st)
-    dH = dH_out if dH_out is not None else torch.empty_like(Y)
-    nblk_t = int(lib.query("ddmp_spmm_bn_bwd_tile_blocks", n, C))
-    colsum = torch.empty(nblk_t, 1, C, dtype=torch.float32, device=dev)
-    ab = torch.empty(int(lib.query("ddmp_spmm_bn_bwd_tile_amax_len", n, C)), dtype=torch.float32, device=dev) \
-        if amax else None
-    lib.call("ddmp_spmm_bn_bwd_tile", ptr(graph.rowptr), ptr(graph.col), ptr(graph.w), ptr(gX), ptr(Y), ptr(mean),
-             ptr(rstd), ptr(scale), ptr(shift), ptr(small[2]), ptr(small[3]), SLOPE, ptr(dH), ptr(colsum), ptr(ab), n, C,
-             st)
-    lib.call("ddmp_colsum_finalize", ptr(colsum), nblk_t, 1, C, ptr(small[4]), st)
-    return dH, small[0], small[1], small[4], ab
+bn_bwd_spmm_tile = None     # never called: bench.py's per-phase timer patches this name; goes with that line of bench.py
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -402,8 +344,7 @@ class GcnNetFunction(torch.autograd.Function):
         comm = graph if hasattr(graph, "exchange") else None
         n_ext = graph.n_ext if comm is not None else n
         bufA = torch.empty(n * cmax, dtype=torch.float32, device=dev)      # gX (grad wrt activated layer output)
-        fused = comm is None and (FUSE_BN_SPMM or FUSE_BN_SPMM_TILE) and graph.symmetric
-        bufB = None if fused else torch.empty(n_ext * cmax, dtype=torch.float32, device=dev)   # dY ([owned | halo])
+        bufB = torch.empty(n_ext * cmax, dtype=torch.float32, device=dev)  # dY ([owned | halo])
         bufC = torch.empty(n * cmax, dtype=torch.float32, device=dev)      # dH
         gX = bufA[: n * 32].view(n, 32)
         lib.call("ddmp_head_bwd", kind, ptr(g_out), ptr(graph.perm), ptr(W1), ptr(W2), ptr(ctx.h_save),
@@ -418,23 +359,15 @@ class GcnNetFunction(torch.autograd.Function):
         for l in range(L - 1, -1, -1):
             cout, cin = Ws[l].shape
             dH = bufC[: n * cout].view(n, cout)
+            dY = bufB[: n_ext * cout].view(n_ext, cout)
+            _, dgamma, dbeta, dbias = bn_lrelu_backward(gX, Ys[l], stats[l], dY_out=dY, comm=comm)
+            if comm is not None:
+                comm.exchange(dY)                   # A_hat symmetric: the backward needs dY of the halo rows
             dh_max = None                           # row-block maxima of |dH| when the aggregation kernel provides them
-            if comm is None and FUSE_BN_SPMM_TILE and graph.symmetric and cout in TILE_WIDTHS:
-                _, dgamma, dbeta, dbias, dh_max = bn_bwd_spmm_tile(graph, gX, Ys[l], stats[l], dH_out=dH,
-                                                                   amax=cout in AMAX_WIDTHS and l > 0)
-            elif comm is None and FUSE_BN_SPMM and graph.symmetric and cout in (32, 64, 128, 256, 512):
-                _, dgamma, dbeta, dbias = bn_bwd_spmm_fused(graph, gX, Ys[l], stats[l], dH_out=dH)
+            if cout in AMAX_WIDTHS and l > 0:
+                _, dh_max = spmm_gcn(graph, dY, transposed=True, out=dH, n_rows=n, amax=True)
             else:
-                if bufB is None:
-                    bufB = torch.empty(n_ext * cmax, dtype=torch.float32, device=dev)
-                dY = bufB[: n_ext * cout].view(n_ext, cout)
-                _, dgamma, dbeta, dbias = bn_lrelu_backward(gX, Ys[l], stats[l], dY_out=dY, comm=comm)
-                if comm is not None:
-                    comm.exchange(dY)               # A_hat symmetric: the backward needs dY of the halo rows
-                if cout in AMAX_WIDTHS and l > 0:
-                    _, dh_max = spmm_gcn(graph, dY, transposed=True, out=dH, n_rows=n, amax=True)
-                else:
-                    spmm_gcn(graph, dY, transposed=True, out=dH, n_rows=n)
+                spmm_gcn(graph, dY, transposed=True, out=dH, n_rows=n)
             if l == 0:
                 gW = gemm_dw(dH, x_in, cin, row_map=graph.perm, dense_precision=dense)
             else:

@@ -159,7 +159,7 @@ class PartitionedGraph:
         self.w = torch.from_numpy(p["w"]).to(dev)
         self.rowptr_t, self.col_t, self.w_t = self.rowptr, self.col, self.w
         self.nnz = int(p["col"].shape[0])
-        self.symmetric, self.identity, self.perm = True, False, None
+        self.identity, self.perm = False, None
         self.send_idx = torch.from_numpy(p["send_idx"]).to(dev)
         self.send_counts: List[int] = [int(x) for x in p["send_counts"]]
         self.recv_counts: List[int] = [int(x) for x in p["recv_counts"]]

@@ -91,29 +91,6 @@ int64_t ddmp_spmm_amax_len(int64_t n, int32_t C);
  * value (0 or 1). */
 int ddmp_spmm_reference_kernel(int on);
 
-/* Backward aggregation fused with ddmp_bn_bwd_apply:  dH = A_hat * dY  with dY recomputed on the fly from the gathered
- * rows of gX and Y (dY is never materialised); optional colsum_partials[b][0][c] = column sums of dY (conv bias
- * gradient).  Symmetric graphs only (the CSR is used as its own transpose); C in {32,64,128,256,512}. */
-int ddmp_spmm_bn_bwd(const int32_t* rowptr, const int32_t* col, const float* w, const float* gX, const float* Y,
-                     const float* mean, const float* rstd, const float* scale, const float* shift, const float* c1,
-                     const float* c2, float slope, float* dH, float* colsum_partials, int64_t n, int32_t C,
-                     void* stream);
-
-/* The same fusion on the tile-staged kernel (csrc/spmm_tile.cu): the row block's own rows of gX and Y arrive by two TMA
- * tensor copies, dY of those rows is formed once in shared memory and gathered from there; only references that leave
- * the block recompute dY from global rows.  Per layer the backward pass then moves 3 tensor passes (+ halo) instead of 5
- * (ddmp_bn_bwd_apply: read gX, Y, write dY; ddmp_spmm_gcn: read dY, write dH).  colsum_partials (optional):
- * [ddmp_spmm_bn_bwd_tile_blocks(n,C)][C] column sums of dY per row block (conv-bias gradient); amax_blocks (optional):
- * [ddmp_spmm_bn_bwd_tile_amax_len(n,C)] max |dH| per CTA.  n may be smaller than the row count of gX / Y (partitioned
- * mode: [owned | halo] rows, only owned rows are produced).  Symmetric graphs only.
- * [ref: autograd of nn.BatchNorm1d + nn.LeakyReLU + GCNConv.propagate, util/networks.py:51-62,112-123] */
-int ddmp_spmm_bn_bwd_tile(const int32_t* rowptr, const int32_t* col, const float* w, const float* gX, const float* Y,
-                          const float* mean, const float* rstd, const float* scale, const float* shift,
-                          const float* c1, const float* c2, float slope, float* dH, float* colsum_partials,
-                          float* amax_blocks, int64_t n, int32_t C, void* stream);
-int64_t ddmp_spmm_bn_bwd_tile_blocks(int64_t n, int32_t C);
-int64_t ddmp_spmm_bn_bwd_tile_amax_len(int64_t n, int32_t C);
-
 /* ---- BatchNorm1d (training mode) + LeakyReLU ------------------------------------------------------------ */
 /* partials [nblk][2][C] = per row block (sum of y, M2 = sum of (y - block mean)^2), as ddmp_spmm_gcn's epilogue emits
  * them (Welford per thread, Chan merge per block; nblk = ddmp_num_row_blocks(n, C)) -> batch mean / biased var, combined

@@ -203,53 +203,6 @@ def test_aggregation_default_kernels_equal_reference_on_long_rows(agg, C, restor
     report(f"long rows: aggregation kernels bitwise equal C={C}", len(res))
 
 
-def _ident(n):
-    from dual_dmp_b200.graph import GcnGraph
-    return GcnGraph(torch.zeros(2, 0, dtype=torch.long), n, DEV, reorder=False)
-
-
-@pytest.mark.parametrize("C", WIDTHS)
-def test_fused_bn_backward_aggregation_on_long_rows(agg, C):
-    """ddmp_spmm_bn_bwd (dY recomputed in the gather) and ddmp_spmm_bn_bwd_tile (dY formed in shared memory; global (col, w)
-    stream in the heavy row blocks) against ddmp_bn_bwd_apply + the backward aggregation, per row within
-    sum_k |w_k| (4 (L_i + 1) 2^-24 |dY_ck| + 16 2^-24 T_ck), T = |scale| (|gZ| + |c1| + |c2| rstd (|Y| + |mean|)) the
-    magnitude of the terms dY is formed from; dgamma / dbeta equal, conv-bias gradient and max|dH| checked, reruns equal"""
-    from dual_dmp_b200 import functional as F_
-    worst = 0.0
-    for name, g in agg["graphs"].items():
-        n = g.n
-        torch.manual_seed(300 + C)
-        Y = (torch.randn(n, C) * 1.5 + 0.3).to(DEV)
-        gX = torch.randn(n, C, device=DEV)
-        st = F_.bn_stats_finalize(F_.spmm_gcn(_ident(n), Y, stats=True)[1], n, (torch.rand(C) + 0.5).to(DEV),
-                                  torch.randn(C).to(DEV))
-        sc, sh, mu, rs = (st[i].double() for i in (2, 3, 0, 1))
-        for _ in range(3):        # away from the LeakyReLU kink: the slope must not depend on rounding
-            z = Y.double() * sc + sh
-            Y = torch.where(z.abs() < 1e-3, Y + 0.05, Y)
-        dY, dgamma, dbeta, dbias = F_.bn_lrelu_backward(gX, Y, st)
-        dH_ref = F_.spmm_gcn(g, dY, transposed=True)
-        z = Y.double() * sc + sh
-        gZ = torch.where(z > 0, gX.double(), gX.double() * F_.SLOPE)
-        c1, c2 = dbeta.double() / n, dgamma.double() / n
-        T = sc.abs() * (gZ.abs() + c1.abs() + c2.abs() * rs * (Y.double().abs() + mu.abs()))
-        aw = g.w.abs()
-        bound = 4.0 * (_row_len(g.rowptr, n) + 1.0).view(-1, 1) * U32 * _csr64(g.rowptr, g.col, aw, dY.abs(), n) + \
-            16.0 * U32 * _csr64(g.rowptr, g.col, aw, T, n) + 1e-30
-        dH1, dgamma1, dbeta1, dbias1 = F_.bn_bwd_spmm_fused(g, gX, Y, st)
-        dH2, dgamma2, dbeta2, dbias2, ab = F_.bn_bwd_spmm_tile(g, gX, Y, st, amax=True)
-        for which, dH, dg, db, dbb in (("gather", dH1, dgamma1, dbeta1, dbias1), ("tile", dH2, dgamma2, dbeta2, dbias2)):
-            r = float(((dH.double() - dH_ref.double()).abs() / bound).max())
-            worst = max(worst, r)
-            assert r <= 1.0, (name, which, r)
-            assert torch.equal(dg, dgamma) and torch.equal(db, dbeta), (name, which)
-            assert (dbb - dbias).abs().max() <= 1e-5 * dY.abs().sum(dim=0).max(), (name, which)
-        assert float(ab.max()) == float(dH2.abs().max())
-        assert torch.equal(F_.bn_bwd_spmm_fused(g, gX, Y, st)[0], dH1)
-        assert torch.equal(F_.bn_bwd_spmm_tile(g, gX, Y, st)[0], dH2)
-    report(f"long rows: fused BN backward aggregation C={C}: max |dH - unfused| / bound", worst)
-
-
 # ---------------------------------------------------------------------------------------------------------------------
 # losses, geometry, preprocessing
 # ---------------------------------------------------------------------------------------------------------------------

@@ -515,34 +515,6 @@ def test_fused_clip_adam_matches_torch():
 
 
 @pytest.mark.parametrize("C", [32, 64, 128, 256, 512])
-@pytest.mark.parametrize("which", ["vg", "fg"])
-def test_fused_bn_backward_aggregation(graphs, C, which):
-    """ddmp_spmm_bn_bwd (dY recomputed inside the gather) == bn_bwd_apply followed by spmm_gcn"""
-    from dual_dmp_b200 import functional as F_
-    g = graphs["open"][which]
-    torch.manual_seed(C)
-    n = g.n
-    Y = (torch.randn(n, C) * 1.5 + 0.3).to(DEV)
-    gX = torch.randn(n, C, device=DEV)
-    st = F_.bn_stats_finalize(F_.spmm_gcn(GcnGraphIdentity(n), Y, stats=True)[1], n,
-                              (torch.rand(C) + 0.5).to(DEV), torch.randn(C).to(DEV))
-    dY, dgamma, dbeta, dbias = F_.bn_lrelu_backward(gX, Y, st)
-    dH_ref = F_.spmm_gcn(g, dY, transposed=True)
-    dH, dgamma2, dbeta2, dbias2 = F_.bn_bwd_spmm_fused(g, gX, Y, st)
-    e = rel_err(dH, dH_ref)
-    report(f"fused bn+spmm bwd C={C} {which}", e)
-    assert e < 2e-6 and torch.equal(dgamma, dgamma2) and torch.equal(dbeta, dbeta2)
-    assert (dbias2 - dbias).abs().max() <= 1e-5 * dY.abs().sum(dim=0).max()
-    a, _, _, _ = F_.bn_bwd_spmm_fused(g, gX, Y, st)
-    assert torch.equal(a, dH)
-
-
-def GcnGraphIdentity(n):
-    from dual_dmp_b200.graph import GcnGraph
-    return GcnGraph(torch.zeros(2, 0, dtype=torch.long), n, DEV, reorder=False)
-
-
-@pytest.mark.parametrize("C", [32, 64, 128, 256, 512])
 @pytest.mark.parametrize("kind,n", [("ico", 3), ("ico", 10), ("open", 9), ("ico", 40)])
 def test_spmm_default_kernels_equal_reference_kernel_bitwise(kind, n, C):
     """the default kernels (csrc/spmm_tile.cu, TMA-staged row block + shared-memory index stream, at C <= 128) against
@@ -627,36 +599,3 @@ def test_spmm_tensor_memory_statistics_kernel_equals_reference_kernel_bitwise(ki
                 assert torch.equal(x, x0), (i, graph.n, C)
     finally:
         lib.query("ddmp_spmm_reference_kernel", prev)
-
-
-@pytest.mark.parametrize("C", [32, 64, 128, 256, 512])
-@pytest.mark.parametrize("kind,n,which", [("open", 9, "vg"), ("open", 9, "fg"), ("ico", 3, "fg"), ("ico", 24, "vg"),
-                                          ("ico", 24, "fg_id")])
-def test_tile_fused_bn_backward_aggregation(kind, n, which, C):
-    """ddmp_spmm_bn_bwd_tile (dY formed in shared memory from TMA-staged gX / Y tiles, never written to HBM) ==
-    ddmp_bn_bwd_apply followed by ddmp_spmm_gcn, including the conv-bias gradient (column sums of dY) and max|dH|"""
-    from dual_dmp_b200 import functional as F_
-    from dual_dmp_b200.graph import GcnGraph
-    from oracle.step_ref import make_dataset
-    n_mesh, s_mesh, _ = small_case(kind, n)
-    ds = make_dataset(n_mesh, s_mesh)
-    if which == "vg":
-        g = GcnGraph(ds.edge_index, len(n_mesh.vs), DEV, coords=ds.x_pos, reorder=True)
-    else:
-        g = GcnGraph(ds.face_index, len(n_mesh.faces), DEV, coords=ds.z2.detach()[:, :3], reorder=which == "fg")
-    torch.manual_seed(C + n)
-    rows = g.n
-    Y = (torch.randn(rows, C) * 1.5 + 0.3).to(DEV)
-    gX = torch.randn(rows, C, device=DEV)
-    st = F_.bn_stats_finalize(F_.spmm_gcn(GcnGraphIdentity(rows), Y, stats=True)[1], rows,
-                              (torch.rand(C) + 0.5).to(DEV), torch.randn(C).to(DEV))
-    dY, dgamma, dbeta, dbias = F_.bn_lrelu_backward(gX, Y, st)
-    dH_ref = F_.spmm_gcn(g, dY, transposed=True)
-    dH, dgamma2, dbeta2, dbias2, ab = F_.bn_bwd_spmm_tile(g, gX, Y, st, amax=True)
-    e = rel_err(dH, dH_ref)
-    report(f"tile-fused bn+spmm bwd C={C} {kind}{n} {which}", e)
-    assert e < 2e-6 and torch.equal(dgamma, dgamma2) and torch.equal(dbeta, dbeta2)
-    assert (dbias2 - dbias).abs().max() <= 1e-5 * dY.abs().sum(dim=0).max()
-    assert float(ab.max()) == float(dH.abs().max())
-    a, _, _, _, _ = F_.bn_bwd_spmm_tile(g, gX, Y, st)
-    assert torch.equal(a, dH)                                                   # deterministic
